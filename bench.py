@@ -17,6 +17,10 @@ on both sides, max over ranks.
 --impl reference times the reference's CPU algorithm (the C oracle port, kind "port": the Rust crate cannot be built here)
 with all host threads on the same number of blobs per step; it does not load libkzgb200.so.
 --config tuples: BASELINE configs[4], m independent verify_kzg_proof tuples (checks / second).
+--dump-outputs DIR writes what the last timed step returned, as DIR/<name>.npy: the batch path's verdict and every blob's z and y
+(32-bit words of each 32-byte big-endian field element, most significant first, as float64), the tuple path's verdict per tuple
+(1 true, 0 false, 2 Err).  The inputs are seeded, so two builds run with the same arguments can be compared output for output.
+Above DUMP_ROWS blobs or tuples a fixed seeded sample of them is written, with their positions in index.npy.
 """
 import argparse
 import ctypes as C
@@ -30,7 +34,9 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True           # the tree may be read-only: nothing is written into it
 BLOB = 131072
+DUMP_ROWS = 1 << 18                      # z and y of 2^18 blobs as float64 words: 32 MB
 ALGO_BYTES_PER_BLOB = 131072 + 48 + 48   # SURVEY.md 8(d)
 PHASES = ["g1_decompress", "challenge_sha256", "evaluate_barycentric", "transcript_r_exposed", "lincomb_terms", "reduce", "final_pairing",
           "g1_subgroup_deferred"]
@@ -55,7 +61,38 @@ def parse_args():
     ap.add_argument("--lowdegree-blobs", action="store_true",
                     help="blobs = evaluations of random degree<8 polynomials (cheap generator) instead of uniformly random "
                          "blobs committed / proved by the GPU commit/prove path")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy")
     return ap.parse_args()
+
+
+def field_words(raw):
+    """32-byte big-endian field elements -> (n, 8) float64 of their 32-bit words, most significant first (exact)."""
+    import numpy as np
+    return np.frombuffer(raw, dtype=">u4").reshape(-1, 8).astype(np.float64)
+
+
+def dump_outputs(path, arrays):
+    """Writes every array as path/<name>.npy.  Arrays longer than DUMP_ROWS keep a fixed seeded sample of their rows, the same
+    rows for all of them, whose positions go to index.npy."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    n = max(len(a) for a in arrays.values())
+    if n > DUMP_ROWS:
+        idx = np.sort(np.random.default_rng(0x4B5A47).choice(n, DUMP_ROWS, replace=False))
+        arrays = {k: a[idx] if len(a) == n else a for k, a in arrays.items()}
+        arrays["index"] = idx.astype(np.float64)
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
+def all_ranks(dist, t):
+    """A CUDA tensor of the same shape on every rank -> all ranks' copies concatenated in rank order."""
+    import torch
+    if dist is None:
+        return t
+    parts = [torch.empty_like(t) for _ in range(dist.get_world_size())]
+    dist.all_gather(parts, t)
+    return torch.cat(parts)
 
 
 class ClockSampler(threading.Thread):
@@ -150,7 +187,6 @@ def run_reference(args, rank, world):
     if rank != 0:
         return
     from oracle import oracle as O
-    O.build()
     cores = os.cpu_count() or 1
     if args.config == "tuples":
         return run_reference_tuples(args, O, cores)
@@ -159,11 +195,14 @@ def run_reference(args, rank, world):
     times = []
     for i in range(args.warmup + args.steps):
         t = time.perf_counter()
-        rc, ok, _, _ = O.verify_batch_raw(blobs, cs, ps, n, nthreads=cores)
+        rc, ok, z, y = O.verify_batch_raw(blobs, cs, ps, n, nthreads=cores)
         dt = time.perf_counter() - t
         assert rc == 0 and ok, "reference arm rejected a valid batch"
         if i >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        import numpy as np
+        dump_outputs(args.dump_outputs, {"verdict": np.ones(1), "z": field_words(z), "y": field_words(y)})
     ms = 1e3 * sum(times) / len(times)
     val = n / (ms / 1e3)
     sample = "%d blobs per step (the b200 arm's size), %d threads (blob-parallel; the reference itself is single-threaded), SHA-NI=%d" % (
@@ -227,6 +266,9 @@ def run_reference_tuples(args, O, cores):
         assert got == want
         if it >= args.warmup:
             times.append(dt)
+    if args.dump_outputs:
+        import numpy as np
+        dump_outputs(args.dump_outputs, {"verdict": np.frombuffer(got, dtype=np.uint8).astype(np.float32)})
     ms = 1e3 * sum(times) / len(times)
     val = m / (ms / 1e3)
     print(json.dumps({"impl": "reference", "metric": "verify_kzg_proof checks/sec (independent tuples)", "value": val, "unit": "checks/s", "n_gpus": args.gpus,
@@ -281,6 +323,10 @@ def run_tuples(args, rank, world, local_rank):
     sampler.stop_flag = True
     sampler.join(timeout=2)
     ok = out.numpy().tobytes() == want
+    if args.dump_outputs:
+        verdicts = all_ranks(dist, out.cuda()).cpu().numpy()
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"verdict": verdicts.astype("float32")})
     kernel_ms = (C.c_float * 8)()
     lib.kzgb200_get_phase_ms(ctx, kernel_ms)
     if rank == 0:
@@ -438,6 +484,10 @@ def main():
     # ---- headline: library default (exact transcript), one blocking call at a time ----------------------------------
     plan.set_transcript_mode(0)
     ms, phases = timed(lambda: must(plan.verify_device(d_blobs, d_cs, d_ps), "resident"), args.steps, W)
+    if args.dump_outputs:      # the last step's verdict (must() passed: true) and the z, y it wrote; later calls overwrite them
+        z, y = (all_ranks(dist, t).cpu().numpy().tobytes() for t in (plan.z_out, plan.y_out))
+        if rank == 0:
+            dump_outputs(args.dump_outputs, {"verdict": np.ones(1), "z": field_words(z), "y": field_words(y)})
     ms_e2e, _ = timed(lambda: must(plan.verify_host(h_blobs, h_cs, h_ps), "e2e pinned"), args.steps, W)
     launches = args.steps * (count_launches(n, True, "exact", world, rank == 0) + count_launches(n, False, "exact", world, rank == 0))
     sampler.stop_flag = True
@@ -462,7 +512,7 @@ def main():
         # pageable caller memory (an ordinary Vec<Blob>): the library's pinned staging ring
         p_blobs = torch.from_numpy(np.empty(n * BLOB, dtype=np.uint8))
         p_blobs.copy_(h_blobs)
-        ms_pg, _ = timed(lambda: must(plan.verify_host(p_blobs, h_cs, h_ps), "e2e pageable"), max(2, args.steps // 2), 2)
+        ms_pg, _ = timed(lambda: must(plan.verify_host(p_blobs, h_cs, h_ps), "e2e pageable"), args.steps, 2)
         extras["pageable"] = ms_pg
         del p_blobs
         # the other transcript modes, same workload
@@ -470,16 +520,15 @@ def main():
             if world > 1 and mode == 2:
                 continue
             plan.set_transcript_mode(mode)
-            st = args.steps if mode == 1 else min(args.steps, 3)
-            m1, ph1 = timed(lambda: must(plan.verify_device(d_blobs, d_cs, d_ps), name), st, 2)
-            m2 = timed(lambda: must(plan.verify_host(h_blobs, h_cs, h_ps), name + " e2e"), st, 2)[0] if mode == 1 else None
+            m1, ph1 = timed(lambda: must(plan.verify_device(d_blobs, d_cs, d_ps), name), args.steps, 2)
+            m2 = timed(lambda: must(plan.verify_host(h_blobs, h_cs, h_ps), name + " e2e"), args.steps, 2)[0] if mode == 1 else None
             extras[name] = (m1, ph1, m2)
         plan.set_transcript_mode(0)
 
     # Streaming front-end (kzgb200_pipeline_*, SURVEY 8f-3), single GPU, default transcript: several batches in flight
     pipelined = None
     if world == 1 and not args.no_extras:
-        pipe_batches = max(args.steps, 12)
+        pipe_batches = args.steps
         with K.BatchPipeline(S, depth=args.inflight, device=local_rank) as pipe:
             def run(submit, steps):
                 tickets = [submit() for _ in range(steps)]
@@ -592,7 +641,6 @@ def main():
                                                      "the exact chain on one warp of the GPU (round 1's default)", **modes}
     if rank == 0 and not args.no_cpu_baseline:
         from oracle import oracle as O
-        O.build()
         cores = os.cpu_count() or 1
         m = m_par
         hb = h_blobs[:m * BLOB].numpy().tobytes(); hc = h_cs[:m * 48].numpy().tobytes(); hp = h_ps[:m * 48].numpy().tobytes()

@@ -1,3 +1,4 @@
+import gzip
 import json
 import os
 import sys
@@ -24,7 +25,8 @@ class Vectors:
     def __init__(self):
         with open(os.path.join(GOLDEN, "ckzg_vectors.json")) as fh:
             self.v = json.load(fh)
-        raw = open(os.path.join(GOLDEN, "ckzg_blobs.bin"), "rb").read()
+        with gzip.open(os.path.join(GOLDEN, "ckzg_blobs.bin.gz"), "rb") as fh:
+            raw = fh.read()
         self.blobs, off = [], 0
         for n in self.v["blob_lengths"]:
             self.blobs.append(raw[off:off + n])

@@ -12,11 +12,11 @@ Sources (all read-only):
   /root/reference/src/trusted_setup.txt                         (mainnet ceremony output)
 Outputs:
   tests/golden/ckzg_vectors.json   cases; blobs are referenced by index into the blob store
-  tests/golden/ckzg_blobs.bin      the distinct blobs, concatenated (lengths in the json)
+  tests/golden/ckzg_blobs.bin.gz   the distinct blobs, concatenated (lengths in the json), gzip-compressed
   kzg_rs_b200/data/mainnet_setup.bin   "KZGS" | u32 n1 | u32 n2 | n1*48 B G1 Lagrange (file order) | n2*96 B G2 monomial
 Also records the two known-answer tests of kzg_proof.rs:739-778.
 """
-import glob, hashlib, json, os, struct, sys
+import glob, gzip, hashlib, json, os, struct, sys
 import yaml
 
 REF = "/root/reference"
@@ -73,9 +73,8 @@ out["blob_sha256"] = [hashlib.sha256(b).hexdigest() for b in blob_store]
 
 with open(os.path.join(HERE, "ckzg_vectors.json"), "w") as fh:
     json.dump(out, fh, indent=0, separators=(",", ":"))
-with open(os.path.join(HERE, "ckzg_blobs.bin"), "wb") as fh:
-    for b in blob_store:
-        fh.write(b)
+with open(os.path.join(HERE, "ckzg_blobs.bin.gz"), "wb") as fh:
+    fh.write(gzip.compress(b"".join(blob_store), 9, mtime=0))
 
 lines = open(REF + "/src/trusted_setup.txt").read().split()
 n1, n2 = int(lines[0]), int(lines[1])
