@@ -5,6 +5,7 @@
 //   kzg_rs::KzgSettings::load_trusted_setup_file                                                src/trusted_setup.rs:94-98
 //   kzg_rs::Blob / Bytes32 / Bytes48 (from_slice length check, as_slice)                        src/dtypes.rs:7-46
 //   kzg_rs::KzgError                                                                            src/enums.rs:6-18
+// plus EIP-7594 cells: kzg_rs::Cell, KzgProof::verify_cell_kzg_proof_batch, kzg_rs::compute_cells (c-kzg-4844 / rust-kzg names).
 // Result<bool, KzgError> is kzg_rs::Result<bool>: either a value or an error.
 #pragma once
 #include <array>
@@ -24,6 +25,8 @@ constexpr size_t BYTES_PER_BLOB = KZGB200_BYTES_PER_BLOB;
 constexpr size_t BYTES_PER_COMMITMENT = KZGB200_BYTES_PER_COMMITMENT;
 constexpr size_t BYTES_PER_PROOF = KZGB200_BYTES_PER_PROOF;
 constexpr size_t BYTES_PER_FIELD_ELEMENT = KZGB200_BYTES_PER_FIELD_ELEMENT;
+constexpr size_t BYTES_PER_CELL = 2048;          // EIP-7594: 64 field elements of the extended blob
+constexpr size_t CELLS_PER_EXT_BLOB = 128;
 
 struct KzgError {
     enum Kind { BadArgs, InternalError, InvalidBytesLength, InvalidHexFormat, InvalidTrustedSetup } kind;
@@ -59,6 +62,7 @@ struct BytesN {
 using Bytes32 = BytesN<32>;
 using Bytes48 = BytesN<48>;
 using Blob = BytesN<BYTES_PER_BLOB>;
+using Cell = BytesN<BYTES_PER_CELL>;
 static_assert(sizeof(Blob) == BYTES_PER_BLOB && sizeof(Bytes48) == 48, "vectors of these are contiguous byte arrays");
 
 class KzgSettings {
@@ -83,6 +87,14 @@ public:
         return s;
     }
     kzgb200_ctx* ctx() const { return ctx_.get(); }
+    // cell proofs (EIP-7594): the setup's [tau^j]G1, j < 64 at least (for mainnet: kzg_rs_b200/data/g1_monomial.txt, hex-decoded), and
+    // g2_points[64]; once, before the cell calls
+    Result<bool> load_cell_setup(const uint8_t* g1_monomial48, size_t n_points) const {
+        if (g2_points.size() < 65 * 96) return KzgError{KzgError::InvalidTrustedSetup, "the setup has no G2 point 64"};
+        int rc = kzgb200_load_cell_setup(ctx(), g1_monomial48, n_points, g2_points.data() + 64 * 96);
+        if (rc) return KzgError{rc == KZGB200_INVALID_SETUP ? KzgError::InvalidTrustedSetup : KzgError::InternalError, "kzgb200_load_cell_setup failed"};
+        return true;
+    }
 };
 
 namespace detail {
@@ -121,7 +133,28 @@ struct KzgProof {
                                                      nullptr, nullptr);
         return detail::to_result(rc, ok, blobs.size() != commitments_bytes.size() ? "Invalid commitments length" : "Invalid proofs length");
     }
+    // EIP-7594: one entry per cell (its blob's commitment, its index < 128, the cell, its proof)
+    static Result<bool> verify_cell_kzg_proof_batch(const std::vector<Bytes48>& commitments_bytes, const std::vector<uint64_t>& cell_indices,
+                                                    const std::vector<Cell>& cells, const std::vector<Bytes48>& proofs_bytes,
+                                                    const KzgSettings& kzg_settings) {
+        const size_t n = cell_indices.size();
+        if (commitments_bytes.size() != n || cells.size() != n || proofs_bytes.size() != n)
+            return KzgError{KzgError::InvalidBytesLength, "Invalid cells / commitments / proofs length"};
+        int ok = 0;
+        int rc = kzgb200_verify_cell_kzg_proof_batch(kzg_settings.ctx(), reinterpret_cast<const uint8_t*>(commitments_bytes.data()),
+                                                     cell_indices.data(), reinterpret_cast<const uint8_t*>(cells.data()),
+                                                     reinterpret_cast<const uint8_t*>(proofs_bytes.data()), n, &ok);
+        return detail::to_result(rc, ok);
+    }
 };
+
+// EIP-7594 compute_cells: the 128 cells of the blob's extension
+inline Result<std::vector<Cell>> compute_cells(const Blob& blob, const KzgSettings& kzg_settings) {
+    std::vector<Cell> cells(CELLS_PER_EXT_BLOB);
+    int rc = kzgb200_compute_cells(kzg_settings.ctx(), blob.as_slice(), reinterpret_cast<uint8_t*>(cells.data()));
+    if (rc) return detail::to_result(rc, 0).unwrap_err();
+    return cells;
+}
 
 // Streaming front-end (include/kzgb200.h, kzgb200_pipeline_*): `depth` verify_blob_kzg_proof_batch calls in flight on one GPU.
 // The pipeline owns the submitted vectors until the ticket has been waited for (the C ABI reads them asynchronously).

@@ -153,7 +153,7 @@ int kzgb200_group_host_protocol_test(const char* session, int rank, int world, c
 #define KZGB200_TRANSCRIPT_TREE 1
 #define KZGB200_TRANSCRIPT_EXACT_DEVICE 2
 int kzgb200_set_transcript_mode(kzgb200_ctx* ctx, int mode);
-/* canonical big-endian r of the last batch verified on this context (n >= 2) */
+/* canonical big-endian r of the last batch verified on this context (blob batches: n >= 2; cell batches: n >= 1) */
 int kzgb200_last_r(kzgb200_ctx* ctx, uint8_t* r_out32);
 /* test hook: SHA-256 of msg by the host code that hashes the transcript; force_portable = 1 selects the portable compression
  * function; returns 1 if the SHA-NI path was used */
@@ -179,6 +179,32 @@ int kzgb200_load_g1_lagrange(kzgb200_ctx* ctx, const uint8_t* g1_lagrange, size_
 int kzgb200_blob_to_kzg_commitment_batch(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8_t* d_commitments_out);
 int kzgb200_compute_blob_kzg_proof_batch(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t* d_commitments, size_t n,
                                          uint8_t* d_proofs_out);
+
+/* ---- EIP-7594 cells (PeerDAS; consensus-specs Fulu, polynomial-commitments-sampling.md) ---------------------------------
+ * A blob extends to 8192 values (the polynomial on the 8192 roots of unity, bit-reversed order), split into 128 cells of 64 field
+ * elements (2048 bytes, 32 big-endian bytes each).  Cells 0..63 are the blob itself.  Each cell has its own KZG multi-proof.
+ * kzgb200_load_cell_setup: [tau^j]G1 for j < 64 at least (host, n_points x 48, compressed; for mainnet the
+ *   points of kzg_rs_b200/data/g1_monomial.txt, one hex line each) and g2_monomial[64] = [tau^64]G2 (96 bytes).  Once per context; every cell entry point returns
+ *   KZGB200_INVALID_SETUP before it.
+ * kzgb200_verify_cell_kzg_proof_batch: one entry per cell -- the commitment of its blob, its index (< 128), the cell, its proof;
+ *   n == 0 -> Ok(true); an index >= 128, a non-canonical cell element, or a commitment / proof that is not a valid compressed
+ *   point of the G1 subgroup -> KZGB200_BAD_ARGS.  The batch challenge r is the spec's (commitments deduplicated by their bytes),
+ *   hashed by a host thread over the caller's buffers while the GPU parses the inputs; kzgb200_last_r returns it afterwards.
+ *   The _device form takes device pointers; the inputs are copied back to pinned host memory once for the hash.
+ * kzgb200_compute_cells: the 128 cells of one host blob (cells_out: 128 x 2048 bytes, host);
+ * kzgb200_compute_cells_batch_device: n device blobs -> n x 128 cells (device, blob-major).  Non-canonical element -> BAD_ARGS. */
+int kzgb200_load_cell_setup(kzgb200_ctx* ctx, const uint8_t* g1_monomial48, size_t n_points, const uint8_t* g2_tau64_96);
+int kzgb200_verify_cell_kzg_proof_batch(kzgb200_ctx* ctx, const uint8_t* commitments, const uint64_t* cell_indices, const uint8_t* cells,
+                                        const uint8_t* proofs, size_t n, int* ok);
+int kzgb200_verify_cell_kzg_proof_batch_device(kzgb200_ctx* ctx, const uint8_t* d_commitments, const uint64_t* d_cell_indices,
+                                               const uint8_t* d_cells, const uint8_t* d_proofs, size_t n, int* ok);
+int kzgb200_compute_cells(kzgb200_ctx* ctx, const uint8_t* blob, uint8_t* cells_out);
+int kzgb200_compute_cells_batch_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8_t* d_cells);
+/* cell workload (test / bench data): n_blobs seeded polynomials of degree < `degree` (128 < degree <= 192) built from their
+ * coefficients, their cells (n_blobs x 128 x 2048, device), commitments (n_blobs x 48) and the proofs of all their cells
+ * (n_blobs x 128 x 48, same order as the cells); tau_powers48 = [tau^j]G1, j < degree (host).  Needs the cell setup. */
+int kzgb200_harness_generate_cells(kzgb200_ctx* ctx, uint64_t seed, size_t n_blobs, int degree, const uint8_t* tau_powers48,
+                                   uint8_t* d_cells, uint8_t* d_commitments, uint8_t* d_proofs);
 
 /* per-phase device timing of batch calls (CUDA event pairs on the stream each phase runs on).  out8 = milliseconds of
  * {G1 decompression, challenge, evaluate, transcript r (exposed part: last chunk copy + host hash + upload), lincomb terms, reduce,

@@ -19,6 +19,8 @@ BYTES_PER_BLOB = 131072          # src/consts.rs:8
 BYTES_PER_COMMITMENT = 48        # src/consts.rs:9
 BYTES_PER_PROOF = 48             # src/consts.rs:10
 BYTES_PER_FIELD_ELEMENT = 32     # src/consts.rs:3
+BYTES_PER_CELL = 2048            # EIP-7594: 64 field elements of the extended blob
+CELLS_PER_EXT_BLOB = 128
 PARTIAL_BYTES = 352
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
@@ -111,6 +113,12 @@ class Library:
         d.kzgb200_alloc_pinned.argtypes = [sz]
         d.kzgb200_alloc_pinned.restype = p
         d.kzgb200_free_pinned.argtypes = [p]
+        d.kzgb200_load_cell_setup.argtypes = [p, C.c_char_p, sz, C.c_char_p]
+        d.kzgb200_verify_cell_kzg_proof_batch.argtypes = [p, p, p, p, p, sz, ip]
+        d.kzgb200_verify_cell_kzg_proof_batch_device.argtypes = [p, p, p, p, p, sz, ip]
+        d.kzgb200_compute_cells.argtypes = [p, C.c_char_p, p]
+        d.kzgb200_compute_cells_batch_device.argtypes = [p, p, sz, p]
+        d.kzgb200_harness_generate_cells.argtypes = [p, C.c_uint64, sz, C.c_int, C.c_char_p, p, p, p]
 
 
 def _raise(rc, ctx=None, msg=None):
@@ -166,27 +174,38 @@ class Blob(_BytesN):
     SIZE = BYTES_PER_BLOB
 
 
+class Cell(_BytesN):
+    """EIP-7594 cell: 64 field elements (32 bytes big-endian each) of the extended blob."""
+    SIZE = BYTES_PER_CELL
+
+
 class KzgSettings:
     """src/trusted_setup.rs:44-50.  Holds the setup and one device context per GPU (created on first use:
     the device-resident tables -- roots of unity, Miller-loop lines of g2_points[0..2] -- are built there)."""
     _default = None
     _dlock = threading.Lock()
 
-    def __init__(self, g1_lagrange_bytes, g2_monomial_bytes):
+    def __init__(self, g1_lagrange_bytes, g2_monomial_bytes, g1_monomial_bytes=None):
         self.g1_lagrange_bytes = g1_lagrange_bytes      # 4096 x 48 (file order); unused by verification
-        self.g2_monomial_bytes = g2_monomial_bytes      # 65 x 96; verification reads [0] and [1]
+        self.g2_monomial_bytes = g2_monomial_bytes      # 65 x 96; blob verification reads [0] and [1], cell verification [64]
+        # [tau^j]G1, j >= 64, compressed: cell verification needs j < 64.  None: the shipped points when this is the mainnet setup
+        self.g1_monomial_bytes = g1_monomial_bytes
         self._ctx = {}
+        self._cells = set()
         self._lock = threading.Lock()
 
     @classmethod
-    def load_trusted_setup_file(cls, path=None):
-        """Default: the embedded mainnet setup (the reference embeds it at build time, build.rs:23-87)."""
+    def load_trusted_setup_file(cls, path=None, g1_monomial_bytes=None):
+        """Default: the embedded mainnet setup (the reference embeds it at build time, build.rs:23-87).  g1_monomial_bytes: the
+        setup's [tau^j]G1 (j < 64 at least) for cell proofs under a custom setup."""
         if path is None:
             with cls._dlock:
                 if cls._default is None:
                     cls._default = cls._load(os.path.join(_HERE, "data", "mainnet_setup.bin"))
                 return cls._default
-        return cls._load(path)
+        s = cls._load(path)
+        s.g1_monomial_bytes = g1_monomial_bytes
+        return s
 
     @classmethod
     def _load(cls, path):
@@ -220,11 +239,42 @@ class KzgSettings:
                 self._ctx[device] = h
             return self._ctx[device]
 
+    def _monomial_points(self):
+        if self.g1_monomial_bytes is not None:
+            return self.g1_monomial_bytes
+        with open(os.path.join(_HERE, "data", "mainnet_setup.bin"), "rb") as fh:
+            raw = fh.read()
+        n1 = struct.unpack("<I", raw[4:8])[0]
+        if self.g1_lagrange_bytes == raw[12:12 + n1 * 48] and self.g2_monomial_bytes[:65 * 96] == raw[12 + n1 * 48:12 + n1 * 48 + 65 * 96]:
+            return mainnet_g1_monomial()
+        raise KzgError("InvalidTrustedSetup", "cell proofs need the setup's monomial G1 points (g1_monomial_bytes)")
+
+    def cell_context(self, device=0):
+        """The device context with the cell tables loaded (EIP-7594: [tau^j]G1, j < 64, and g2_monomial[64])."""
+        ctx = self.context(device)
+        with self._lock:
+            if device not in self._cells:
+                if len(self.g2_monomial_bytes) < 65 * 96:
+                    raise KzgError("InvalidTrustedSetup", "cell proofs need the setup's G2 point 64")
+                g1m = self._monomial_points()
+                rc = Library.get().dll.kzgb200_load_cell_setup(ctx, g1m, len(g1m) // 48, self.g2_monomial_bytes[64 * 96:65 * 96])
+                if rc:
+                    _raise(rc, ctx)
+                self._cells.add(device)
+        return ctx
+
     def close(self):
         with self._lock:
             for h in self._ctx.values():
                 Library.get().dll.kzgb200_destroy(h)
             self._ctx = {}
+            self._cells = set()
+
+
+def mainnet_g1_monomial():
+    """[tau^j]G1, j < 192, of the mainnet setup: 192 x 48 bytes, compressed (kzg_rs_b200/data/g1_monomial.txt, one hex point per line)."""
+    with open(os.path.join(_HERE, "data", "g1_monomial.txt")) as fh:
+        return b"".join(bytes.fromhex(line) for line in fh.read().split())
 
 
 def _b(x, size, what):
@@ -318,6 +368,39 @@ class KzgProof:
         if rc:
             _raise(rc, ctx)
         return out.raw[:m]
+
+
+    @staticmethod
+    def verify_cell_kzg_proof_batch(commitments_bytes, cell_indices, cells, proofs_bytes, kzg_settings, device=0):
+        """EIP-7594 verify_cell_kzg_proof_batch: commitments_bytes / cell_indices / cells / proofs_bytes are sequences of one
+        entry per cell (commitment of the cell's blob, its index < 128, the cell, its proof).  Mismatched lengths ->
+        KzgError(InvalidBytesLength); an index >= 128, a non-canonical cell element or an invalid point -> KzgError(BadArgs)."""
+        n = len(cell_indices)
+        if not (len(commitments_bytes) == len(cells) == len(proofs_bytes) == n):
+            raise KzgError("InvalidBytesLength", "Invalid cells / commitments / proofs length")
+        cs = b"".join(_b(x, 48, "commitment") for x in commitments_bytes)
+        ce = b"".join(_b(x, BYTES_PER_CELL, "cell") for x in cells)
+        ps = b"".join(_b(x, 48, "proof") for x in proofs_bytes)
+        if any(not 0 <= int(i) < 1 << 64 for i in cell_indices):
+            raise KzgError("BadArgs", "Invalid cell index")
+        idx = (C.c_uint64 * max(n, 1))(*[int(i) for i in cell_indices])
+        ctx, ok = kzg_settings.cell_context(device), C.c_int(0)
+        rc = Library.get().dll.kzgb200_verify_cell_kzg_proof_batch(ctx, _ptr(cs), C.cast(idx, C.c_void_p), _ptr(ce), _ptr(ps), n, C.byref(ok))
+        if rc:
+            _raise(rc, ctx, "Failed to parse cell / G1Affine / cell index" if rc == 1 else None)
+        return bool(ok.value)
+
+
+def compute_cells(blob, kzg_settings, device=0):
+    """EIP-7594 compute_cells: the 128 cells (2048 bytes each) of the blob's extension; BadArgs on a non-canonical element."""
+    b = _b(blob, BYTES_PER_BLOB, "blob")
+    ctx = kzg_settings.cell_context(device)
+    out = C.create_string_buffer(BYTES_PER_CELL * CELLS_PER_EXT_BLOB)
+    rc = Library.get().dll.kzgb200_compute_cells(ctx, b, out)
+    if rc:
+        _raise(rc, ctx, "Failed to parse blob" if rc == 1 else None)
+    raw = out.raw
+    return [raw[BYTES_PER_CELL * k:BYTES_PER_CELL * (k + 1)] for k in range(CELLS_PER_EXT_BLOB)]
 
 
 def compute_challenge(blob, commitment_bytes, kzg_settings, device=0):

@@ -58,6 +58,12 @@ constexpr int kManyCtasPerSm = 1;                     // (two CTAs of 14 checks 
 constexpr int kManyWarps = 4;         // many_pairing_warp_kernel (identity inputs): one check per warp
 constexpr int kHarnessMaxDegree = 16;
 constexpr int kLagWindows = 32, kLagEntries = 255;
+// EIP-7594 cells (k_cells.cu)
+constexpr int kCellsPerExtBlob = 128, kFieldElementsPerCell = 64, kBytesPerCell = 2048;
+constexpr int kCellNttThreads = 512;                              // compute_cells_kernel: one CTA per blob, 4096 values in shared memory
+constexpr int kCellNttSmemBytes = kFieldElementsPerBlob * 32;     // 128 KiB
+constexpr int kCellAggSlices = 16;                                // CTAs per cell index of the r-weighted value sums
+constexpr int kCellHarnessMaxDegree = 192;
 
 __device__ __forceinline__ Fr load_fe_be(const uint4* p) {
     uint4 hi = __ldg(p), lo = __ldg(p + 1);   // 32 big-endian bytes: hi holds the most significant 16
@@ -97,6 +103,20 @@ struct FinalPts { G1Affine pts[2]; uint32_t go; };
 constexpr int kManyStride = vliw::kTotalRegsThr * 12 + 1;     // words between the register files of consecutive groups (odd: bank skew)
 constexpr int kManySmemBytes = kManyGroups * kManyStride * 4 + (int)sizeof(vliw::SharedTables) + vliw::kNumSharedRegs * (int)sizeof(Fp) +
                                kManyGroups * (2 * (int)sizeof(G1Affine) + 2) + 64;
+// Device tables of the cell path (kzgb200_load_cell_setup): roots of unity of the extended domain, the fixed bases of the RLI
+// MSM, and the Miller-loop lines of [tau^64]G2.
+struct CellTables {
+    Fr w4096[2048], w4096_inv[2048];   // omega4096^(+-k), natural order, Montgomery
+    Fr coset[4096];                    // omega8192^m / 4096
+    Fr shift64[kCellsPerExtBlob];      // h_k^64 = omega128^rev7(k)
+    Fr shift_inv[kCellsPerExtBlob];    // h_k^-1
+    Fr w64_inv[kFieldElementsPerCell / 2];
+    Fr omega8192, inv64;
+    G1Affine tau_tab[kFieldElementsPerCell][4];   // [2^(64q) tau^m]G1
+    LineCoeffs tau64_lines[kMillerSteps];
+    vliw29::LineCoeffs29 lines29[kMillerSteps];    // [tau^64]G2 for pairing_check_kernel
+    uint32_t ok;
+};
 // ---- kernels (k_*.cu) ----------------------------------------------------------------------------------------
 __global__ void setup_tables_kernel(DeviceTables* T, const uint8_t* g2_points);
 __global__ void setup_lines29_kernel(DeviceTables* T);
@@ -137,16 +157,17 @@ __global__ void batch_final_kernel(const Partial* __restrict__ parts, int nparts
 __global__ void single_final_kernel(const G1Affine* __restrict__ C, const G1Affine* __restrict__ P, const ZY* __restrict__ zy,
                                     const uint32_t* __restrict__ status, const DeviceTables* __restrict__ T, uint32_t* __restrict__ result,
                                     FinalPts* __restrict__ out);
-__global__ void pairing_check_kernel(const FinalPts* __restrict__ in, const DeviceTables* __restrict__ T, uint32_t* __restrict__ result,
-                                     long long* __restrict__ ticks);
+// lines_b: line table of the G2 point paired with pts[0]; nullptr = [tau]G2 (T->lines29[1], the blob checks)
+__global__ void pairing_check_kernel(const FinalPts* __restrict__ in, const DeviceTables* __restrict__ T, const vliw29::LineCoeffs29* __restrict__ lines_b,
+                                     uint32_t* __restrict__ result, long long* __restrict__ ticks);
 __global__ void engine_selftest_kernel(uint32_t seed, int rounds, f29::F29* __restrict__ ref, uint32_t* __restrict__ mismatches);
 // final check of a batch = G1 prelude + pairing engine, back to back on `st`; scratch512 = the context's 512-byte device scratch
-// (ticks at +128 when profiling, the hand-over points at +256)
+// (ticks at +128 when profiling, the hand-over points at +256); lines_b: see pairing_check_kernel (cells: [tau^64]G2)
 inline void launch_batch_final(cudaStream_t st, const Partial* parts, int nparts, const DeviceTables* T, uint32_t* result, unsigned char* scratch512,
-                               bool ticks) {
+                               bool ticks, const vliw29::LineCoeffs29* lines_b = nullptr) {
     FinalPts* fp = reinterpret_cast<FinalPts*>(scratch512 + 256);
     batch_final_kernel<<<1, kFinalThreads, sizeof(FinalSmem), st>>>(parts, nparts, T, result, fp);
-    pairing_check_kernel<<<1, kPairThreads, sizeof(PairSmem), st>>>(fp, T, result, ticks ? reinterpret_cast<long long*>(scratch512 + 128) : nullptr);
+    pairing_check_kernel<<<1, kPairThreads, sizeof(PairSmem), st>>>(fp, T, lines_b, result, ticks ? reinterpret_cast<long long*>(scratch512 + 128) : nullptr);
 }
 __global__ void many_lhs_kernel(const uint8_t* __restrict__ z32, const uint8_t* __restrict__ y32, const G1Affine* __restrict__ C,
                                 const G1Affine* __restrict__ P, size_t m, const DeviceTables* __restrict__ T, G1Affine* __restrict__ X,
@@ -170,5 +191,26 @@ __global__ void blob_scalars_kernel(const uint8_t* __restrict__ blobs, int n, Fr
 __global__ void quotient_kernel(const uint8_t* __restrict__ blobs, int n, const Fr* __restrict__ z_mont, const ZY* __restrict__ zy,
                                 const DeviceTables* __restrict__ T, Fr* __restrict__ scalars);
 __global__ void lag_msm_kernel(const Fr* __restrict__ scalars, int n, const G1* __restrict__ table, uint8_t* __restrict__ out48);
+__global__ void cell_setup_kernel(CellTables* T, const uint8_t* __restrict__ g2_tau64);
+__global__ void cell_setup_points_kernel(CellTables* T, const uint8_t* __restrict__ g1_monomial48);
+__global__ void cell_setup_lines29_kernel(CellTables* T);
+__global__ void compute_cells_kernel(const uint8_t* __restrict__ blobs, int n, const CellTables* __restrict__ T, uint8_t* __restrict__ cells,
+                                     uint32_t* __restrict__ status);
+__global__ void cell_points_kernel(const uint8_t* __restrict__ bytes, int count, G1Affine* __restrict__ out, uint32_t* __restrict__ status, uint32_t flag);
+__global__ void cell_check_kernel(const uint8_t* __restrict__ cells, int n, uint32_t* __restrict__ status);
+// meta = [cell index (n) | unique-commitment index (n) | cells ordered by cell index (n) | start of each index in that order (129)]
+__global__ void cell_scalars_kernel(const uint32_t* __restrict__ meta, int n, const G1Affine* __restrict__ U, const uint32_t* __restrict__ ustatus,
+                                    const CellTables* __restrict__ T, Fr* __restrict__ z_mont, ZY* __restrict__ zy, G1Affine* __restrict__ C,
+                                    uint32_t* __restrict__ status);
+__global__ void cell_rpow_kernel(const Fr* __restrict__ r_mont, int n, Fr* __restrict__ rk);
+__global__ void cell_agg_kernel(const uint8_t* __restrict__ cells, const uint32_t* __restrict__ meta, int n, const Fr* __restrict__ rk, Fr* __restrict__ agg);
+__global__ void cell_interp_kernel(const Fr* __restrict__ agg, const uint32_t* __restrict__ meta, int n, const CellTables* __restrict__ T,
+                                   Fr* __restrict__ coeffs);
+__global__ void cell_rli_kernel(const Fr* __restrict__ coeffs, const CellTables* __restrict__ T, Partial* __restrict__ out);
+__global__ void cell_harness_terms_kernel(uint64_t seed, int n, int D, const G1Affine* __restrict__ M, G1* __restrict__ terms);
+__global__ void cell_harness_sums_kernel(int n, const G1* __restrict__ terms, G1* __restrict__ sums);
+__global__ void cell_harness_points_kernel(int n, const G1* __restrict__ sums, const CellTables* __restrict__ T, uint8_t* __restrict__ commitments,
+                                           uint8_t* __restrict__ proofs);
+__global__ void cell_harness_eval_kernel(uint64_t seed, int n, int D, const CellTables* __restrict__ T, uint8_t* __restrict__ cells);
 
 }  // namespace kzgb200

@@ -39,9 +39,11 @@ __global__ void __launch_bounds__(kFinalThreads) batch_final_kernel(const Partia
     }
 }
 
-// e(pts[1], G2) e(pts[0], [tau]G2) == 1 on the cooperative engine (vliw29.cuh): kPairThreads threads = 24 warps.
+// e(pts[1], G2) e(pts[0], Q) == 1 on the cooperative engine (vliw29.cuh): kPairThreads threads = 24 warps.  Q = [tau]G2, or the
+// point whose line table lines_b is (cell proofs: [tau^64]G2).
 __global__ void __launch_bounds__(kPairThreads) pairing_check_kernel(const FinalPts* __restrict__ in, const DeviceTables* __restrict__ T,
-                                                                     uint32_t* __restrict__ result, long long* __restrict__ ticks) {
+                                                                     const vliw29::LineCoeffs29* __restrict__ lines_b, uint32_t* __restrict__ result,
+                                                                     long long* __restrict__ ticks) {
     extern __shared__ __align__(16) unsigned char dyn_smem[];
     PairSmem& S = *reinterpret_cast<PairSmem*>(dyn_smem);
     const int t = threadIdx.x;
@@ -50,7 +52,7 @@ __global__ void __launch_bounds__(kPairThreads) pairing_check_kernel(const Final
     vliw29::Tables tab = vliw29::load_tables(&S.stab, t, kPairThreads);
     vliw29::Lanes L{t, kPairThreads, tab, ticks, S.stab.p29};
     const G1Affine p0 = in->pts[0], p1 = in->pts[1];
-    bool ok = vliw29::coop_pairing_product_is_one(S.regs, p1, T->lines29[0], p0, T->lines29[1], L);
+    bool ok = vliw29::coop_pairing_product_is_one(S.regs, p1, T->lines29[0], p0, lines_b ? lines_b : T->lines29[1], L);
     L.tick(5);
     if (t == 0) { result[0] = ok ? kTrue : kFalse; result[1] = 0; }
 }

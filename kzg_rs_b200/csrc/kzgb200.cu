@@ -510,10 +510,12 @@ extern "C" int kzgb200_create(kzgb200_ctx** out, int device, const uint8_t* g2_p
     return KZGB200_OK;
 }
 
+static void cell_destroy(kzgb200_ctx* ctx);
 extern "C" void kzgb200_destroy(kzgb200_ctx* ctx) {
     if (!ctx) return;
     DeviceGuard dev(ctx->device);
     cudaDeviceSynchronize();
+    cell_destroy(ctx);
     delete ctx->pool;
     for (cudaStream_t st : {ctx->s_aux, ctx->s_copy, ctx->s_d2h, ctx->s_work[0], ctx->s_work[1], ctx->s_work[2], ctx->s_work[3]}) if (st) cudaStreamDestroy(st);
     for (cudaEvent_t e : {ctx->ev_begin, ctx->ev_parse, ctx->ev_decomp, ctx->ev_bucket, ctx->ev_sha_all, ctx->ev_leaf}) if (e) cudaEventDestroy(e);
@@ -562,7 +564,7 @@ static int batch_locked(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t*
         CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_parse, 0));
         FinalPts* fp = reinterpret_cast<FinalPts*>(ctx->d_scratch + 256);
         single_final_kernel<<<1, kFinalThreads, sizeof(FinalSmem), ctx->stream>>>(ctx->d_C, ctx->d_P, ctx->d_zy, ctx->d_status, ctx->tables, ctx->d_result, fp);
-        pairing_check_kernel<<<1, kPairThreads, sizeof(PairSmem), ctx->stream>>>(fp, ctx->tables, ctx->d_result, nullptr);
+        pairing_check_kernel<<<1, kPairThreads, sizeof(PairSmem), ctx->stream>>>(fp, ctx->tables, nullptr, ctx->d_result, nullptr);
     } else {
         if ((rc = transcript_progress(ctx, true))) return rc;     // the host hashes the transcript behind the evaluation chunks
         if ((rc = transcript_finish(ctx))) return rc;
@@ -972,3 +974,295 @@ extern "C" void* kzgb200_alloc_pinned(size_t bytes) {
     return cudaMallocHost(&p, bytes) == cudaSuccess ? p : nullptr;
 }
 extern "C" void kzgb200_free_pinned(void* p) { if (p) cudaFreeHost(p); }
+
+// ---- EIP-7594 cells (k_cells.cu; consensus-specs Fulu polynomial-commitments-sampling.md) ---------------------------------
+static void cell_destroy(kzgb200_ctx* ctx) {
+    CellCtx* c = ctx->cells;
+    if (!c) return;
+    void* d[] = {c->tables, c->d_cells, c->d_p, c->d_uc, c->d_meta, c->d_ustatus, c->d_U, c->d_rk, c->d_agg, c->d_coeffs, c->d_part, c->d_ext};
+    for (void* p : d) if (p) cudaFree(p);
+    void* h[] = {c->h_meta, c->h_uc, c->h_c, c->h_cells, c->h_p, c->h_idx};
+    for (void* p : h) if (p) cudaFreeHost(p);
+    for (cudaEvent_t e : {c->ev_r, c->ev_rli}) if (e) cudaEventDestroy(e);
+    delete c;
+    ctx->cells = nullptr;
+}
+
+extern "C" int kzgb200_load_cell_setup(kzgb200_ctx* ctx, const uint8_t* g1_monomial48, size_t n_points, const uint8_t* g2_tau64_96) {
+    if (!ctx) return KZGB200_BAD_ARGS;
+    if (!g1_monomial48 || n_points < (size_t)kFieldElementsPerCell || !g2_tau64_96) return KZGB200_INVALID_SETUP;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    if (ctx->cells) return KZGB200_OK;
+    CellCtx* c = new (std::nothrow) CellCtx();
+    if (!c) return KZGB200_INTERNAL_ERROR;
+    ctx->cells = c;
+    uint8_t* d_bytes = nullptr;
+    uint32_t ok = 0;
+    int rc = [&]() -> int {
+        CK(cudaMalloc(&c->tables, sizeof(CellTables)));
+        CK(cudaMalloc(&d_bytes, kFieldElementsPerCell * 48 + 96));
+        CK(cudaMemcpyAsync(d_bytes, g1_monomial48, kFieldElementsPerCell * 48, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(d_bytes + kFieldElementsPerCell * 48, g2_tau64_96, 96, cudaMemcpyHostToDevice, ctx->stream));
+        cell_setup_kernel<<<4096 / 128, 128, 0, ctx->stream>>>(c->tables, d_bytes + kFieldElementsPerCell * 48);
+        cell_setup_points_kernel<<<kFieldElementsPerCell * 4 / 64, 64, 0, ctx->stream>>>(c->tables, d_bytes);
+        cell_setup_lines29_kernel<<<(kMillerSteps * 6 + 127) / 128, 128, 0, ctx->stream>>>(c->tables);
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(&ok, &c->tables->ok, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        CK(cudaFuncSetAttribute(compute_cells_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCellNttSmemBytes));
+        CK(cudaMalloc(&c->d_agg, (size_t)kCellsPerExtBlob * kCellAggSlices * kFieldElementsPerCell * sizeof(Fr)));
+        CK(cudaMalloc(&c->d_coeffs, (size_t)kCellsPerExtBlob * kFieldElementsPerCell * sizeof(Fr)));
+        CK(cudaMalloc(&c->d_part, 2 * sizeof(Partial)));
+        CK(cudaEventCreateWithFlags(&c->ev_r, cudaEventDisableTiming));
+        CK(cudaEventCreateWithFlags(&c->ev_rli, cudaEventDisableTiming));
+        return KZGB200_OK;
+    }();
+    if (d_bytes) cudaFree(d_bytes);
+    if (rc == KZGB200_OK && !ok) rc = KZGB200_INVALID_SETUP;
+    if (rc != KZGB200_OK) cell_destroy(ctx);
+    return rc;
+}
+
+static int cell_capacity(kzgb200_ctx* ctx, size_t n, bool host_inputs, bool device_inputs) {
+    CellCtx* c = ctx->cells;
+    int rc = ensure_capacity(ctx, n, false);
+    if (rc) return rc;
+    if (n > c->cap) {
+        CK(regrow(c->d_meta, 3 * n + kCellsPerExtBlob + 1)); CK(regrow(c->d_ustatus, n)); CK(regrow(c->d_uc, n * 48));
+        CK(regrow(c->d_U, n)); CK(regrow(c->d_rk, n));
+        if (c->d_cells) { cudaFree(c->d_cells); c->d_cells = nullptr; }
+        if (c->d_p) { cudaFree(c->d_p); c->d_p = nullptr; }
+        c->cap = n;
+        c->slot.assign(1, 0);
+    }
+    if (host_inputs && !c->d_cells) { CK(cudaMalloc(&c->d_cells, c->cap * kBytesPerCell)); CK(cudaMalloc(&c->d_p, c->cap * 48)); }
+    if (n > c->host_cap) {
+        for (void* p : {(void*)c->h_meta, (void*)c->h_uc, (void*)c->h_c, (void*)c->h_cells, (void*)c->h_p, (void*)c->h_idx}) if (p) cudaFreeHost(p);
+        c->h_meta = nullptr; c->h_uc = c->h_c = c->h_cells = c->h_p = nullptr; c->h_idx = nullptr;
+        CK(cudaMallocHost(&c->h_meta, (3 * n + kCellsPerExtBlob + 1) * 4)); CK(cudaMallocHost(&c->h_uc, n * 48));
+        c->host_cap = n;
+    }
+    if (device_inputs && !c->h_cells) {
+        CK(cudaMallocHost(&c->h_c, c->host_cap * 48)); CK(cudaMallocHost(&c->h_cells, c->host_cap * kBytesPerCell));
+        CK(cudaMallocHost(&c->h_p, c->host_cap * 48)); CK(cudaMallocHost(&c->h_idx, c->host_cap * 8));
+    }
+    return KZGB200_OK;
+}
+
+// Host side of a cell batch: commitments deduplicated by their bytes (first-occurrence order), the cells grouped by cell index,
+// both into h_meta (see cell_scalars_kernel); returns the number of unique commitments.
+static size_t cell_plan(CellCtx* c, const uint8_t* commitments, const uint64_t* idx, size_t n) {
+    uint32_t* meta = c->h_meta;
+    uint32_t *cidx = meta + n, *order = meta + 2 * n, *start = meta + 3 * n;
+    size_t tsize = 1;
+    while (tsize < 2 * n) tsize <<= 1;
+    if (c->slot.size() < tsize) c->slot.resize(tsize);
+    std::fill(c->slot.begin(), c->slot.begin() + tsize, 0u);
+    size_t m = 0;
+    for (size_t k = 0; k < n; k++) {
+        const uint8_t* key = commitments + 48 * k;
+        uint64_t h;
+        memcpy(&h, key + 8, 8);                         // x-coordinate bytes: uniform for valid points
+        size_t s = (size_t)(h * 0x9e3779b97f4a7c15ull) & (tsize - 1);
+        for (;; s = (s + 1) & (tsize - 1)) {
+            const uint32_t u = c->slot[s];
+            if (!u) { c->slot[s] = (uint32_t)(m + 1); memcpy(c->h_uc + 48 * m, key, 48); cidx[k] = (uint32_t)m++; break; }
+            if (!memcmp(c->h_uc + 48 * (u - 1), key, 48)) { cidx[k] = u - 1; break; }
+        }
+        meta[k] = (uint32_t)idx[k];
+    }
+    for (int i = 0; i <= kCellsPerExtBlob; i++) start[i] = 0;
+    for (size_t k = 0; k < n; k++) start[meta[k] + 1]++;
+    for (int i = 0; i < kCellsPerExtBlob; i++) start[i + 1] += start[i];
+    std::vector<uint32_t> cur(start, start + kCellsPerExtBlob);
+    for (size_t k = 0; k < n; k++) order[cur[meta[k]]++] = (uint32_t)k;
+    return m;
+}
+// r = SHA-256("RCKZGCBATCH__V1_" | u64be 4096 | u64be 64 | u64be m | u64be n | unique commitments |
+//             per cell: u64be commitment index | u64be cell index | cell | proof) mod q; every byte is caller input
+static void cell_transcript(uint8_t digest[32], const uint8_t* uc, size_t m, const uint32_t* cidx, const uint64_t* idx, const uint8_t* cells,
+                            const uint8_t* proofs, size_t n) {
+    HostSha256 s;
+    host_sha256_init(&s);
+    uint8_t hdr[48] = {'R', 'C', 'K', 'Z', 'G', 'C', 'B', 'A', 'T', 'C', 'H', '_', '_', 'V', '1', '_'};
+    const uint64_t v[4] = {(uint64_t)kFieldElementsPerBlob, (uint64_t)kFieldElementsPerCell, (uint64_t)m, (uint64_t)n};
+    for (int w = 0; w < 4; w++) for (int i = 0; i < 8; i++) hdr[16 + 8 * w + i] = (uint8_t)(v[w] >> (56 - 8 * i));
+    host_sha256_update(&s, hdr, 48);
+    host_sha256_update(&s, uc, m * 48);
+    constexpr size_t kEntry = 16 + kBytesPerCell + 48, kBatch = 16;   // 2112 bytes = 33 SHA-256 blocks per cell
+    std::vector<uint8_t> buf(kEntry * kBatch);
+    for (size_t k = 0; k < n;) {
+        size_t cnt = n - k < kBatch ? n - k : kBatch;
+        for (size_t e = 0; e < cnt; e++, k++) {
+            uint8_t* p = buf.data() + kEntry * e;
+            for (int i = 0; i < 8; i++) { p[i] = (uint8_t)((uint64_t)cidx[k] >> (56 - 8 * i)); p[8 + i] = (uint8_t)(idx[k] >> (56 - 8 * i)); }
+            memcpy(p + 16, cells + k * kBytesPerCell, kBytesPerCell);
+            memcpy(p + 16 + kBytesPerCell, proofs + 48 * k, 48);
+        }
+        host_sha256_update(&s, buf.data(), kEntry * cnt);
+    }
+    host_sha256_final(&s, digest);
+}
+
+// verify_cell_kzg_proof_batch.  hc / hidx / hcells / hp: host copies (the caller's, or the pinned read-back of device inputs);
+// d_cells / d_p: the cells / proofs on the device.
+static int cell_verify_locked(kzgb200_ctx* ctx, const uint8_t* hc, const uint64_t* hidx, const uint8_t* hcells, const uint8_t* hp,
+                              const uint8_t* d_cells, const uint8_t* d_p, size_t n, int* ok, bool copy_inputs) {
+    CellCtx* c = ctx->cells;
+    for (size_t k = 0; k < n; k++) if (hidx[k] >= (uint64_t)kCellsPerExtBlob) return KZGB200_BAD_ARGS;
+    const size_t m = cell_plan(c, hc, hidx, n);
+    // the host hashes the transcript while the GPU parses
+    uint8_t digest[32];
+    std::thread hasher(cell_transcript, digest, c->h_uc, m, c->h_meta + n, hidx, hcells, hp, n);
+    const int ni = (int)n, mi = (int)m;
+    int rc = [&]() -> int {
+        for (int i = 0; i < 8; i++) ctx->ph_started[i] = false;
+        CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_parse, 0));       // a previous call's deferred subgroup checks still write status
+        CK(cudaMemsetAsync(ctx->d_status, 0, n * sizeof(uint32_t), ctx->stream));
+        CK(cudaMemsetAsync(c->d_ustatus, 0, m * sizeof(uint32_t), ctx->stream));
+        CK(cudaMemcpyAsync(c->d_meta, c->h_meta, (3 * n + kCellsPerExtBlob + 1) * 4, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(c->d_uc, c->h_uc, m * 48, cudaMemcpyHostToDevice, ctx->stream));
+        if (copy_inputs) {
+            CK(cudaMemcpyAsync(c->d_p, hp, n * 48, cudaMemcpyHostToDevice, ctx->stream));
+            CK(cudaMemcpyAsync(c->d_cells, hcells, n * kBytesPerCell, cudaMemcpyHostToDevice, ctx->stream));
+            d_cells = c->d_cells; d_p = c->d_p;
+        }
+        phase_begin(ctx, kPhParse, ctx->stream);
+        cell_points_kernel<<<(mi + 127) / 128, 128, 0, ctx->stream>>>(c->d_uc, mi, c->d_U, c->d_ustatus, kErrCommitment);
+        cell_points_kernel<<<(ni + 127) / 128, 128, 0, ctx->stream>>>(d_p, ni, ctx->d_P, ctx->d_status, kErrProof);
+        cell_check_kernel<<<(unsigned)(((size_t)n * kFieldElementsPerCell + 255) / 256), 256, 0, ctx->stream>>>(d_cells, ni, ctx->d_status);
+        cell_scalars_kernel<<<(ni + 127) / 128, 128, 0, ctx->stream>>>(c->d_meta, ni, c->d_U, c->d_ustatus, c->tables, ctx->d_z_mont, ctx->d_zy,
+                                                                        ctx->d_C, ctx->d_status);
+        phase_end(ctx, kPhParse, ctx->stream);
+        CK(cudaGetLastError());
+        return KZGB200_OK;
+    }();
+    hasher.join();
+    if (rc) return rc;
+    phase_begin(ctx, kPhTranscript, ctx->stream);
+    if ((rc = upload_r_digest(ctx, digest))) return rc;
+    phase_end(ctx, kPhTranscript, ctx->stream);
+    // RLI depends only on r: on the aux stream beside the big MSM
+    CK(cudaEventRecord(c->ev_r, ctx->stream));
+    CK(cudaStreamWaitEvent(ctx->s_aux, c->ev_r, 0));
+    cell_rpow_kernel<<<(ni + 127) / 128, 128, 0, ctx->s_aux>>>(ctx->d_r, ni, c->d_rk);
+    cell_agg_kernel<<<dim3(kCellsPerExtBlob, kCellAggSlices), kFieldElementsPerCell, 0, ctx->s_aux>>>(d_cells, c->d_meta, ni, c->d_rk, c->d_agg);
+    cell_interp_kernel<<<kCellsPerExtBlob, kFieldElementsPerCell, 0, ctx->s_aux>>>(c->d_agg, c->d_meta, ni, c->tables, c->d_coeffs);
+    cell_rli_kernel<<<1, 256, 0, ctx->s_aux>>>(c->d_coeffs, c->tables, c->d_part + 1);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(c->ev_rli, ctx->s_aux));
+    // LL and RLC + RLP: the blob batch's MSM with z_k = h_k^64, y_k = 0
+    ctx->cur_c = nullptr; ctx->cur_p = d_p; ctx->cur_n = n; ctx->subgroup_pending = false;
+    if ((rc = launch_lincomb(ctx, 0, c->d_part, false))) return rc;
+    CK(cudaStreamWaitEvent(ctx->stream, c->ev_rli, 0));
+    phase_begin(ctx, kPhFinal, ctx->stream);
+    launch_batch_final(ctx->stream, c->d_part, 2, ctx->tables, ctx->d_result, ctx->d_scratch, false, c->tables->lines29);
+    phase_end(ctx, kPhFinal, ctx->stream);
+    CK(cudaGetLastError());
+    rc = read_result(ctx, ok);
+    collect_phase_times(ctx);
+    return rc;
+}
+
+extern "C" int kzgb200_verify_cell_kzg_proof_batch(kzgb200_ctx* ctx, const uint8_t* commitments, const uint64_t* cell_indices, const uint8_t* cells,
+                                                   const uint8_t* proofs, size_t n, int* ok) {
+    if (!ctx || !ok || (n && (!commitments || !cell_indices || !cells || !proofs)) || n > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
+    if (!ctx->cells) return KZGB200_INVALID_SETUP;
+    if (n == 0) { *ok = 1; return KZGB200_OK; }
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    int rc = cell_capacity(ctx, n, true, false);
+    if (rc) return rc;
+    return cell_verify_locked(ctx, commitments, cell_indices, cells, proofs, nullptr, nullptr, n, ok, true);
+}
+
+extern "C" int kzgb200_verify_cell_kzg_proof_batch_device(kzgb200_ctx* ctx, const uint8_t* d_commitments, const uint64_t* d_cell_indices,
+                                                          const uint8_t* d_cells, const uint8_t* d_proofs, size_t n, int* ok) {
+    if (!ctx || !ok || (n && (!d_commitments || !d_cell_indices || !d_cells || !d_proofs)) || n > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
+    if (!ctx->cells) return KZGB200_INVALID_SETUP;
+    if (n == 0) { *ok = 1; return KZGB200_OK; }
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    int rc = cell_capacity(ctx, n, false, true);
+    if (rc) return rc;
+    CellCtx* c = ctx->cells;
+    // the exact transcript is a host chain over every input byte: the inputs come back to pinned memory once
+    CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_parse, 0));
+    CK(cudaMemcpyAsync(c->h_idx, d_cell_indices, n * 8, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaMemcpyAsync(c->h_c, d_commitments, n * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaMemcpyAsync(c->h_p, d_proofs, n * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaMemcpyAsync(c->h_cells, d_cells, n * kBytesPerCell, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaStreamSynchronize(ctx->s_d2h));
+    return cell_verify_locked(ctx, c->h_c, c->h_idx, c->h_cells, c->h_p, d_cells, d_proofs, n, ok, false);
+}
+
+static int compute_cells_locked(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8_t* d_out) {
+    int rc = ensure_capacity(ctx, n, false);
+    if (rc) return rc;
+    CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_parse, 0));
+    CK(cudaMemsetAsync(ctx->d_status, 0, n * sizeof(uint32_t), ctx->stream));
+    compute_cells_kernel<<<(unsigned)n, kCellNttThreads, kCellNttSmemBytes, ctx->stream>>>(d_blobs, (int)n, ctx->cells->tables, d_out, ctx->d_status);
+    status_or_kernel<<<1, 256, 0, ctx->stream>>>(ctx->d_status, (int)n, ctx->d_result);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(ctx->h_result, ctx->d_result, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return ctx->h_result[0] ? KZGB200_BAD_ARGS : KZGB200_OK;
+}
+extern "C" int kzgb200_compute_cells(kzgb200_ctx* ctx, const uint8_t* blob, uint8_t* cells_out) {
+    if (!ctx || !blob || !cells_out) return KZGB200_BAD_ARGS;
+    if (!ctx->cells) return KZGB200_INVALID_SETUP;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    int rc = ensure_capacity(ctx, 1, true);
+    if (rc) return rc;
+    CellCtx* c = ctx->cells;
+    if (!c->d_ext) CK(cudaMalloc(&c->d_ext, (size_t)kCellsPerExtBlob * kBytesPerCell));
+    CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_parse, 0));
+    CK(cudaMemcpyAsync(ctx->d_blobs, blob, kBytesPerBlob, cudaMemcpyHostToDevice, ctx->stream));
+    if ((rc = compute_cells_locked(ctx, ctx->d_blobs, 1, c->d_ext))) return rc;
+    CK(cudaMemcpyAsync(cells_out, c->d_ext, (size_t)kCellsPerExtBlob * kBytesPerCell, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return KZGB200_OK;
+}
+extern "C" int kzgb200_compute_cells_batch_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8_t* d_cells) {
+    if (!ctx || (n && (!d_blobs || !d_cells)) || n > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
+    if (!ctx->cells) return KZGB200_INVALID_SETUP;
+    if (n == 0) return KZGB200_OK;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    return compute_cells_locked(ctx, d_blobs, n, d_cells);
+}
+
+// cell workload: n_blobs polynomials of degree < `degree` (128 < degree <= 192), their 128 cells each (n_blobs x 128 x 2048
+// bytes, blob-major), commitments (n_blobs x 48) and cell proofs (n_blobs x 128 x 48); tau_powers48 = [tau^j]G1, j < degree
+extern "C" int kzgb200_harness_generate_cells(kzgb200_ctx* ctx, uint64_t seed, size_t n_blobs, int degree, const uint8_t* tau_powers48,
+                                              uint8_t* d_cells, uint8_t* d_commitments, uint8_t* d_proofs) {
+    if (!ctx || n_blobs == 0 || n_blobs > (1u << 20) || degree <= 2 * kFieldElementsPerCell || degree > kCellHarnessMaxDegree || !tau_powers48 ||
+        !d_cells || !d_commitments || !d_proofs)
+        return KZGB200_BAD_ARGS;
+    if (!ctx->cells) return KZGB200_INVALID_SETUP;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    const int n = (int)n_blobs;
+    uint8_t* d_bytes = nullptr; G1Affine* d_M = nullptr; uint32_t* d_bad = nullptr; G1 *d_terms = nullptr, *d_sums = nullptr;
+    uint32_t bad = 0;
+    int rc = [&]() -> int {
+        CK(cudaMalloc(&d_bytes, degree * 48)); CK(cudaMalloc(&d_M, degree * sizeof(G1Affine))); CK(cudaMalloc(&d_bad, 4));
+        CK(cudaMalloc(&d_terms, (size_t)n * 6 * 64 * sizeof(G1))); CK(cudaMalloc(&d_sums, (size_t)n * 6 * sizeof(G1)));
+        CK(cudaMemsetAsync(d_bad, 0, 4, ctx->stream));
+        CK(cudaMemcpyAsync(d_bytes, tau_powers48, degree * 48, cudaMemcpyHostToDevice, ctx->stream));
+        harness_parse_points_kernel<<<(degree + 31) / 32, 32, 0, ctx->stream>>>(d_bytes, degree, d_M, d_bad);
+        cell_harness_eval_kernel<<<dim3(kCellsPerExtBlob * kFieldElementsPerCell / 128, n), 128, 0, ctx->stream>>>(seed, n, degree, ctx->cells->tables, d_cells);
+        cell_harness_terms_kernel<<<(n * 6 * 64 + 127) / 128, 128, 0, ctx->stream>>>(seed, n, degree, d_M, d_terms);
+        cell_harness_sums_kernel<<<(n * 6 + 127) / 128, 128, 0, ctx->stream>>>(n, d_terms, d_sums);
+        cell_harness_points_kernel<<<(n * (kCellsPerExtBlob + 1) + 127) / 128, 128, 0, ctx->stream>>>(n, d_sums, ctx->cells->tables, d_commitments, d_proofs);
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        return KZGB200_OK;
+    }();
+    for (void* p : {(void*)d_bytes, (void*)d_M, (void*)d_bad, (void*)d_terms, (void*)d_sums}) if (p) cudaFree(p);
+    if (rc) return rc;
+    return bad ? KZGB200_BAD_ARGS : KZGB200_OK;
+}

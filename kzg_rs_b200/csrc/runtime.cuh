@@ -44,6 +44,25 @@ struct CopyPool {
     bool grab(size_t* off, size_t* len);
 };
 
+// State of the cell path (EIP-7594), created by kzgb200_load_cell_setup.  Workspace sized for `cap` cells / `blob_cap` blobs.
+struct CellCtx {
+    CellTables* tables = nullptr;
+    size_t cap = 0, blob_cap = 0;
+    uint8_t *d_cells = nullptr, *d_p = nullptr, *d_uc = nullptr;   // staging of host cells / proofs, unique commitment bytes
+    uint32_t *d_meta = nullptr, *d_ustatus = nullptr;              // see cell_scalars_kernel
+    G1Affine* d_U = nullptr;                                       // unique commitments
+    Fr *d_rk = nullptr, *d_agg = nullptr, *d_coeffs = nullptr;
+    Partial* d_part = nullptr;                                     // [0] = LL / RLC + RLP (launch_lincomb), [1] = (O, -RLI)
+    uint8_t* d_ext = nullptr;                                      // compute_cells output of a host blob (128 cells)
+    // pinned host side: metadata, unique commitments, and (device-resident inputs) the copies the transcript is hashed from
+    size_t host_cap = 0;
+    uint32_t* h_meta = nullptr;
+    uint8_t *h_uc = nullptr, *h_c = nullptr, *h_cells = nullptr, *h_p = nullptr;
+    uint64_t* h_idx = nullptr;
+    std::vector<uint32_t> slot;                                    // open-addressing table of the commitment deduplication
+    cudaEvent_t ev_r = nullptr, ev_rli = nullptr;
+};
+
 }  // namespace kzgb200
 
 struct kzgb200_ctx {
@@ -119,6 +138,7 @@ struct kzgb200_ctx {
     cudaEvent_t ev_s[8] = {nullptr}, ev_e[8] = {nullptr};
     bool ph_started[8] = {false};
     float phase_ms[8] = {0};
+    kzgb200::CellCtx* cells = nullptr;   // EIP-7594 cell path (kzgb200_load_cell_setup)
     std::mutex lock;
     char err[256] = {0};
 };
