@@ -27,6 +27,7 @@ def lib():
         _LIB.kzgco_init.argtypes = [C.c_char_p, C.c_size_t]
         _LIB.kzgco_compute_cells.argtypes = [C.c_char_p, C.c_char_p]
         _LIB.kzgco_compute_cell_kzg_proof.argtypes = [C.c_char_p, C.c_int, C.c_char_p]
+        _LIB.kzgco_recover_cells.argtypes = [C.POINTER(C.c_uint64), C.c_char_p, C.c_size_t, C.c_char_p]
         _LIB.kzgco_verify_cell_kzg_proof_batch.argtypes = [C.c_char_p, C.POINTER(C.c_uint64), C.c_char_p, C.c_char_p, C.c_size_t,
                                                            C.POINTER(C.c_int), C.c_char_p]
         use_setup(None)
@@ -54,6 +55,18 @@ def compute_cell_kzg_proof(blob, k):
     out = C.create_string_buffer(48)
     rc = lib().kzgco_compute_cell_kzg_proof(bytes(blob), k, out)
     return None if rc else out.raw
+
+
+def recover_cells(cell_indices, cells):
+    """recover_cells_and_kzg_proofs' cells: the 128 cells (bytes) recovered from the given ones, or None (BadArgs)."""
+    n = len(cell_indices)
+    assert len(cells) == n
+    if any(len(x) != BYTES_PER_CELL for x in cells) or any(not 0 <= i < 1 << 64 for i in cell_indices):
+        return None
+    out = C.create_string_buffer(BYTES_PER_CELL * CELLS_PER_EXT_BLOB)
+    idx = (C.c_uint64 * max(n, 1))(*cell_indices)
+    rc = lib().kzgco_recover_cells(idx, b"".join(cells), n, out)
+    return None if rc else [out.raw[BYTES_PER_CELL * k:BYTES_PER_CELL * (k + 1)] for k in range(CELLS_PER_EXT_BLOB)]
 
 
 def verify_cell_kzg_proof_batch(commitments, cell_indices, cells, proofs, want_r=False):

@@ -7,6 +7,7 @@
  * Setup: the "KZGS" container (kzg_rs_b200/data/mainnet_setup.bin, tests/golden/custom_setup.bin): 4096 Lagrange G1 points
  * (bit-reversal permuted on load, as the blob oracle does) and at least 65 G2 points (g2[0] = G2, g2[64] = [tau^64]G2).
  * [tau^j]G1 for j < 64 (the interpolation commitment RLI) are derived from the Lagrange points on first use.
+ * kzgco_recover_cells restates recover_polynomialcoeff step by step, so that inconsistent cells give the spec's bytes too.
  */
 #include <pthread.h>
 #include <stdio.h>
@@ -286,5 +287,63 @@ int kzgco_verify_cell_kzg_proof_batch(const uint8_t *cb, const uint64_t *cell_in
         free(s_ll); free(s_rlp); free(s_rlc); free(w_c); free(agg);
     }
     free(vals); free(P); free(U); free(ci); free(first);
+    return rc;
+}
+
+/* recover_cells_and_kzg_proofs, cells only: the spec's argument checks, recover_polynomialcoeff literally (zeros at the missing
+ * cells, the vanishing polynomial Z(X) = z(X^64), (E Z) on the 8192-point domain, inverse transform, coset transforms with the shift
+ * PRIMITIVE_ROOT_OF_UNITY = 7, division by Z on the coset, first 4096 coefficients), then the cells of the recovered polynomial.
+ * (Its proofs are those of the blob formed by the recovered cells 0..63: kzgco_compute_cell_kzg_proof.) */
+static void coset_shift(fr *a, int n, const fr *factor) {
+    fr x; fr_set_one(&x);
+    for (int i = 0; i < n; i++) { fr_mul(&a[i], &a[i], &x); fr_mul(&x, &x, factor); }
+}
+int kzgco_recover_cells(const uint64_t *indices, const uint8_t *cells, size_t n, uint8_t *cells_out /* 128 x 2048 */) {
+    if (!S.ready) return KZG_BADSETUP;
+    if (n < CELLS_PER_EXT_BLOB / 2 || n > CELLS_PER_EXT_BLOB) return KZG_BADARGS;
+    int present[CELLS_PER_EXT_BLOB] = {0};
+    for (size_t j = 0; j < n; j++) {
+        if (indices[j] >= CELLS_PER_EXT_BLOB || present[indices[j]]) return KZG_BADARGS;
+        present[indices[j]] = 1;
+    }
+    fr *rbo = (fr *)calloc(N_EXT, sizeof(fr)), *E = (fr *)malloc(N_EXT * sizeof(fr)), *Z = (fr *)calloc(N_EXT, sizeof(fr));
+    fr *Zev = (fr *)malloc(N_EXT * sizeof(fr)), *Zcos = (fr *)malloc(N_EXT * sizeof(fr));
+    int rc = KZG_OK;
+    /* extended_evaluation_rbo, then bit_reversal_permutation */
+    for (size_t j = 0; j < n && !rc; j++)
+        for (int i = 0; i < FE_PER_CELL && !rc; i++) rc = safe_scalar_from_bytes(&rbo[indices[j] * FE_PER_CELL + i], cells + j * BYTES_PER_CELL + 32 * i);
+    if (!rc) {
+        for (int i = 0; i < N_EXT; i++) E[i] = rbo[bitrev((uint32_t)i, 13)];
+        /* construct_vanishing_polynomial: prod over the missing k of (Y - omega128^rev7(k)), spread to X^(64 i) */
+        fr w128, shortz[CELLS_PER_EXT_BLOB + 1], root, t;
+        int deg = 0;
+        omega_pow(&w128, &S.omega8192, FE_PER_CELL);
+        fr_set_one(&shortz[0]);
+        for (int k = 0; k < CELLS_PER_EXT_BLOB; k++) {
+            if (present[k]) continue;
+            omega_pow(&root, &w128, bitrev((uint32_t)k, 7));
+            fr_set_zero(&shortz[deg + 1]);
+            for (int i = deg + 1; i >= 1; i--) { fr_mul(&t, &shortz[i], &root); fr_sub(&shortz[i], &shortz[i - 1], &t); }   /* p * (X - root) */
+            fr_mul(&t, &shortz[0], &root); fr_set_zero(&shortz[0]); fr_sub(&shortz[0], &shortz[0], &t);
+            deg++;
+        }
+        for (int i = 0; i <= deg; i++) Z[i * FE_PER_CELL] = shortz[i];
+        memcpy(Zev, Z, N_EXT * sizeof(fr));
+        fr_dft(Zev, N_EXT, &S.omega8192);
+        for (int i = 0; i < N_EXT; i++) fr_mul(&E[i], &E[i], &Zev[i]);          /* (E Z) on the domain */
+        fr_idft(E, N_EXT, &S.omega8192);                                        /* (P Z) coefficients */
+        fr seven, seven_inv;
+        fr_from_u64(&seven, 7); fr_inv(&seven_inv, &seven);
+        coset_shift(E, N_EXT, &seven); fr_dft(E, N_EXT, &S.omega8192);        /* (P Z) on the coset */
+        memcpy(Zcos, Z, N_EXT * sizeof(fr));
+        coset_shift(Zcos, N_EXT, &seven); fr_dft(Zcos, N_EXT, &S.omega8192);  /* Z on the coset */
+        for (int i = 0; i < N_EXT; i++) { fr_inv(&t, &Zcos[i]); fr_mul(&E[i], &E[i], &t); }
+        fr_idft(E, N_EXT, &S.omega8192); coset_shift(E, N_EXT, &seven_inv);   /* P coefficients */
+        /* compute_cells of the first 4096 coefficients */
+        for (int i = N_FE; i < N_EXT; i++) fr_set_zero(&E[i]);
+        fr_dft(E, N_EXT, &S.omega8192);
+        for (int i = 0; i < N_EXT; i++) fr_to_bytes_be(cells_out + 32 * (size_t)i, &E[bitrev((uint32_t)i, 13)]);
+    }
+    free(rbo); free(E); free(Z); free(Zev); free(Zcos);
     return rc;
 }

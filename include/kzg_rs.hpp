@@ -5,7 +5,8 @@
 //   kzg_rs::KzgSettings::load_trusted_setup_file                                                src/trusted_setup.rs:94-98
 //   kzg_rs::Blob / Bytes32 / Bytes48 (from_slice length check, as_slice)                        src/dtypes.rs:7-46
 //   kzg_rs::KzgError                                                                            src/enums.rs:6-18
-// plus EIP-7594 cells: kzg_rs::Cell, KzgProof::verify_cell_kzg_proof_batch, kzg_rs::compute_cells (c-kzg-4844 / rust-kzg names).
+// plus EIP-7594 cells: kzg_rs::Cell, KzgProof::verify_cell_kzg_proof_batch, kzg_rs::compute_cells, kzg_rs::compute_cells_and_kzg_proofs,
+// kzg_rs::recover_cells_and_kzg_proofs (c-kzg-4844 / rust-kzg names).
 // Result<bool, KzgError> is kzg_rs::Result<bool>: either a value or an error.
 #pragma once
 #include <array>
@@ -154,6 +155,33 @@ inline Result<std::vector<Cell>> compute_cells(const Blob& blob, const KzgSettin
     int rc = kzgb200_compute_cells(kzg_settings.ctx(), blob.as_slice(), reinterpret_cast<uint8_t*>(cells.data()));
     if (rc) return detail::to_result(rc, 0).unwrap_err();
     return cells;
+}
+
+// EIP-7594 compute_cells_and_kzg_proofs / recover_cells_and_kzg_proofs (FK20 on the GPU).  Both need the proof setup once per
+// context: load_cell_proof_setup with the setup's 4096 Lagrange G1 points (file order), after load_cell_setup.
+inline Result<bool> load_cell_proof_setup(const KzgSettings& kzg_settings, const uint8_t* g1_lagrange48, size_t n_points) {
+    int rc = kzgb200_load_cell_proof_setup(kzg_settings.ctx(), g1_lagrange48, n_points);
+    if (rc) return KzgError{rc == KZGB200_INVALID_SETUP ? KzgError::InvalidTrustedSetup : KzgError::InternalError, "kzgb200_load_cell_proof_setup failed"};
+    return true;
+}
+struct CellsAndProofs { std::vector<Cell> cells; std::vector<Bytes48> proofs; };
+inline Result<CellsAndProofs> compute_cells_and_kzg_proofs(const Blob& blob, const KzgSettings& kzg_settings) {
+    CellsAndProofs out{std::vector<Cell>(CELLS_PER_EXT_BLOB), std::vector<Bytes48>(CELLS_PER_EXT_BLOB)};
+    int rc = kzgb200_compute_cells_and_kzg_proofs(kzg_settings.ctx(), blob.as_slice(), reinterpret_cast<uint8_t*>(out.cells.data()),
+                                                  reinterpret_cast<uint8_t*>(out.proofs.data()));
+    if (rc) return detail::to_result(rc, 0).unwrap_err();
+    return out;
+}
+// 64..128 cells of a blob, indices in any order -> all 128 cells and proofs; BadArgs for the spec's failed assertions
+inline Result<CellsAndProofs> recover_cells_and_kzg_proofs(const std::vector<uint64_t>& cell_indices, const std::vector<Cell>& cells,
+                                                          const KzgSettings& kzg_settings) {
+    if (cells.size() != cell_indices.size()) return KzgError{KzgError::InvalidBytesLength, "Invalid cells / cell indices length"};
+    CellsAndProofs out{std::vector<Cell>(CELLS_PER_EXT_BLOB), std::vector<Bytes48>(CELLS_PER_EXT_BLOB)};
+    int rc = kzgb200_recover_cells_and_kzg_proofs(kzg_settings.ctx(), cell_indices.data(), reinterpret_cast<const uint8_t*>(cells.data()),
+                                                  cells.size(), reinterpret_cast<uint8_t*>(out.cells.data()),
+                                                  reinterpret_cast<uint8_t*>(out.proofs.data()));
+    if (rc) return detail::to_result(rc, 0).unwrap_err();
+    return out;
 }
 
 // Streaming front-end (include/kzgb200.h, kzgb200_pipeline_*): `depth` verify_blob_kzg_proof_batch calls in flight on one GPU.

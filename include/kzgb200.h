@@ -206,6 +206,35 @@ int kzgb200_compute_cells_batch_device(kzgb200_ctx* ctx, const uint8_t* d_blobs,
 int kzgb200_harness_generate_cells(kzgb200_ctx* ctx, uint64_t seed, size_t n_blobs, int degree, const uint8_t* tau_powers48,
                                    uint8_t* d_cells, uint8_t* d_commitments, uint8_t* d_proofs);
 
+/* ---- EIP-7594 cell proofs and recovery (FK20; consensus-specs Fulu compute_cells_and_kzg_proofs / recover_cells_and_kzg_proofs) --
+ * kzgb200_load_cell_proof_setup: the setup's 4096 Lagrange G1 points (host, 4096 x 48 compressed, file order: point j pairs with
+ *   omega4096^j; KzgSettings.g1_lagrange_bytes).  n_points must be 4096 and the cell setup must be loaded, else INVALID_SETUP.  Derives
+ *   every [tau^m]G1 (m < 4096) on the device (a 4096-point DFT over G1), checks that the first 64 are the points given to
+ *   kzgb200_load_cell_setup (INVALID_SETUP otherwise), and builds the FK20 tables.  Device memory: 3.34 GB of window tables
+ *   (8192 bases x 16 windows x 255 affine points), 0.4 MB of monomial points, 0.4 MB of scalar tables; a workspace of ~0.9 MB per
+ *   blob (at most 512 blobs at a time) is allocated by the first call that needs it.  Once per context (later calls return OK);
+ *   the blob and cell verification paths keep working.  Every entry point below returns INVALID_SETUP before it.
+ * kzgb200_cell_proof_monomial: the derived [tau^m]G1, m < n_points (<= 4096; else BAD_ARGS), compressed, to out48 (host).
+ * kzgb200_compute_cells_and_kzg_proofs: one host blob -> its 128 cells (cells_out, 128 x 2048) and their proofs (proofs_out,
+ *   128 x 48, compressed; the identity is 0xc0 then 47 zero bytes), host pointers, none nullable.
+ * kzgb200_compute_cells_and_kzg_proofs_batch_device: n device blobs -> n x 128 cells and n x 128 proofs (device, blob-major, proofs
+ *   in the order of the cells); n == 0 -> OK.  A non-canonical blob element -> BAD_ARGS for the whole call (outputs undefined).
+ * kzgb200_recover_cells_and_kzg_proofs: all 128 cells and proofs of a blob from n_cells of its cells (host: cell_indices n_cells x u64,
+ *   cells n_cells x 2048 in the same order, any order of indices).  BAD_ARGS unless 64 <= n_cells <= 128, every index < 128, no index
+ *   twice and every element canonical.  Inconsistent cells are not detected (as in the spec): the result is the spec's bytes.
+ * kzgb200_recover_cells_and_kzg_proofs_batch_device: n_blobs blobs that share one index set (host cell_indices, n_cells); d_cells =
+ *   n_blobs x n_cells x 2048 (device, blob-major, each blob's cells in index-set order); outputs as the batch compute call.
+ * With kzgb200_set_profiling on, kzgb200_get_phase_ms reports for these calls {coefficients (with compute_cells), fixed-base products
+ * (with the scalar DFTs), G1 transforms (with compression), recovery transforms, 0, 0, 0, 0}, first start to last end. */
+int kzgb200_load_cell_proof_setup(kzgb200_ctx* ctx, const uint8_t* g1_lagrange48, size_t n_points);
+int kzgb200_cell_proof_monomial(kzgb200_ctx* ctx, uint8_t* out48, size_t n_points);
+int kzgb200_compute_cells_and_kzg_proofs(kzgb200_ctx* ctx, const uint8_t* blob, uint8_t* cells_out, uint8_t* proofs_out);
+int kzgb200_compute_cells_and_kzg_proofs_batch_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8_t* d_cells, uint8_t* d_proofs);
+int kzgb200_recover_cells_and_kzg_proofs(kzgb200_ctx* ctx, const uint64_t* cell_indices, const uint8_t* cells, size_t n_cells,
+                                         uint8_t* cells_out, uint8_t* proofs_out);
+int kzgb200_recover_cells_and_kzg_proofs_batch_device(kzgb200_ctx* ctx, const uint64_t* cell_indices, size_t n_cells, const uint8_t* d_cells,
+                                                      size_t n_blobs, uint8_t* d_cells_out, uint8_t* d_proofs_out);
+
 /* per-phase device timing of batch calls (CUDA event pairs on the stream each phase runs on).  out8 = milliseconds of
  * {G1 decompression, challenge, evaluate, transcript r (exposed part: last chunk copy + host hash + upload), lincomb terms, reduce,
  * final pairing, deferred subgroup checks (run beside the last three)} of the last call. */

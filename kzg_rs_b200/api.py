@@ -119,6 +119,12 @@ class Library:
         d.kzgb200_compute_cells.argtypes = [p, C.c_char_p, p]
         d.kzgb200_compute_cells_batch_device.argtypes = [p, p, sz, p]
         d.kzgb200_harness_generate_cells.argtypes = [p, C.c_uint64, sz, C.c_int, C.c_char_p, p, p, p]
+        d.kzgb200_load_cell_proof_setup.argtypes = [p, C.c_char_p, sz]
+        d.kzgb200_cell_proof_monomial.argtypes = [p, p, sz]
+        d.kzgb200_compute_cells_and_kzg_proofs.argtypes = [p, C.c_char_p, p, p]
+        d.kzgb200_compute_cells_and_kzg_proofs_batch_device.argtypes = [p, p, sz, p, p]
+        d.kzgb200_recover_cells_and_kzg_proofs.argtypes = [p, p, p, sz, p, p]
+        d.kzgb200_recover_cells_and_kzg_proofs_batch_device.argtypes = [p, p, sz, p, sz, p, p]
 
 
 def _raise(rc, ctx=None, msg=None):
@@ -192,6 +198,7 @@ class KzgSettings:
         self.g1_monomial_bytes = g1_monomial_bytes
         self._ctx = {}
         self._cells = set()
+        self._proofs = set()
         self._lock = threading.Lock()
 
     @classmethod
@@ -263,12 +270,27 @@ class KzgSettings:
                 self._cells.add(device)
         return ctx
 
+    def cell_proof_context(self, device=0):
+        """The cell context with the proof setup loaded as well (compute / recover cells and proofs): every [tau^j]G1, j < 4096,
+        derived on the GPU from g1_lagrange_bytes, and the FK20 tables (3.3 GB of device memory)."""
+        ctx = self.cell_context(device)
+        with self._lock:
+            if device not in self._proofs:
+                if len(self.g1_lagrange_bytes) != 4096 * 48:
+                    raise KzgError("InvalidTrustedSetup", "cell proofs need the setup's 4096 Lagrange G1 points")
+                rc = Library.get().dll.kzgb200_load_cell_proof_setup(ctx, self.g1_lagrange_bytes, 4096)
+                if rc:
+                    _raise(rc, ctx)
+                self._proofs.add(device)
+        return ctx
+
     def close(self):
         with self._lock:
             for h in self._ctx.values():
                 Library.get().dll.kzgb200_destroy(h)
             self._ctx = {}
             self._cells = set()
+            self._proofs = set()
 
 
 def mainnet_g1_monomial():
@@ -401,6 +423,44 @@ def compute_cells(blob, kzg_settings, device=0):
         _raise(rc, ctx, "Failed to parse blob" if rc == 1 else None)
     raw = out.raw
     return [raw[BYTES_PER_CELL * k:BYTES_PER_CELL * (k + 1)] for k in range(CELLS_PER_EXT_BLOB)]
+
+
+def _cells_and_proofs(raw_cells, raw_proofs):
+    return ([raw_cells[BYTES_PER_CELL * k:BYTES_PER_CELL * (k + 1)] for k in range(CELLS_PER_EXT_BLOB)],
+            [raw_proofs[BYTES_PER_PROOF * k:BYTES_PER_PROOF * (k + 1)] for k in range(CELLS_PER_EXT_BLOB)])
+
+
+def compute_cells_and_kzg_proofs(blob, kzg_settings, device=0):
+    """EIP-7594 compute_cells_and_kzg_proofs: (cells, proofs), 128 of each (2048 / 48 bytes), the proofs by FK20 on the GPU;
+    BadArgs on a non-canonical element."""
+    b = _b(blob, BYTES_PER_BLOB, "blob")
+    ctx = kzg_settings.cell_proof_context(device)
+    cells = C.create_string_buffer(BYTES_PER_CELL * CELLS_PER_EXT_BLOB)
+    proofs = C.create_string_buffer(BYTES_PER_PROOF * CELLS_PER_EXT_BLOB)
+    rc = Library.get().dll.kzgb200_compute_cells_and_kzg_proofs(ctx, b, cells, proofs)
+    if rc:
+        _raise(rc, ctx, "Failed to parse blob" if rc == 1 else None)
+    return _cells_and_proofs(cells.raw, proofs.raw)
+
+
+def recover_cells_and_kzg_proofs(cell_indices, cells, kzg_settings, device=0):
+    """EIP-7594 recover_cells_and_kzg_proofs: all 128 (cells, proofs) of a blob from 64 or more of its cells, in any order.
+    Mismatched lengths -> KzgError(InvalidBytesLength); fewer than 64 or more than 128 cells, an index >= 128, a repeated index or a
+    non-canonical element -> KzgError(BadArgs)."""
+    n = len(cell_indices)
+    if len(cells) != n:
+        raise KzgError("InvalidBytesLength", "Invalid cells / cell indices length")
+    ce = b"".join(_b(x, BYTES_PER_CELL, "cell") for x in cells)
+    if any(not 0 <= int(i) < 1 << 64 for i in cell_indices):
+        raise KzgError("BadArgs", "Invalid cell index")
+    idx = (C.c_uint64 * max(n, 1))(*[int(i) for i in cell_indices])
+    ctx = kzg_settings.cell_proof_context(device)
+    out_cells = C.create_string_buffer(BYTES_PER_CELL * CELLS_PER_EXT_BLOB)
+    out_proofs = C.create_string_buffer(BYTES_PER_PROOF * CELLS_PER_EXT_BLOB)
+    rc = Library.get().dll.kzgb200_recover_cells_and_kzg_proofs(ctx, C.cast(idx, C.c_void_p), _ptr(ce), n, out_cells, out_proofs)
+    if rc:
+        _raise(rc, ctx, "Invalid cell indices / cells" if rc == 1 else None)
+    return _cells_and_proofs(out_cells.raw, out_proofs.raw)
 
 
 def compute_challenge(blob, commitment_bytes, kzg_settings, device=0):

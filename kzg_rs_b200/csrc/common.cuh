@@ -117,6 +117,19 @@ struct CellTables {
     vliw29::LineCoeffs29 lines29[kMillerSteps];    // [tau^64]G2 for pairing_check_kernel
     uint32_t ok;
 };
+// Cell proofs (kzgb200_load_cell_proof_setup, k_cell_proofs.cu): FK20 over the fixed bases W_b[f] = DFT_128(w_b)[f] (b < 64,
+// f < 128), each with a GLV window table tab[f * 64 + b][w][d - 1] = [d * 256^w] W_b[f] (w < 16, d = 1..255), and the scalar tables
+// of the 8192-point recovery transforms.
+constexpr int kFk20Bases = kFieldElementsPerCell * kCellsPerExtBlob;   // 8192
+constexpr int kFk20Windows = 16, kFk20Entries = 255;
+constexpr size_t kFk20TablePoints = (size_t)kFk20Bases * kFk20Windows * kFk20Entries;
+constexpr int kExtElements = 2 * kFieldElementsPerBlob;                  // 8192
+struct ProofTables {
+    Fr w8192[kFieldElementsPerBlob], w8192_inv[kFieldElementsPerBlob];   // omega8192^(+-i)
+    Fr pow7[kExtElements];                  // 7^i / 8192: the spec's coset shift (PRIMITIVE_ROOT_OF_UNITY) with the inverse 1/n
+    Fr pow7_inv[kFieldElementsPerBlob];     // 7^-i / 8192
+    Fr s7_64;                               // 7^64
+};
 // ---- kernels (k_*.cu) ----------------------------------------------------------------------------------------
 __global__ void setup_tables_kernel(DeviceTables* T, const uint8_t* g2_points);
 __global__ void setup_lines29_kernel(DeviceTables* T);
@@ -196,6 +209,28 @@ __global__ void cell_setup_points_kernel(CellTables* T, const uint8_t* __restric
 __global__ void cell_setup_lines29_kernel(CellTables* T);
 __global__ void compute_cells_kernel(const uint8_t* __restrict__ blobs, int n, const CellTables* __restrict__ T, uint8_t* __restrict__ cells,
                                      uint32_t* __restrict__ status);
+__global__ void compute_cells_coeffs_kernel(const uint8_t* __restrict__ blobs, int n, const CellTables* __restrict__ T, uint8_t* __restrict__ cells,
+                                            uint32_t* __restrict__ status, Fr* __restrict__ coeffs);
+// cell proofs / recovery (k_cell_proofs.cu)
+__global__ void proof_setup_kernel(ProofTables* P);
+__global__ void mono_load_kernel(const uint8_t* __restrict__ lag48, G1* __restrict__ a, uint32_t* __restrict__ bad);
+__global__ void mono_level_kernel(G1* __restrict__ a, int len, const CellTables* __restrict__ T);
+__global__ void mono_finish_kernel(const G1* __restrict__ a, const CellTables* __restrict__ T, G1Affine* __restrict__ mono, uint32_t* __restrict__ bad);
+__global__ void mono_compress_kernel(const G1Affine* __restrict__ mono, int n, uint8_t* __restrict__ out48);
+__global__ void fk20_w_kernel(const G1Affine* __restrict__ mono, const CellTables* __restrict__ T, G1Affine* __restrict__ W);
+__global__ void fk20_table_kernel(const G1Affine* __restrict__ W, G1Affine* __restrict__ tab);
+__global__ void fk20_scalars_kernel(const Fr* __restrict__ coeffs, const CellTables* __restrict__ T, Fr* __restrict__ U);
+__global__ void fk20_products_kernel(const Fr* __restrict__ U, const G1Affine* __restrict__ tab, G1* __restrict__ V);
+__global__ void fk20_proofs_kernel(const G1* __restrict__ V, const CellTables* __restrict__ T, uint8_t* __restrict__ proofs);
+__global__ void recover_z_kernel(const uint32_t* __restrict__ missing, int n_missing, const CellTables* __restrict__ T, const ProofTables* __restrict__ P,
+                                 Fr* __restrict__ zvals);
+__global__ void recover_load_kernel(const uint8_t* __restrict__ cells, int n_cells, const int* __restrict__ pos, const Fr* __restrict__ zvals, int nb,
+                                    Fr* __restrict__ A, uint32_t* __restrict__ status);
+__global__ void recover_ntt_inv_kernel(Fr* __restrict__ A, const CellTables* __restrict__ T);
+__global__ void recover_ntt_div_kernel(Fr* __restrict__ A, const CellTables* __restrict__ T, const Fr* __restrict__ zvals);
+__global__ void recover_mid_kernel(Fr* __restrict__ A, const ProofTables* __restrict__ P, int nb);
+__global__ void recover_final_kernel(const Fr* __restrict__ A, const ProofTables* __restrict__ P, int nb, Fr* __restrict__ coeffs);
+__global__ void recover_blob_kernel(const Fr* __restrict__ coeffs, const CellTables* __restrict__ T, uint8_t* __restrict__ blobs);
 __global__ void cell_points_kernel(const uint8_t* __restrict__ bytes, int count, G1Affine* __restrict__ out, uint32_t* __restrict__ status, uint32_t flag);
 __global__ void cell_check_kernel(const uint8_t* __restrict__ cells, int n, uint32_t* __restrict__ status);
 // meta = [cell index (n) | unique-commitment index (n) | cells ordered by cell index (n) | start of each index in that order (129)]

@@ -82,8 +82,11 @@ __global__ void cell_setup_lines29_kernel(CellTables* T) {
 // in bit-reversed order, so a decimation-in-time inverse transform gives the coefficients in natural order; coefficient m is
 // scaled by omega8192^m / 4096 (the odd coset, and the inverse transform's 1/n); a decimation-in-frequency forward transform
 // then leaves p(omega8192 * omega4096^rev12(i)) at position i -- extended element 4096 + i -- with no explicit permutation.
-__global__ void __launch_bounds__(kCellNttThreads) compute_cells_kernel(const uint8_t* __restrict__ blobs, int n, const CellTables* __restrict__ T,
-                                                                     uint8_t* __restrict__ cells, uint32_t* __restrict__ status) {
+// kCoeffs: also write the inverse transform's output -- 4096 x the blob's coefficients, natural order, Montgomery -- to coeffs
+// (the FK20 proof path, k_cell_proofs.cu).
+template <bool kCoeffs>
+__device__ __forceinline__ void compute_cells_body(const uint8_t* __restrict__ blobs, int n, const CellTables* __restrict__ T,
+                                                   uint8_t* __restrict__ cells, uint32_t* __restrict__ status, Fr* __restrict__ coeffs) {
     extern __shared__ __align__(16) unsigned char dyn_smem[];
     Fr* a = reinterpret_cast<Fr*>(dyn_smem);
     const int blob = blockIdx.x, t = threadIdx.x;
@@ -108,6 +111,7 @@ __global__ void __launch_bounds__(kCellNttThreads) compute_cells_kernel(const ui
         }
         __syncthreads();
     }
+    if (kCoeffs) for (int i = t; i < kFieldElementsPerBlob; i += kCellNttThreads) coeffs[(size_t)blob * kFieldElementsPerBlob + i] = a[i];
     for (int i = t; i < kFieldElementsPerBlob; i += kCellNttThreads) a[i] = a[i].mul_inl(T->coset[i]);
     __syncthreads();
     for (int len = kFieldElementsPerBlob; len >= 2; len >>= 1) {           // forward DIF, natural in, bit-reversed out
@@ -121,6 +125,14 @@ __global__ void __launch_bounds__(kCellNttThreads) compute_cells_kernel(const ui
     }
     uint8_t* odd = cells + ((size_t)blob * kCellsPerExtBlob + kCellsPerExtBlob / 2) * kBytesPerCell;
     for (int i = t; i < kFieldElementsPerBlob; i += kCellNttThreads) store_fe_be(odd + 32 * (size_t)i, a[i]);
+}
+__global__ void __launch_bounds__(kCellNttThreads) compute_cells_kernel(const uint8_t* __restrict__ blobs, int n, const CellTables* __restrict__ T,
+                                                                     uint8_t* __restrict__ cells, uint32_t* __restrict__ status) {
+    compute_cells_body<false>(blobs, n, T, cells, status, nullptr);
+}
+__global__ void __launch_bounds__(kCellNttThreads) compute_cells_coeffs_kernel(const uint8_t* __restrict__ blobs, int n, const CellTables* __restrict__ T,
+                                                                            uint8_t* __restrict__ cells, uint32_t* __restrict__ status, Fr* __restrict__ coeffs) {
+    compute_cells_body<true>(blobs, n, T, cells, status, coeffs);
 }
 
 // ---- verify_cell_kzg_proof_batch --------------------------------------------------------------------------------------

@@ -976,6 +976,12 @@ extern "C" void* kzgb200_alloc_pinned(size_t bytes) {
 extern "C" void kzgb200_free_pinned(void* p) { if (p) cudaFreeHost(p); }
 
 // ---- EIP-7594 cells (k_cells.cu; consensus-specs Fulu polynomial-commitments-sampling.md) ---------------------------------
+static void proof_destroy(CellCtx* c) {
+    void* d[] = {c->ptables, c->d_mono, c->d_fk_tab, c->d_pcoef, c->d_fkU, c->d_A, c->d_V, c->d_rblobs, c->d_rin, c->d_pout, c->d_pos, c->d_missing, c->d_z};
+    for (void* p : d) if (p) cudaFree(p);
+    c->ptables = nullptr; c->d_mono = c->d_fk_tab = nullptr; c->d_pcoef = c->d_fkU = c->d_A = c->d_z = nullptr; c->d_V = nullptr;
+    c->d_rblobs = c->d_rin = c->d_pout = nullptr; c->d_pos = nullptr; c->d_missing = nullptr; c->proof_cap = 0;
+}
 static void cell_destroy(kzgb200_ctx* ctx) {
     CellCtx* c = ctx->cells;
     if (!c) return;
@@ -984,6 +990,7 @@ static void cell_destroy(kzgb200_ctx* ctx) {
     void* h[] = {c->h_meta, c->h_uc, c->h_c, c->h_cells, c->h_p, c->h_idx};
     for (void* p : h) if (p) cudaFreeHost(p);
     for (cudaEvent_t e : {c->ev_r, c->ev_rli}) if (e) cudaEventDestroy(e);
+    proof_destroy(c);
     delete c;
     ctx->cells = nullptr;
 }
@@ -1265,4 +1272,229 @@ extern "C" int kzgb200_harness_generate_cells(kzgb200_ctx* ctx, uint64_t seed, s
     for (void* p : {(void*)d_bytes, (void*)d_M, (void*)d_bad, (void*)d_terms, (void*)d_sums}) if (p) cudaFree(p);
     if (rc) return rc;
     return bad ? KZGB200_BAD_ARGS : KZGB200_OK;
+}
+
+// ---- EIP-7594 cell proofs and recovery (k_cell_proofs.cu) ---------------------------------------------------------------
+// FK20 tables: 8192 bases x 16 windows x 255 affine points (3.34 GB); monomial points 4096 x 100 bytes; scalar tables 416 KiB.
+constexpr size_t kProofChunk = 512;          // blobs per pass through the proof / recovery workspace (~0.4 GB at 512)
+
+extern "C" int kzgb200_load_cell_proof_setup(kzgb200_ctx* ctx, const uint8_t* g1_lagrange48, size_t n_points) {
+    if (!ctx) return KZGB200_BAD_ARGS;
+    if (!g1_lagrange48 || n_points != (size_t)kFieldElementsPerBlob) return KZGB200_INVALID_SETUP;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    CellCtx* c = ctx->cells;
+    if (!c) return KZGB200_INVALID_SETUP;
+    if (c->d_fk_tab) return KZGB200_OK;
+    uint8_t* d_bytes = nullptr; G1* d_a = nullptr; G1Affine* d_W = nullptr; uint32_t* d_bad = nullptr;
+    uint32_t bad = 0;
+    int rc = [&]() -> int {
+        CK(cudaMalloc(&c->ptables, sizeof(ProofTables)));
+        CK(cudaMalloc(&c->d_mono, kFieldElementsPerBlob * sizeof(G1Affine)));
+        CK(cudaMalloc(&d_bytes, kFieldElementsPerBlob * 48)); CK(cudaMalloc(&d_a, kFieldElementsPerBlob * sizeof(G1)));
+        CK(cudaMalloc(&d_W, kFk20Bases * sizeof(G1Affine))); CK(cudaMalloc(&d_bad, 4));
+        CK(cudaMemsetAsync(d_bad, 0, 4, ctx->stream));
+        CK(cudaMemcpyAsync(d_bytes, g1_lagrange48, kFieldElementsPerBlob * 48, cudaMemcpyHostToDevice, ctx->stream));
+        proof_setup_kernel<<<kExtElements / 128, 128, 0, ctx->stream>>>(c->ptables);
+        mono_load_kernel<<<kFieldElementsPerBlob / 128, 128, 0, ctx->stream>>>(d_bytes, d_a, d_bad);
+        for (int len = 2; len <= kFieldElementsPerBlob; len <<= 1)
+            mono_level_kernel<<<kFieldElementsPerBlob / 2 / 128, 128, 0, ctx->stream>>>(d_a, len, c->tables);
+        mono_finish_kernel<<<kFieldElementsPerBlob / 128, 128, 0, ctx->stream>>>(d_a, c->tables, c->d_mono, d_bad);
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(&bad, d_bad, 4, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        if (bad) return KZGB200_INVALID_SETUP;      // not the setup of the loaded cell points (or a point that does not parse)
+        CK(cudaMalloc(&c->d_fk_tab, kFk20TablePoints * sizeof(G1Affine)));
+        fk20_w_kernel<<<kFieldElementsPerCell, 64, 0, ctx->stream>>>(c->d_mono, c->tables, d_W);
+        fk20_table_kernel<<<kFk20Bases * kFk20Windows / 128, 128, 0, ctx->stream>>>(d_W, c->d_fk_tab);
+        CK(cudaGetLastError());
+        CK(cudaFuncSetAttribute(compute_cells_coeffs_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCellNttSmemBytes));
+        CK(cudaFuncSetAttribute(recover_ntt_inv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCellNttSmemBytes));
+        CK(cudaFuncSetAttribute(recover_ntt_div_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCellNttSmemBytes));
+        CK(cudaFuncSetAttribute(recover_blob_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCellNttSmemBytes));
+        CK(cudaMalloc(&c->d_rin, (size_t)kCellsPerExtBlob * kBytesPerCell)); CK(cudaMalloc(&c->d_pout, (size_t)kCellsPerExtBlob * 48));
+        CK(cudaMalloc(&c->d_pos, kCellsPerExtBlob * sizeof(int))); CK(cudaMalloc(&c->d_missing, kCellsPerExtBlob * sizeof(uint32_t)));
+        CK(cudaMalloc(&c->d_z, 2 * kCellsPerExtBlob * sizeof(Fr)));
+        CK(cudaStreamSynchronize(ctx->stream));
+        return KZGB200_OK;
+    }();
+    for (void* p : {(void*)d_bytes, (void*)d_a, (void*)d_W, (void*)d_bad}) if (p) cudaFree(p);
+    if (rc != KZGB200_OK) proof_destroy(c);
+    return rc;
+}
+
+extern "C" int kzgb200_cell_proof_monomial(kzgb200_ctx* ctx, uint8_t* out48, size_t n_points) {
+    if (!ctx || !out48 || n_points > (size_t)kFieldElementsPerBlob) return KZGB200_BAD_ARGS;
+    if (!ctx->cells || !ctx->cells->d_fk_tab) return KZGB200_INVALID_SETUP;
+    if (n_points == 0) return KZGB200_OK;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    uint8_t* d_out = nullptr;
+    int rc = [&]() -> int {
+        CK(cudaMalloc(&d_out, n_points * 48));
+        mono_compress_kernel<<<(unsigned)((n_points + 127) / 128), 128, 0, ctx->stream>>>(ctx->cells->d_mono, (int)n_points, d_out);
+        CK(cudaGetLastError());
+        CK(cudaMemcpyAsync(out48, d_out, n_points * 48, cudaMemcpyDeviceToHost, ctx->stream));
+        CK(cudaStreamSynchronize(ctx->stream));
+        return KZGB200_OK;
+    }();
+    if (d_out) cudaFree(d_out);
+    return rc;
+}
+
+static int proof_workspace(kzgb200_ctx* ctx, size_t n) {
+    CellCtx* c = ctx->cells;
+    const size_t nb = n < kProofChunk ? n : kProofChunk;
+    if (nb <= c->proof_cap) return KZGB200_OK;
+    c->proof_cap = 0;
+    CK(regrow(c->d_pcoef, nb * kFieldElementsPerBlob)); CK(regrow(c->d_fkU, nb * kFk20Bases)); CK(regrow(c->d_A, nb * kExtElements));
+    CK(regrow(c->d_V, nb * kCellsPerExtBlob)); CK(regrow(c->d_rblobs, nb * kBytesPerBlob));
+    c->proof_cap = nb;
+    return KZGB200_OK;
+}
+// cells and proofs of n device blobs (the caller has checked n <= proof_cap or chunks; status: n flags, zeroed by the caller).
+// Profiling slots: 0 = coefficients (with the cells), 1 = fixed-base products (with the scalar DFTs), 2 = G1 transforms.
+static int fk20_launch(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8_t* d_cells, uint8_t* d_proofs, uint32_t* status) {
+    CellCtx* c = ctx->cells;
+    cudaStream_t st = ctx->stream;
+    for (size_t lo = 0; lo < n; lo += kProofChunk) {
+        const int cnt = (int)(n - lo < kProofChunk ? n - lo : kProofChunk);
+        phase_begin(ctx, 0, st);
+        compute_cells_coeffs_kernel<<<cnt, kCellNttThreads, kCellNttSmemBytes, st>>>(d_blobs + lo * kBytesPerBlob, cnt, c->tables,
+                                                                                    d_cells + lo * kCellsPerExtBlob * kBytesPerCell, status + lo, c->d_pcoef);
+        phase_end(ctx, 0, st);
+        phase_begin(ctx, 1, st);
+        fk20_scalars_kernel<<<dim3(kFieldElementsPerCell, cnt), 64, 0, st>>>(c->d_pcoef, c->tables, c->d_fkU);
+        fk20_products_kernel<<<dim3(kCellsPerExtBlob, cnt), 64, 0, st>>>(c->d_fkU, c->d_fk_tab, c->d_V);
+        phase_end(ctx, 1, st);
+        phase_begin(ctx, 2, st);
+        fk20_proofs_kernel<<<cnt, 64, 0, st>>>(c->d_V, c->tables, d_proofs + lo * kCellsPerExtBlob * 48);
+        phase_end(ctx, 2, st);
+    }
+    CK(cudaGetLastError());
+    return KZGB200_OK;
+}
+static int proof_begin(kzgb200_ctx* ctx, size_t n) {
+    for (int i = 0; i < 8; i++) ctx->ph_started[i] = false;
+    int rc = ensure_capacity(ctx, n, false);
+    if (!rc) rc = proof_workspace(ctx, n);
+    if (rc) return rc;
+    CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_parse, 0));
+    CK(cudaMemsetAsync(ctx->d_status, 0, n * sizeof(uint32_t), ctx->stream));
+    return KZGB200_OK;
+}
+// BAD_ARGS if any of the n blobs had a non-canonical element
+static int proof_result(kzgb200_ctx* ctx, size_t n) {
+    status_or_kernel<<<1, 256, 0, ctx->stream>>>(ctx->d_status, (int)n, ctx->d_result);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(ctx->h_result, ctx->d_result, 4, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    collect_phase_times(ctx);
+    return ctx->h_result[0] ? KZGB200_BAD_ARGS : KZGB200_OK;
+}
+static bool proof_ready(kzgb200_ctx* ctx) { return ctx->cells && ctx->cells->d_fk_tab; }
+
+extern "C" int kzgb200_compute_cells_and_kzg_proofs(kzgb200_ctx* ctx, const uint8_t* blob, uint8_t* cells_out, uint8_t* proofs_out) {
+    if (!ctx || !blob || !cells_out || !proofs_out) return KZGB200_BAD_ARGS;
+    if (!proof_ready(ctx)) return KZGB200_INVALID_SETUP;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    int rc = ensure_capacity(ctx, 1, true);
+    if (!rc) rc = proof_begin(ctx, 1);
+    if (rc) return rc;
+    CellCtx* c = ctx->cells;
+    if (!c->d_ext) CK(cudaMalloc(&c->d_ext, (size_t)kCellsPerExtBlob * kBytesPerCell));
+    CK(cudaMemcpyAsync(ctx->d_blobs, blob, kBytesPerBlob, cudaMemcpyHostToDevice, ctx->stream));
+    if ((rc = fk20_launch(ctx, ctx->d_blobs, 1, c->d_ext, c->d_pout, ctx->d_status))) return rc;
+    if ((rc = proof_result(ctx, 1))) return rc;
+    CK(cudaMemcpyAsync(cells_out, c->d_ext, (size_t)kCellsPerExtBlob * kBytesPerCell, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(proofs_out, c->d_pout, (size_t)kCellsPerExtBlob * 48, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return KZGB200_OK;
+}
+extern "C" int kzgb200_compute_cells_and_kzg_proofs_batch_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8_t* d_cells, uint8_t* d_proofs) {
+    if (!ctx || (n && (!d_blobs || !d_cells || !d_proofs)) || n > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
+    if (!proof_ready(ctx)) return KZGB200_INVALID_SETUP;
+    if (n == 0) return KZGB200_OK;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    int rc = proof_begin(ctx, n);
+    if (!rc) rc = fk20_launch(ctx, d_blobs, n, d_cells, d_proofs, ctx->d_status);
+    return rc ? rc : proof_result(ctx, n);
+}
+
+// The spec's argument checks on one index set: 64 <= n_cells <= 128, every index < 128, no index twice.  pos[k] = the input
+// position of cell index k or -1; missing = the absent indices.
+static int recover_plan(const uint64_t* idx, size_t n_cells, int* pos, uint32_t* missing, int* n_missing) {
+    if (!idx || n_cells < (size_t)kCellsPerExtBlob / 2 || n_cells > (size_t)kCellsPerExtBlob) return KZGB200_BAD_ARGS;
+    for (int k = 0; k < kCellsPerExtBlob; k++) pos[k] = -1;
+    for (size_t j = 0; j < n_cells; j++) {
+        if (idx[j] >= (uint64_t)kCellsPerExtBlob || pos[idx[j]] >= 0) return KZGB200_BAD_ARGS;
+        pos[idx[j]] = (int)j;
+    }
+    *n_missing = 0;
+    for (int k = 0; k < kCellsPerExtBlob; k++) if (pos[k] < 0) missing[(*n_missing)++] = (uint32_t)k;
+    return KZGB200_OK;
+}
+// recovery of nb blobs that share one index set: d_in = nb x n_cells cells (blob-major), outputs as compute_cells_and_kzg_proofs.
+// Profiling slot 3 = the recovery transforms (E Z, the three 8192-point transforms, the 4096-point transform back to the blob).
+static int recover_launch(kzgb200_ctx* ctx, const int* pos, const uint32_t* missing, int n_missing, const uint8_t* d_in, size_t n_cells, size_t nb,
+                          uint8_t* d_cells_out, uint8_t* d_proofs_out) {
+    CellCtx* c = ctx->cells;
+    cudaStream_t st = ctx->stream;
+    CK(cudaMemcpyAsync(c->d_pos, pos, kCellsPerExtBlob * sizeof(int), cudaMemcpyHostToDevice, st));
+    if (n_missing) CK(cudaMemcpyAsync(c->d_missing, missing, n_missing * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
+    recover_z_kernel<<<1, 2 * kCellsPerExtBlob, 0, st>>>(c->d_missing, n_missing, c->tables, c->ptables, c->d_z);
+    for (size_t lo = 0; lo < nb; lo += kProofChunk) {
+        const int cnt = (int)(nb - lo < kProofChunk ? nb - lo : kProofChunk);
+        phase_begin(ctx, 3, st);
+        recover_load_kernel<<<(unsigned)((size_t)cnt * kExtElements / 256), 256, 0, st>>>(d_in + lo * n_cells * kBytesPerCell, (int)n_cells, c->d_pos,
+                                                                                         c->d_z, cnt, c->d_A, ctx->d_status + lo);
+        recover_ntt_inv_kernel<<<dim3(2, cnt), kCellNttThreads, kCellNttSmemBytes, st>>>(c->d_A, c->tables);
+        recover_mid_kernel<<<(unsigned)((size_t)cnt * kFieldElementsPerBlob / 256), 256, 0, st>>>(c->d_A, c->ptables, cnt);
+        recover_ntt_div_kernel<<<dim3(2, cnt), kCellNttThreads, kCellNttSmemBytes, st>>>(c->d_A, c->tables, c->d_z);
+        recover_final_kernel<<<(unsigned)((size_t)cnt * kFieldElementsPerBlob / 256), 256, 0, st>>>(c->d_A, c->ptables, cnt, c->d_pcoef);
+        recover_blob_kernel<<<cnt, kCellNttThreads, kCellNttSmemBytes, st>>>(c->d_pcoef, c->tables, c->d_rblobs);
+        phase_end(ctx, 3, st);
+        CK(cudaGetLastError());
+        int rc = fk20_launch(ctx, c->d_rblobs, cnt, d_cells_out + lo * kCellsPerExtBlob * kBytesPerCell, d_proofs_out + lo * kCellsPerExtBlob * 48,
+                             ctx->d_status + lo);
+        if (rc) return rc;
+    }
+    return KZGB200_OK;
+}
+extern "C" int kzgb200_recover_cells_and_kzg_proofs(kzgb200_ctx* ctx, const uint64_t* cell_indices, const uint8_t* cells, size_t n_cells,
+                                                    uint8_t* cells_out, uint8_t* proofs_out) {
+    if (!ctx || !cells || !cells_out || !proofs_out) return KZGB200_BAD_ARGS;
+    if (!proof_ready(ctx)) return KZGB200_INVALID_SETUP;
+    int pos[kCellsPerExtBlob], n_missing = 0;
+    uint32_t missing[kCellsPerExtBlob];
+    int rc = recover_plan(cell_indices, n_cells, pos, missing, &n_missing);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    if ((rc = proof_begin(ctx, 1))) return rc;
+    CellCtx* c = ctx->cells;
+    if (!c->d_ext) CK(cudaMalloc(&c->d_ext, (size_t)kCellsPerExtBlob * kBytesPerCell));
+    CK(cudaMemcpyAsync(c->d_rin, cells, n_cells * kBytesPerCell, cudaMemcpyHostToDevice, ctx->stream));
+    if ((rc = recover_launch(ctx, pos, missing, n_missing, c->d_rin, n_cells, 1, c->d_ext, c->d_pout))) return rc;
+    if ((rc = proof_result(ctx, 1))) return rc;
+    CK(cudaMemcpyAsync(cells_out, c->d_ext, (size_t)kCellsPerExtBlob * kBytesPerCell, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaMemcpyAsync(proofs_out, c->d_pout, (size_t)kCellsPerExtBlob * 48, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return KZGB200_OK;
+}
+extern "C" int kzgb200_recover_cells_and_kzg_proofs_batch_device(kzgb200_ctx* ctx, const uint64_t* cell_indices, size_t n_cells, const uint8_t* d_cells,
+                                                                 size_t n_blobs, uint8_t* d_cells_out, uint8_t* d_proofs_out) {
+    if (!ctx || (n_blobs && (!d_cells || !d_cells_out || !d_proofs_out)) || n_blobs > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
+    if (!proof_ready(ctx)) return KZGB200_INVALID_SETUP;
+    int pos[kCellsPerExtBlob], n_missing = 0;
+    uint32_t missing[kCellsPerExtBlob];
+    int rc = recover_plan(cell_indices, n_cells, pos, missing, &n_missing);
+    if (rc || n_blobs == 0) return rc;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    if ((rc = proof_begin(ctx, n_blobs))) return rc;
+    if ((rc = recover_launch(ctx, pos, missing, n_missing, d_cells, n_cells, n_blobs, d_cells_out, d_proofs_out))) return rc;
+    return proof_result(ctx, n_blobs);
 }

@@ -61,6 +61,17 @@ struct CellCtx {
     uint64_t* h_idx = nullptr;
     std::vector<uint32_t> slot;                                    // open-addressing table of the commitment deduplication
     cudaEvent_t ev_r = nullptr, ev_rli = nullptr;
+    // cell proofs and recovery (kzgb200_load_cell_proof_setup): tables, and a workspace for up to proof_cap blobs at a time
+    ProofTables* ptables = nullptr;
+    G1Affine *d_mono = nullptr, *d_fk_tab = nullptr;               // [tau^m]G1 (m < 4096), FK20 window tables (kFk20TablePoints)
+    size_t proof_cap = 0;
+    Fr *d_pcoef = nullptr, *d_fkU = nullptr, *d_A = nullptr;        // coefficients x 4096 / recovered coefficients, U_b[f], 8192-point work
+    G1* d_V = nullptr;                                             // V[f] = sum_b U_b[f] W_b[f]
+    uint8_t* d_rblobs = nullptr;                                   // recovered blobs
+    uint8_t *d_rin = nullptr, *d_pout = nullptr;                   // staging of one host call: input cells, 128 proofs
+    int* d_pos = nullptr;                                          // recovery: input position of each cell index (-1: missing)
+    uint32_t* d_missing = nullptr;
+    Fr* d_z = nullptr;                                             // see recover_z_kernel
 };
 
 }  // namespace kzgb200
