@@ -5,7 +5,7 @@
 //   kzg_rs::KzgSettings::load_trusted_setup_file                                                src/trusted_setup.rs:94-98
 //   kzg_rs::Blob / Bytes32 / Bytes48 (from_slice length check, as_slice)                        src/dtypes.rs:7-46
 //   kzg_rs::KzgError                                                                            src/enums.rs:6-18
-// plus EIP-7594 cells: kzg_rs::Cell, KzgProof::verify_cell_kzg_proof_batch, kzg_rs::compute_cells, kzg_rs::compute_cells_and_kzg_proofs,
+// plus EIP-7594 cells: kzg_rs::Cell, KzgProof::verify_cell_kzg_proof_batch[_many], kzg_rs::compute_cells, kzg_rs::compute_cells_and_kzg_proofs,
 // kzg_rs::recover_cells_and_kzg_proofs (c-kzg-4844 / rust-kzg names).
 // Result<bool, KzgError> is kzg_rs::Result<bool>: either a value or an error.
 #pragma once
@@ -146,6 +146,24 @@ struct KzgProof {
                                                      cell_indices.data(), reinterpret_cast<const uint8_t*>(cells.data()),
                                                      reinterpret_cast<const uint8_t*>(proofs_bytes.data()), n, &ok);
         return detail::to_result(rc, ok);
+    }
+    // k independent verify_cell_kzg_proof_batch calls in one: the cells of all groups contiguous, group g = cells
+    // [group_offsets[g], group_offsets[g + 1]) (k + 1 offsets, the first 0, the last n).  One verdict per group: 1 = true, 0 = false,
+    // 2 = the group alone would give BadArgs.  An error only for the call itself (lengths, offsets, setup).
+    static Result<std::vector<uint8_t>> verify_cell_kzg_proof_batch_many(const std::vector<Bytes48>& commitments_bytes,
+                                                                         const std::vector<uint64_t>& cell_indices, const std::vector<Cell>& cells,
+                                                                         const std::vector<Bytes48>& proofs_bytes,
+                                                                         const std::vector<uint64_t>& group_offsets, const KzgSettings& kzg_settings) {
+        const size_t n = cell_indices.size();
+        if (commitments_bytes.size() != n || cells.size() != n || proofs_bytes.size() != n || group_offsets.empty() || group_offsets.back() != n)
+            return KzgError{KzgError::InvalidBytesLength, "Invalid cells / commitments / proofs / group offsets length"};
+        std::vector<uint8_t> verdicts(group_offsets.size() - 1);
+        int rc = kzgb200_verify_cell_kzg_proof_batch_many(kzg_settings.ctx(), reinterpret_cast<const uint8_t*>(commitments_bytes.data()),
+                                                          cell_indices.data(), reinterpret_cast<const uint8_t*>(cells.data()),
+                                                          reinterpret_cast<const uint8_t*>(proofs_bytes.data()), group_offsets.data(),
+                                                          verdicts.size(), verdicts.data());
+        if (rc) return detail::to_result(rc, 0).unwrap_err();
+        return verdicts;
     }
 };
 

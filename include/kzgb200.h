@@ -206,6 +206,31 @@ int kzgb200_compute_cells_batch_device(kzgb200_ctx* ctx, const uint8_t* d_blobs,
 int kzgb200_harness_generate_cells(kzgb200_ctx* ctx, uint64_t seed, size_t n_blobs, int degree, const uint8_t* tau_powers48,
                                    uint8_t* d_cells, uint8_t* d_commitments, uint8_t* d_proofs);
 
+/* ---- many cell batches in one call, one verdict each (PeerDAS data column sidecars) ----------------------------------------
+ * kzgb200_verify_cell_kzg_proof_batch_many: n cells in the per-cell layout of kzgb200_verify_cell_kzg_proof_batch, split into
+ *   n_groups groups by group_offsets[0..n_groups] (host: offsets[0] = 0, never decreasing, offsets[n_groups] = n; group g = cells
+ *   [offsets[g], offsets[g + 1])).  verdicts[g] (host, n_groups bytes) = 1 / 0 / 2: verify_cell_kzg_proof_batch on group g alone
+ *   returns true / false / fails an assertion (an index >= 128, a non-canonical element, a commitment or proof that is not a valid
+ *   compressed subgroup point).  An empty group gets 1; a bad group never changes another group's verdict.  Each group's challenge
+ *   r_g is the spec's, hashed over that group's bytes alone (its own deduplication of commitments) by up to 16 host threads while
+ *   the GPU parses.  All groups are checked together first (weights rho^g r_g^j, one MSM and one pairing; a false group passes it
+ *   with probability <= n_groups / q); only if that fails does every group get its own check (one extra pass for any number of bad
+ *   groups).  Returns BAD_ARGS only for a malformed call (a null pointer with n > 0 or n_groups > 0, bad offsets, n or n_groups
+ *   above 0x7fffffff / 2), INVALID_SETUP without the cell setup; n_groups == 0 -> OK.
+ *   The _device form takes device pointers for the four data arrays (group_offsets and verdicts stay host memory); the inputs are
+ *   copied back to pinned host memory once for the transcripts.
+ *   kzgb200_get_phase_ms after a _many call: {parse, host hashing (wall ms, every call), hasher threads (every call), r_g upload and
+ *   weights, lincomb, reduce, combined pairing, per-group fallback}; the device slots with kzgb200_set_profiling on.
+ * kzgb200_last_cell_many_r: the last _many call's r_g (r_out: n_groups x 32, zeros for empty groups) and rho (rho_out32), canonical
+ *   big-endian; n_groups must be that call's (else BAD_ARGS).  A _many call leaves what kzgb200_last_r and kzgb200_last_partial
+ *   report untouched. */
+int kzgb200_verify_cell_kzg_proof_batch_many(kzgb200_ctx* ctx, const uint8_t* commitments, const uint64_t* cell_indices, const uint8_t* cells,
+                                             const uint8_t* proofs, const uint64_t* group_offsets, size_t n_groups, uint8_t* verdicts);
+int kzgb200_verify_cell_kzg_proof_batch_many_device(kzgb200_ctx* ctx, const uint8_t* d_commitments, const uint64_t* d_cell_indices,
+                                                    const uint8_t* d_cells, const uint8_t* d_proofs, const uint64_t* group_offsets,
+                                                    size_t n_groups, uint8_t* verdicts);
+int kzgb200_last_cell_many_r(kzgb200_ctx* ctx, uint8_t* r_out, size_t n_groups, uint8_t* rho_out32);
+
 /* ---- EIP-7594 cell proofs and recovery (FK20; consensus-specs Fulu compute_cells_and_kzg_proofs / recover_cells_and_kzg_proofs) --
  * kzgb200_load_cell_proof_setup: the setup's 4096 Lagrange G1 points (host, 4096 x 48 compressed, file order: point j pairs with
  *   omega4096^j; KzgSettings.g1_lagrange_bytes).  n_points must be 4096 and the cell setup must be loaded, else INVALID_SETUP.  Derives

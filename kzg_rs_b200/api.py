@@ -116,6 +116,9 @@ class Library:
         d.kzgb200_load_cell_setup.argtypes = [p, C.c_char_p, sz, C.c_char_p]
         d.kzgb200_verify_cell_kzg_proof_batch.argtypes = [p, p, p, p, p, sz, ip]
         d.kzgb200_verify_cell_kzg_proof_batch_device.argtypes = [p, p, p, p, p, sz, ip]
+        d.kzgb200_verify_cell_kzg_proof_batch_many.argtypes = [p, p, p, p, p, p, sz, p]
+        d.kzgb200_verify_cell_kzg_proof_batch_many_device.argtypes = [p, p, p, p, p, p, sz, p]
+        d.kzgb200_last_cell_many_r.argtypes = [p, p, sz, p]
         d.kzgb200_compute_cells.argtypes = [p, C.c_char_p, p]
         d.kzgb200_compute_cells_batch_device.argtypes = [p, p, sz, p]
         d.kzgb200_harness_generate_cells.argtypes = [p, C.c_uint64, sz, C.c_int, C.c_char_p, p, p, p]
@@ -411,6 +414,33 @@ class KzgProof:
         if rc:
             _raise(rc, ctx, "Failed to parse cell / G1Affine / cell index" if rc == 1 else None)
         return bool(ok.value)
+
+    @staticmethod
+    def verify_cell_kzg_proof_batch_many(batches, kzg_settings, device=0):
+        """Many independent verify_cell_kzg_proof_batch calls in one GPU call (e.g. one per data column sidecar): batches is a
+        sequence of (commitments_bytes, cell_indices, cells, proofs_bytes), each as for verify_cell_kzg_proof_batch.  Returns one
+        verdict per batch: True / False / None, None = that batch alone would raise BadArgs; a bad batch does not change another's
+        verdict.  Mismatched lengths inside a batch or wrong byte lengths -> KzgError(InvalidBytesLength) for the whole call."""
+        cs, ce, ps, idx, offs = [], [], [], [], [0]
+        for commitments_bytes, cell_indices, cells, proofs_bytes in batches:
+            n = len(cell_indices)
+            if not (len(commitments_bytes) == len(cells) == len(proofs_bytes) == n):
+                raise KzgError("InvalidBytesLength", "Invalid cells / commitments / proofs length")
+            cs += [_b(x, 48, "commitment") for x in commitments_bytes]
+            ce += [_b(x, BYTES_PER_CELL, "cell") for x in cells]
+            ps += [_b(x, 48, "proof") for x in proofs_bytes]
+            idx += [int(i) if 0 <= int(i) < 1 << 64 else (1 << 64) - 1 for i in cell_indices]   # out of range: that batch gets None
+            offs.append(offs[-1] + n)
+        k, n = len(offs) - 1, offs[-1]
+        ctx = kzg_settings.cell_context(device)
+        out = C.create_string_buffer(max(k, 1))
+        off = (C.c_uint64 * (k + 1))(*offs)
+        ia = (C.c_uint64 * max(n, 1))(*idx)
+        rc = Library.get().dll.kzgb200_verify_cell_kzg_proof_batch_many(ctx, _ptr(b"".join(cs)), C.cast(ia, C.c_void_p), _ptr(b"".join(ce)),
+                                                                        _ptr(b"".join(ps)), C.cast(off, C.c_void_p), k, out)
+        if rc:
+            _raise(rc, ctx)
+        return [{0: False, 1: True, 2: None}[v] for v in out.raw[:k]]
 
 
 def compute_cells(blob, kzg_settings, device=0):

@@ -155,8 +155,9 @@ __global__ void z_setup_kernel(const uint8_t* __restrict__ z_be32, int n, Fr* __
 __global__ void import_parsed_kernel(const uint8_t* __restrict__ c104, const uint8_t* __restrict__ p104, const uint8_t* __restrict__ z32,
                                      const uint8_t* __restrict__ y32, int n, G1Affine* __restrict__ C, G1Affine* __restrict__ P,
                                      uint8_t* __restrict__ c48, uint8_t* __restrict__ p48, Fr* __restrict__ z_mont, ZY* __restrict__ zy);
+// weights: per-entry scalars (Montgomery) in place of r^(offset + i); nullptr = the powers of r
 __global__ void msm_scalars_kernel(const Fr* __restrict__ z_mont, const ZY* __restrict__ zy, const Fr* __restrict__ r_mont, uint64_t offset, int n,
-                                   uint8_t* __restrict__ digits, Fr* __restrict__ ry);
+                                   uint8_t* __restrict__ digits, Fr* __restrict__ ry, const Fr* __restrict__ weights);
 __global__ void msm_sort_kernel(const uint8_t* __restrict__ digits, int n, uint32_t* __restrict__ order, uint32_t* __restrict__ start);
 void launch_msm_bucket(int ctas_per_sm, int n, int slice, cudaStream_t st, const G1Affine* C, const G1Affine* P, const uint32_t* order,
                        const uint32_t* start, G1* halfsum, G1* part);
@@ -187,10 +188,11 @@ __global__ void many_lhs_kernel(const uint8_t* __restrict__ z32, const uint8_t* 
                                 uint32_t* __restrict__ status);
 __global__ void many_lhs_zy_kernel(const ZY* __restrict__ zy, const G1Affine* __restrict__ C, const G1Affine* __restrict__ P, size_t m,
                                    const DeviceTables* __restrict__ T, G1Affine* __restrict__ X, const uint32_t* __restrict__ status);
+// e(X_i, G2) e(-P_i, Q) == 1; lines_b: line table of Q, nullptr = [tau]G2 (T->pairing.tau_g2)
 __global__ void many_pairing_kernel(const G1Affine* __restrict__ X, const G1Affine* __restrict__ P, const uint32_t* __restrict__ status, size_t m,
-                                    const DeviceTables* __restrict__ T, uint8_t* __restrict__ verdicts);
+                                    const DeviceTables* __restrict__ T, const LineCoeffs* __restrict__ lines_b, uint8_t* __restrict__ verdicts);
 __global__ void many_pairing_warp_kernel(const G1Affine* __restrict__ X, const G1Affine* __restrict__ P, size_t m, const DeviceTables* __restrict__ T,
-                                         uint8_t* __restrict__ verdicts);
+                                         const LineCoeffs* __restrict__ lines_b, uint8_t* __restrict__ verdicts);
 __global__ void export_scalars_kernel(const ZY* __restrict__ zy, int n, uint8_t* __restrict__ z_out, uint8_t* __restrict__ y_out);
 __global__ void r_to_raw_kernel(const Fr* __restrict__ r_mont, ZY* __restrict__ out);
 __global__ void status_or_kernel(const uint32_t* __restrict__ status, int n, uint32_t* __restrict__ out);
@@ -242,6 +244,17 @@ __global__ void cell_agg_kernel(const uint8_t* __restrict__ cells, const uint32_
 __global__ void cell_interp_kernel(const Fr* __restrict__ agg, const uint32_t* __restrict__ meta, int n, const CellTables* __restrict__ T,
                                    Fr* __restrict__ coeffs);
 __global__ void cell_rli_kernel(const Fr* __restrict__ coeffs, const CellTables* __restrict__ T, Partial* __restrict__ out);
+// verify_cell_kzg_proof_batch_many (k_cells.cu): goff = the k + 1 group offsets, gbad = per-group BadArgs flags
+__global__ void many_group_status_kernel(const uint32_t* __restrict__ status, int n, const uint32_t* __restrict__ goff, int k, uint32_t* __restrict__ gbad);
+__global__ void many_weights_kernel(int n, const uint32_t* __restrict__ goff, int k, const uint8_t* __restrict__ rg, const uint32_t* __restrict__ gbad,
+                                    Fr* __restrict__ w, uint32_t* __restrict__ status);
+__global__ void many_terms_kernel(int n, const Fr* __restrict__ w, const Fr* __restrict__ z_mont, const G1Affine* __restrict__ C, const G1Affine* __restrict__ P,
+                                  G1* __restrict__ terms);
+__global__ void many_group_sums_kernel(const uint32_t* __restrict__ goff, const G1* __restrict__ terms, G1* __restrict__ AB);
+__global__ void many_run_interp_kernel(const uint8_t* __restrict__ cells, const uint32_t* __restrict__ fmeta, int n, int runs, const Fr* __restrict__ w,
+                                       const CellTables* __restrict__ T, Fr* __restrict__ rcoef);
+__global__ void many_group_rli_kernel(const Fr* __restrict__ rcoef, const uint32_t* __restrict__ grun, const G1* __restrict__ AB, const CellTables* __restrict__ T,
+                                      G1Affine* __restrict__ X, G1Affine* __restrict__ A);
 __global__ void cell_harness_terms_kernel(uint64_t seed, int n, int D, const G1Affine* __restrict__ M, G1* __restrict__ terms);
 __global__ void cell_harness_sums_kernel(int n, const G1* __restrict__ terms, G1* __restrict__ sums);
 __global__ void cell_harness_points_kernel(int n, const G1* __restrict__ sums, const CellTables* __restrict__ T, uint8_t* __restrict__ commitments,

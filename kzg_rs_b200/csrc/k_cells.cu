@@ -198,17 +198,10 @@ __global__ void __launch_bounds__(kFieldElementsPerCell) cell_agg_kernel(const u
     }
     agg[((size_t)i * kCellAggSlices + s) * kFieldElementsPerCell + j] = acc;
 }
-// per distinct index i: the slices' sums, a 64-point inverse DFT (bit-reversed in, natural out), coefficient m scaled by
-// h_i^-m / 64 -> coeffs[i][m]; an index without cells contributes zeros
-__global__ void __launch_bounds__(kFieldElementsPerCell) cell_interp_kernel(const Fr* __restrict__ agg, const uint32_t* __restrict__ meta, int n,
-                                                                           const CellTables* __restrict__ T, Fr* __restrict__ coeffs) {
-    __shared__ Fr v[kFieldElementsPerCell];
-    const int i = blockIdx.x, j = threadIdx.x;
-    const uint32_t* start = meta + 3 * (size_t)n;
-    if (start[i] == start[i + 1]) { coeffs[i * kFieldElementsPerCell + j] = Fr::zero(); return; }
-    Fr acc = Fr::zero();
-    for (int s = 0; s < kCellAggSlices; s++) acc = acc.add_inl(agg[((size_t)i * kCellAggSlices + s) * kFieldElementsPerCell + j]);
-    v[j] = acc;
+// 64-point inverse DFT of the 64 values v[] of one cell index i (shared memory, bit-reversed in, natural out), coefficient m scaled
+// by h_i^-m / 64: thread j (of 64) gets coefficient j of the interpolant.  Shared by cell_interp_kernel and the per-group checks.
+__device__ __forceinline__ Fr cell_interp_body(Fr* v, int i, const CellTables* __restrict__ T) {
+    const int j = threadIdx.x;
     __syncthreads();
     for (int len = 2; len <= kFieldElementsPerCell; len <<= 1) {
         const int half = len >> 1, stride = kFieldElementsPerCell / len;
@@ -220,15 +213,25 @@ __global__ void __launch_bounds__(kFieldElementsPerCell) cell_interp_kernel(cons
         __syncthreads();
     }
     const Fr scale = fr_pow_u32(T->shift_inv[i], (uint32_t)j, 6).mul_inl(T->inv64);
-    coeffs[i * kFieldElementsPerCell + j] = v[j].mul_inl(scale);
+    return v[j].mul_inl(scale);
 }
-// RLI = sum_m c_m [tau^m]G1, c_m = sum_i coeffs[i][m]; thread (m, q) multiplies [2^(64q) tau^m]G1 by the q-th 64-bit word of c_m,
-// then a tree over the 256 products.  Written as the second partial of the final check: a = O, b = -RLI.
-__global__ void __launch_bounds__(256) cell_rli_kernel(const Fr* __restrict__ coeffs, const CellTables* __restrict__ T, Partial* __restrict__ out) {
-    __shared__ G1 sm[256];
+// per distinct index i: the slices' sums, interpolated (cell_interp_body) -> coeffs[i][m]; an index without cells contributes zeros
+__global__ void __launch_bounds__(kFieldElementsPerCell) cell_interp_kernel(const Fr* __restrict__ agg, const uint32_t* __restrict__ meta, int n,
+                                                                           const CellTables* __restrict__ T, Fr* __restrict__ coeffs) {
+    __shared__ Fr v[kFieldElementsPerCell];
+    const int i = blockIdx.x, j = threadIdx.x;
+    const uint32_t* start = meta + 3 * (size_t)n;
+    if (start[i] == start[i + 1]) { coeffs[i * kFieldElementsPerCell + j] = Fr::zero(); return; }
+    Fr acc = Fr::zero();
+    for (int s = 0; s < kCellAggSlices; s++) acc = acc.add_inl(agg[((size_t)i * kCellAggSlices + s) * kFieldElementsPerCell + j]);
+    v[j] = acc;
+    coeffs[i * kFieldElementsPerCell + j] = cell_interp_body(v, i, T);
+}
+// sum_m c_m [tau^m]G1 over 256 threads: thread t = (m, q) = (t / 4, t % 4) holds c_m and multiplies [2^(64q) tau^m]G1 by the q-th
+// 64-bit word of c_m, then a tree over the 256 products in sm; the sum is returned to thread 0.  Shared by cell_rli_kernel and the
+// per-group checks.
+__device__ __forceinline__ G1 cell_rli_body(const Fr& c, const CellTables* __restrict__ T, G1* sm) {
     const int t = threadIdx.x, m = t / 4, q = t % 4;
-    Fr c = Fr::zero();
-    for (int i = 0; i < kCellsPerExtBlob; i++) c = c.add_inl(coeffs[i * kFieldElementsPerCell + m]);
     const Fr raw = c.to_raw();
     sm[t] = scalar_mul_affine(T->tau_tab[m][q], raw.l + 2 * q, 64);
     __syncthreads();
@@ -236,11 +239,117 @@ __global__ void __launch_bounds__(256) cell_rli_kernel(const Fr* __restrict__ co
         if (t < span) sm[t] = sm[t].add(sm[t + span]);
         __syncthreads();
     }
+    return sm[0];
+}
+// RLI = sum_m c_m [tau^m]G1, c_m = sum_i coeffs[i][m] (cell_rli_body).  Written as the second partial of the final check: a = O, b = -RLI.
+__global__ void __launch_bounds__(256) cell_rli_kernel(const Fr* __restrict__ coeffs, const CellTables* __restrict__ T, Partial* __restrict__ out) {
+    __shared__ G1 sm[256];
+    const int t = threadIdx.x, m = t / 4;
+    Fr c = Fr::zero();
+    for (int i = 0; i < kCellsPerExtBlob; i++) c = c.add_inl(coeffs[i * kFieldElementsPerCell + m]);
+    const G1 rli = cell_rli_body(c, T, sm);
     if (t == 0) {
         out->a = G1::identity();
-        out->b = sm[0].neg();
+        out->b = rli.neg();
         out->ry = Fr::zero();
         out->err = 0;
+    }
+}
+
+// ---- verify_cell_kzg_proof_batch_many: k independent groups of cells, one verdict each ------------------------------------
+// Group g = cells [goff[g], goff[g + 1]).  Every cell gets the weight w_k = rho^g r_g^j (j = its position in the group); the groups
+// are first checked together by the single-call pipeline with these weights in place of r^k, and only if that fails, each group on
+// its own (the fallback below).  gbad[g] != 0: group g fails an assertion of the spec (BadArgs).
+__device__ __forceinline__ uint32_t group_of(const uint32_t* __restrict__ goff, int k, uint32_t cell) {
+    int lo = 0, hi = k - 1;                        // the last g with goff[g] <= cell (empty groups before it are skipped)
+    while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (__ldg(goff + mid) <= cell) lo = mid; else hi = mid - 1; }
+    return (uint32_t)lo;
+}
+// the parse flags of every cell, ORed into its group's flag (gbad starts with the host's index checks)
+__global__ void __launch_bounds__(128) many_group_status_kernel(const uint32_t* __restrict__ status, int n, const uint32_t* __restrict__ goff, int k,
+                                                                uint32_t* __restrict__ gbad) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t s = status[i];
+    if (s) atomicOr(&gbad[group_of(goff, k, (uint32_t)i)], s);
+}
+// w_i = rho^g r_g^j, or 0 in a BadArgs group; rg = k + 1 canonical big-endian values (r_0 .. r_(k-1), rho).  The cell's parse flags are
+// cleared: they have been moved to gbad, and a BadArgs group must not fail the combined check.
+__global__ void __launch_bounds__(128) many_weights_kernel(int n, const uint32_t* __restrict__ goff, int k, const uint8_t* __restrict__ rg,
+                                                           const uint32_t* __restrict__ gbad, Fr* __restrict__ w, uint32_t* __restrict__ status) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const uint32_t g = group_of(goff, k, (uint32_t)i), j = (uint32_t)i - __ldg(goff + g);
+    status[i] = 0;
+    if (gbad[g]) { w[i] = Fr::zero(); return; }
+    const Fr r = Fr::from_raw(load_fe_be(reinterpret_cast<const uint4*>(rg + 32 * (size_t)g)));
+    const Fr rho = Fr::from_raw(load_fe_be(reinterpret_cast<const uint4*>(rg + 32 * (size_t)k)));
+    w[i] = rho.pow(&g, 32).mul_inl(r.pow(&j, 32));
+}
+// fallback, per cell: terms[2i] = [w_i]pi_i, terms[2i + 1] = [w_i]C_i + [w_i z_i]pi_i (GLV multiplications); identity for w_i = 0
+__global__ void __launch_bounds__(128) many_terms_kernel(int n, const Fr* __restrict__ w, const Fr* __restrict__ z_mont, const G1Affine* __restrict__ C,
+                                                         const G1Affine* __restrict__ P, G1* __restrict__ terms) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    const Fr wi = w[i];
+    G1 a = G1::identity(), b = G1::identity();
+    if (!wi.is_zero()) {
+        const G1Affine pi = P[i];
+        a = glv_mul(pi, wi.to_raw());
+        b = glv_mul(C[i], wi.to_raw()).add(glv_mul(pi, wi.mul_inl(z_mont[i]).to_raw()));
+    }
+    terms[2 * (size_t)i] = a;
+    terms[2 * (size_t)i + 1] = b;
+}
+// fallback, per group (one CTA each): A_g = sum of the group's [w]pi terms, B'_g = sum of its [w]C + [wz]pi terms
+__global__ void __launch_bounds__(128) many_group_sums_kernel(const uint32_t* __restrict__ goff, const G1* __restrict__ terms, G1* __restrict__ AB) {
+    __shared__ G1 sm[128];
+    const int g = blockIdx.x, t = threadIdx.x;
+    const uint32_t lo = goff[g], hi = goff[g + 1];
+    for (int part = 0; part < 2; part++) {
+        G1 acc = G1::identity();
+        for (uint32_t p = lo + t; p < hi; p += blockDim.x) acc = acc.add(terms[2 * (size_t)p + part]);
+        sm[t] = acc;
+        __syncthreads();
+        for (int span = 64; span >= 1; span >>= 1) {
+            if (t < span) sm[t] = sm[t].add(sm[t + span]);
+            __syncthreads();
+        }
+        if (t == 0) AB[2 * (size_t)g + part] = sm[0];
+        __syncthreads();
+    }
+}
+// fallback, per (group, cell index) run (one CTA of 64 threads each): the w-weighted sum of the run's cells, interpolated ->
+// rcoef[run][m].  fmeta = [cells of each group ordered by index (n) | start of each run in that order (runs + 1) | index of each run].
+__global__ void __launch_bounds__(kFieldElementsPerCell) many_run_interp_kernel(const uint8_t* __restrict__ cells, const uint32_t* __restrict__ fmeta,
+                                                                               int n, int runs, const Fr* __restrict__ w,
+                                                                               const CellTables* __restrict__ T, Fr* __restrict__ rcoef) {
+    __shared__ Fr v[kFieldElementsPerCell];
+    const int r = blockIdx.x, j = threadIdx.x;
+    const uint32_t* order = fmeta;
+    const uint32_t* rstart = fmeta + n;
+    const uint32_t idx = fmeta[n + runs + 1 + r];
+    Fr acc = Fr::zero();
+    for (uint32_t p = rstart[r]; p < rstart[r + 1]; p++) {
+        const uint32_t k = __ldg(order + p);
+        const Fr x = Fr::from_raw(load_fe_be(reinterpret_cast<const uint4*>(cells + (size_t)k * kBytesPerCell) + 2 * j));
+        acc = acc.add_inl(x.mul_inl(ldg_fr(w + k)));
+    }
+    v[j] = acc;
+    rcoef[(size_t)r * kFieldElementsPerCell + j] = cell_interp_body(v, (int)idx, T);
+}
+// fallback, per group (one CTA of 256 threads each): RLI_g from the coefficients of its runs (grun[g] .. grun[g + 1]), then the
+// two pairing arguments X_g = B'_g - RLI_g and A_g, affine, for e(X_g, G2) e(-A_g, [tau^64]G2) == 1 on the many-check engine
+__global__ void __launch_bounds__(256) many_group_rli_kernel(const Fr* __restrict__ rcoef, const uint32_t* __restrict__ grun, const G1* __restrict__ AB,
+                                                             const CellTables* __restrict__ T, G1Affine* __restrict__ X, G1Affine* __restrict__ A) {
+    __shared__ G1 sm[256];
+    const int g = blockIdx.x, t = threadIdx.x, m = t / 4;
+    Fr c = Fr::zero();
+    for (uint32_t r = grun[g]; r < grun[g + 1]; r++) c = c.add_inl(rcoef[(size_t)r * kFieldElementsPerCell + m]);
+    const G1 rli = cell_rli_body(c, T, sm);
+    if (t == 0) {
+        X[g] = g1_to_affine(AB[2 * (size_t)g + 1].add(rli.neg()));
+        A[g] = g1_to_affine(AB[2 * (size_t)g]);
     }
 }
 

@@ -7,7 +7,8 @@
 //   many_lhs_kernel                                        one thread per tuple: z, y canonical?  X_i = C_i - [y_i]G + [z_i]pi_i, affine
 //   many_pairing_kernel                                    kManyGroups tuples per CTA in lockstep: e(X_i, G2) e(-pi_i, [tau]G2) == 1 on the
 //                                                          cooperative engine (vliw.cuh), the Fp12 values in shared memory
-// Both G2 arguments are setup constants, so all tuples share the 2 x 68 precomputed line triples.
+// Both G2 arguments are setup constants, so all tuples share the 2 x 68 precomputed line triples.  The second one is [tau]G2, or
+// the point of the line table lines_b when it is given (the per-group cell checks: [tau^64]G2).
 #include "common.cuh"
 
 namespace kzgb200 {
@@ -55,7 +56,8 @@ struct ManySmem {
 static_assert(sizeof(ManySmem) <= kManySmemBytes, "keep kManySmemBytes (common.cuh) in step with ManySmem");
 __global__ void __launch_bounds__(kManyThreads, kManyCtasPerSm) many_pairing_kernel(const G1Affine* __restrict__ X, const G1Affine* __restrict__ P,
                                                                        const uint32_t* __restrict__ status, size_t m,
-                                                                       const DeviceTables* __restrict__ T, uint8_t* __restrict__ verdicts) {
+                                                                       const DeviceTables* __restrict__ T, const LineCoeffs* __restrict__ lines_b,
+                                                                       uint8_t* __restrict__ verdicts) {
     extern __shared__ __align__(16) unsigned char dyn_smem[];
     ManySmem& S = *reinterpret_cast<ManySmem*>(dyn_smem);
     vliw::Tables tab = vliw::load_tables(&S.stab, threadIdx.x, blockDim.x, true);
@@ -82,7 +84,7 @@ __global__ void __launch_bounds__(kManyThreads, kManyCtasPerSm) many_pairing_ker
             S.x[t] = x; S.np[t] = np; S.use[t] = use;
         }
         __syncthreads();
-        vliw::coop_pairing_multi(reinterpret_cast<Fp*>(S.regs), S.x, T->pairing.g2_gen, S.np, T->pairing.tau_g2, L, S.ok);
+        vliw::coop_pairing_multi(reinterpret_cast<Fp*>(S.regs), S.x, T->pairing.g2_gen, S.np, lines_b ? lines_b : T->pairing.tau_g2, L, S.ok);
         if (t < kManyGroups && S.use[t]) verdicts[batch * kManyGroups + t] = S.ok[t] ? kTrue : kFalse;
         __syncthreads();
     }

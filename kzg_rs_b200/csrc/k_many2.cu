@@ -10,7 +10,8 @@ struct ManyWarpSmem {
 };
 static_assert(sizeof(ManyWarpSmem) <= kManySmemBytes, "shared-memory budget of the many-tuple kernels");
 __global__ void __launch_bounds__(32 * kManyWarps, 1) many_pairing_warp_kernel(const G1Affine* __restrict__ X, const G1Affine* __restrict__ P, size_t m,
-                                                                               const DeviceTables* __restrict__ T, uint8_t* __restrict__ verdicts) {
+                                                                               const DeviceTables* __restrict__ T, const LineCoeffs* __restrict__ lines_b,
+                                                                               uint8_t* __restrict__ verdicts) {
     extern __shared__ __align__(16) unsigned char dyn_smem[];
     ManyWarpSmem& S = *reinterpret_cast<ManyWarpSmem*>(dyn_smem);
     vliw::Tables tab = vliw::load_tables(&S.stab, threadIdx.x, blockDim.x);
@@ -21,7 +22,7 @@ __global__ void __launch_bounds__(32 * kManyWarps, 1) many_pairing_warp_kernel(c
         if (verdicts[i] != kPending) continue;                            // warp-uniform
         G1Affine x = X[i], np = P[i];
         if (!np.inf) np.y = np.y.neg();
-        bool ok = vliw::coop_pairing_product_is_one(regs, x, T->pairing.g2_gen, np, T->pairing.tau_g2, L);
+        bool ok = vliw::coop_pairing_product_is_one(regs, x, T->pairing.g2_gen, np, lines_b ? lines_b : T->pairing.tau_g2, L);
         __syncwarp();
         if (lane == 0) verdicts[i] = ok ? kTrue : kFalse;
     }

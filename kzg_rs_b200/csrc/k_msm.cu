@@ -16,12 +16,12 @@ namespace kzgb200 {
 // every bucket two contiguous index lists (low halves -> P_i, high halves -> -phi(P_i)); threads own buckets.
 __global__ void __launch_bounds__(128) msm_scalars_kernel(const Fr* __restrict__ z_mont, const ZY* __restrict__ zy, const Fr* __restrict__ r_mont,
                                                           uint64_t offset, int n, uint8_t* __restrict__ digits /* [4*16][n] */,
-                                                          Fr* __restrict__ ry) {
+                                                          Fr* __restrict__ ry, const Fr* __restrict__ weights) {
     int i = blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= n) return;
     uint64_t e = offset + (uint64_t)i;
     uint32_t ee[2] = {(uint32_t)e, (uint32_t)(e >> 32)};
-    Fr ri = r_mont->pow(ee, 64);              // r^(offset+i), Montgomery   (compute_powers, kzg_proof.rs:279-289)
+    Fr ri = weights ? weights[i] : r_mont->pow(ee, 64);   // r^(offset+i), Montgomery (compute_powers, kzg_proof.rs:279-289), or the caller's weight
     Fr ri_raw = ri.to_raw();
     Fr rz_raw = (ri * z_mont[i]).to_raw();    // r_i z_i   (kzg_proof.rs:425)
     ry[i] = ri * zy[i].y;                     // r_i y_i in normal form

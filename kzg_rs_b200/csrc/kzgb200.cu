@@ -4,6 +4,8 @@
 // ordering on the host, every field / curve / pairing operation and every per-blob hash in a kernel.  The one serial hash of
 // the path -- the batch transcript of compute_r_powers (:291-348) -- is hashed by the host behind the kernels (host_sha256.cpp).
 // No CPU fallback: CUDA failures surface as KZGB200_INTERNAL_ERROR.
+#include <algorithm>
+#include <chrono>
 #include <new>
 #include "runtime.cuh"
 
@@ -387,10 +389,10 @@ static int msm_slice_len(const kzgb200_ctx* ctx, int n) {
     return slice < kMinSlice ? kMinSlice : slice;
 }
 // K6: digits, counting sort, buckets, window sums, Horner -> partial (optionally stored into a peer's exchange buffer + flag)
-int launch_lincomb(kzgb200_ctx* ctx, size_t offset, Partial* d_out, bool wait_subgroup, uint32_t* d_flag, uint32_t epoch) {
+int launch_lincomb(kzgb200_ctx* ctx, size_t offset, Partial* d_out, bool wait_subgroup, uint32_t* d_flag, uint32_t epoch, const Fr* d_weights) {
     int n = (int)ctx->cur_n;
     phase_begin(ctx, kPhLincomb, ctx->stream);
-    msm_scalars_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_z_mont, ctx->d_zy, ctx->d_r, (uint64_t)offset, n, ctx->d_digits, ctx->d_ry);
+    msm_scalars_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_z_mont, ctx->d_zy, ctx->d_r, (uint64_t)offset, n, ctx->d_digits, ctx->d_ry, d_weights);
     msm_sort_kernel<<<kDigitRows, 256, 0, ctx->stream>>>(ctx->d_digits, n, ctx->d_order, ctx->d_start);
     {
         const int slice = msm_slice_len(ctx, n);
@@ -541,13 +543,15 @@ extern "C" const char* kzgb200_last_error(const kzgb200_ctx* ctx) { return ctx ?
 // per tuple of the many-tuple path: 3 affine points, a status word, 160 input bytes, a verdict byte (rounded up)
 constexpr size_t kManyBytesPerTuple = 3 * sizeof(G1Affine) + 4 + 160 + 4;
 // the pairing checks of m parsed tuples: kManyGroups per CTA in lockstep (kManyCtasPerSm persistent CTAs per SM), then the rare identity inputs
-static int launch_many_pairings(kzgb200_ctx* ctx, const G1Affine* X, const G1Affine* P, const uint32_t* status, size_t m, uint8_t* dv) {
+// (lines_b: the second G2 point's line table, nullptr = [tau]G2)
+static int launch_many_pairings(kzgb200_ctx* ctx, const G1Affine* X, const G1Affine* P, const uint32_t* status, size_t m, uint8_t* dv,
+                                const LineCoeffs* lines_b = nullptr) {
     size_t nbatch = (m + kManyGroups - 1) / kManyGroups;
     const size_t slots = (size_t)ctx->num_sms * kManyCtasPerSm;
     unsigned grid = (unsigned)(nbatch < slots ? nbatch : slots);
-    many_pairing_kernel<<<grid, kManyThreads, kManySmemBytes, ctx->stream>>>(X, P, status, m, ctx->tables, dv);
+    many_pairing_kernel<<<grid, kManyThreads, kManySmemBytes, ctx->stream>>>(X, P, status, m, ctx->tables, lines_b, dv);
     size_t nw = (m + kManyWarps - 1) / kManyWarps;
-    many_pairing_warp_kernel<<<(unsigned)(nw < (size_t)ctx->num_sms ? nw : (size_t)ctx->num_sms), 32 * kManyWarps, kManySmemBytes, ctx->stream>>>(X, P, m, ctx->tables, dv);
+    many_pairing_warp_kernel<<<(unsigned)(nw < (size_t)ctx->num_sms ? nw : (size_t)ctx->num_sms), 32 * kManyWarps, kManySmemBytes, ctx->stream>>>(X, P, m, ctx->tables, lines_b, dv);
     CK(cudaGetLastError());
     return KZGB200_OK;
 }
@@ -985,7 +989,8 @@ static void proof_destroy(CellCtx* c) {
 static void cell_destroy(kzgb200_ctx* ctx) {
     CellCtx* c = ctx->cells;
     if (!c) return;
-    void* d[] = {c->tables, c->d_cells, c->d_p, c->d_uc, c->d_meta, c->d_ustatus, c->d_U, c->d_rk, c->d_agg, c->d_coeffs, c->d_part, c->d_ext};
+    void* d[] = {c->tables, c->d_cells, c->d_p, c->d_uc, c->d_meta, c->d_ustatus, c->d_U, c->d_rk, c->d_agg, c->d_coeffs, c->d_part, c->d_ext,
+                 c->d_goff, c->d_gbad, c->d_fmeta, c->d_rg, c->d_gv, c->d_terms, c->d_AB, c->d_gX, c->d_rcoef};
     for (void* p : d) if (p) cudaFree(p);
     void* h[] = {c->h_meta, c->h_uc, c->h_c, c->h_cells, c->h_p, c->h_idx};
     for (void* p : h) if (p) cudaFreeHost(p);
@@ -1202,6 +1207,298 @@ extern "C" int kzgb200_verify_cell_kzg_proof_batch_device(kzgb200_ctx* ctx, cons
     CK(cudaMemcpyAsync(c->h_cells, d_cells, n * kBytesPerCell, cudaMemcpyDeviceToHost, ctx->s_d2h));
     CK(cudaStreamSynchronize(ctx->s_d2h));
     return cell_verify_locked(ctx, c->h_c, c->h_idx, c->h_cells, c->h_p, d_cells, d_proofs, n, ok, false);
+}
+
+// ---- verify_cell_kzg_proof_batch_many: k independent cell batches (groups), one verdict each ---------------------------------
+// The spec's check of a group is linear in its per-cell weights r^j.  With w = rho^g r_g^j on the cells of group g, all groups are
+// checked at once by the single-call pipeline above (one MSM, one pairing); only if that fails is every group checked on its own
+// (many_*_kernel, k_cells.cu, and one pairing check per group on the many-check engine).  Each r_g is the spec's challenge of
+// group g alone: its own transcript with its own deduplication of commitments, hashed by a small pool of host threads.
+
+// x mod q for a 32-byte big-endian x (hash_to_bls_field): x < 2^256 < 3q, at most two subtractions
+static void fr_reduce_be(uint8_t v[32]) {
+    static const uint8_t q[32] = {0x73, 0xed, 0xa7, 0x53, 0x29, 0x9d, 0x7d, 0x48, 0x33, 0x39, 0xd8, 0x08, 0x09, 0xa1, 0xd8, 0x05,
+                                  0x53, 0xbd, 0xa4, 0x02, 0xff, 0xfe, 0x5b, 0xfe, 0xff, 0xff, 0xff, 0xff, 0x00, 0x00, 0x00, 0x01};
+    while (memcmp(v, q, 32) >= 0) {
+        int borrow = 0;
+        for (int i = 31; i >= 0; i--) {
+            const int d = (int)v[i] - (int)q[i] - borrow;
+            borrow = d < 0;
+            v[i] = (uint8_t)(d + (borrow ? 256 : 0));
+        }
+    }
+}
+static void put_be64(uint8_t* p, uint64_t v) { for (int i = 0; i < 8; i++) p[i] = (uint8_t)(v >> (56 - 8 * i)); }
+// what the hasher threads read: the globally deduplicated commitments (uc, cidx: see cell_plan) and the caller's host inputs
+struct ManyHashJob {
+    const uint8_t *uc, *cells, *proofs;
+    const uint32_t* cidx;
+    const uint64_t *idx, *off;
+    size_t m;
+};
+// r_g of groups [g0, g1) -> rg + 32 g: the group's commitments deduplicated in first-occurrence order within the group (the global
+// indices mapped to local ones), then cell_transcript as for a single call; an empty group gets 32 zero bytes
+static void many_hash_range(const ManyHashJob* J, size_t g0, size_t g1, uint8_t* rg) {
+    std::vector<size_t> seen(J->m, SIZE_MAX);
+    std::vector<uint32_t> local(J->m), lcidx;
+    std::vector<uint8_t> luc;
+    for (size_t g = g0; g < g1; g++) {
+        const size_t lo = J->off[g], cnt = J->off[g + 1] - lo;
+        if (!cnt) { memset(rg + 32 * g, 0, 32); continue; }
+        luc.clear();
+        lcidx.resize(cnt);
+        uint32_t lm = 0;
+        for (size_t e = 0; e < cnt; e++) {
+            const uint32_t u = J->cidx[lo + e];
+            if (seen[u] != g) { seen[u] = g; local[u] = lm++; luc.insert(luc.end(), J->uc + 48 * (size_t)u, J->uc + 48 * (size_t)u + 48); }
+            lcidx[e] = local[u];
+        }
+        cell_transcript(rg + 32 * g, luc.data(), lm, lcidx.data(), J->idx + lo, J->cells + lo * kBytesPerCell, J->proofs + 48 * lo, cnt);
+        fr_reduce_be(rg + 32 * g);
+    }
+}
+// rho = SHA-256("RCKZGCMANY___V1_" | u64be k | per group: u64be n_g | r_g (32 zero bytes if n_g = 0)) mod q; 0 -> 1
+static void many_rho(const uint8_t* rg, const uint64_t* off, size_t k, uint8_t rho[32]) {
+    HostSha256 s;
+    host_sha256_init(&s);
+    uint8_t hdr[24] = {'R', 'C', 'K', 'Z', 'G', 'C', 'M', 'A', 'N', 'Y', '_', '_', '_', 'V', '1', '_'};
+    put_be64(hdr + 16, k);
+    host_sha256_update(&s, hdr, 24);
+    for (size_t g = 0; g < k; g++) {
+        uint8_t e[40];
+        put_be64(e, off[g + 1] - off[g]);
+        memcpy(e + 8, rg + 32 * g, 32);
+        host_sha256_update(&s, e, 40);
+    }
+    host_sha256_final(&s, rho);
+    fr_reduce_be(rho);
+    uint8_t o = 0;
+    for (int i = 0; i < 32; i++) o |= rho[i];
+    if (!o) rho[31] = 1;
+}
+template <class T>
+static cudaError_t grow(T*& p, size_t& cap, size_t count) {
+    if (count <= cap) return cudaSuccess;
+    cap = 0;
+    cudaError_t e = regrow(p, count);
+    if (e == cudaSuccess) cap = count;
+    return e;
+}
+// the per-group checks (only when the combined check fails): verdicts for every group from the parsed points, the weights and
+// gbad of the combined check (all still on the device)
+static int cell_many_fallback(kzgb200_ctx* ctx, const uint8_t* d_cells, size_t n, const uint64_t* off, const std::vector<uint32_t>& goff,
+                              const std::vector<uint32_t>& gbad, size_t k, uint8_t* verdicts) {
+    CellCtx* c = ctx->cells;
+    const uint32_t* meta = c->h_meta;                 // [cell index | unique commitment | cells ordered by index | start]
+    // the cells of every group ordered by index (a stable pass over the global order), and its runs of one index
+    std::vector<uint32_t> cgroup(n), cur(goff.begin(), goff.end() - 1), ord(n), rstart, ridx, grun(k + 1);
+    for (size_t g = 0; g < k; g++) for (size_t i = off[g]; i < off[g + 1]; i++) cgroup[i] = (uint32_t)g;
+    for (size_t p = 0; p < n; p++) { const uint32_t i = meta[2 * n + p]; ord[cur[cgroup[i]]++] = i; }
+    for (size_t g = 0; g < k; g++) {
+        grun[g] = (uint32_t)ridx.size();
+        if (gbad[g]) continue;                        // weights 0: no runs
+        for (uint32_t p = goff[g]; p < goff[g + 1]; p++)
+            if (p == goff[g] || meta[ord[p]] != meta[ord[p - 1]]) { rstart.push_back(p); ridx.push_back(meta[ord[p]]); }
+    }
+    const size_t runs = ridx.size();
+    grun[k] = (uint32_t)runs;
+    std::vector<uint32_t> fmeta;
+    fmeta.reserve(n + 2 * runs + k + 2);
+    fmeta.insert(fmeta.end(), ord.begin(), ord.end());
+    fmeta.insert(fmeta.end(), rstart.begin(), rstart.end());
+    fmeta.push_back((uint32_t)n);
+    fmeta.insert(fmeta.end(), ridx.begin(), ridx.end());
+    fmeta.insert(fmeta.end(), grun.begin(), grun.end());
+    CK(grow(c->d_fmeta, c->fmeta_cap, fmeta.size()));
+    CK(grow(c->d_terms, c->terms_cap, 2 * n));
+    CK(grow(c->d_rcoef, c->rcoef_cap, (runs ? runs : 1) * kFieldElementsPerCell));
+    const int ni = (int)n, ri = (int)runs;
+    const unsigned kg = (unsigned)k;
+    phase_begin(ctx, 7, ctx->stream);
+    CK(cudaMemcpyAsync(c->d_fmeta, fmeta.data(), fmeta.size() * 4, cudaMemcpyHostToDevice, ctx->stream));
+    many_terms_kernel<<<(ni + 127) / 128, 128, 0, ctx->stream>>>(ni, c->d_rk, ctx->d_z_mont, ctx->d_C, ctx->d_P, c->d_terms);
+    many_group_sums_kernel<<<kg, 128, 0, ctx->stream>>>(c->d_goff, c->d_terms, c->d_AB);
+    if (ri) many_run_interp_kernel<<<ri, kFieldElementsPerCell, 0, ctx->stream>>>(d_cells, c->d_fmeta, ni, ri, c->d_rk, c->tables, c->d_rcoef);
+    many_group_rli_kernel<<<kg, 256, 0, ctx->stream>>>(c->d_rcoef, c->d_fmeta + n + 2 * runs + 1, c->d_AB, c->tables, c->d_gX, c->d_gX + k);
+    CK(cudaGetLastError());
+    int rc = launch_many_pairings(ctx, c->d_gX, c->d_gX + k, c->d_gbad, k, c->d_gv, c->tables->tau64_lines);
+    if (rc) return rc;
+    phase_end(ctx, 7, ctx->stream);
+    CK(cudaMemcpyAsync(verdicts, c->d_gv, k, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    for (size_t g = 0; g < k; g++) if (off[g] == off[g + 1]) verdicts[g] = kTrue;
+    return KZGB200_OK;
+}
+
+// n = off[k] >= 1 cells in k groups.  hc / hidx / hcells / hp, d_cells / d_p, copy_inputs: as cell_verify_locked.
+static int cell_many_locked(kzgb200_ctx* ctx, const uint8_t* hc, const uint64_t* hidx, const uint8_t* hcells, const uint8_t* hp,
+                            const uint8_t* d_cells, const uint8_t* d_p, const uint64_t* off, size_t k, uint8_t* verdicts, bool copy_inputs) {
+    CellCtx* c = ctx->cells;
+    const size_t n = off[k];
+    // an index >= 128 fails its group's first assertion; the plan sees index 0 in its place (the group's weights are 0)
+    std::vector<uint32_t> goff(k + 1), gbad(k, 0);
+    std::vector<uint64_t> sidx;
+    for (size_t g = 0; g < k; g++) {
+        goff[g] = (uint32_t)off[g];
+        for (size_t i = off[g]; i < off[g + 1]; i++) if (hidx[i] >= (uint64_t)kCellsPerExtBlob) { gbad[g] = kErrScalar; break; }
+        if (gbad[g]) {
+            if (sidx.empty()) sidx.assign(hidx, hidx + n);
+            for (size_t i = off[g]; i < off[g + 1]; i++) sidx[i] = 0;
+        }
+    }
+    goff[k] = (uint32_t)n;
+    const size_t m = cell_plan(c, hc, sidx.empty() ? hidx : sidx.data(), n);
+    if (k > c->gcap) {
+        CK(regrow(c->d_goff, k + 1)); CK(regrow(c->d_gbad, k)); CK(regrow(c->d_rg, 32 * (k + 1))); CK(regrow(c->d_gv, k));
+        CK(regrow(c->d_AB, 2 * k)); CK(regrow(c->d_gX, 2 * k));
+        c->gcap = k;
+    }
+    c->many_done = false;
+    c->many_rg.assign(32 * (k + 1), 0);
+    uint8_t* rg = c->many_rg.data();
+    // the k transcripts on up to 16 host threads, each a contiguous range of groups of about n / threads cells, while the GPU parses
+    const ManyHashJob job{c->h_uc, hcells, hp, c->h_meta + n, hidx, off, m};
+    const size_t hw = std::max<size_t>(1, std::thread::hardware_concurrency()), nt = std::min<size_t>({k, hw, 16});
+    const auto t0 = std::chrono::steady_clock::now();
+    std::vector<std::thread> pool;
+    for (size_t t = 0, g = 0; t < nt && g < k; t++) {
+        size_t g1 = g + 1;
+        const uint64_t target = (uint64_t)((unsigned __int128)n * (t + 1) / nt);
+        while (g1 < k && off[g1 + 1] <= target) g1++;
+        if (t + 1 == nt) g1 = k;
+        pool.emplace_back(many_hash_range, &job, g, g1, rg);
+        g = g1;
+    }
+    const int ni = (int)n, mi = (int)m, ki = (int)k;
+    int rc = [&]() -> int {
+        for (int i = 0; i < 8; i++) ctx->ph_started[i] = false;
+        CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_parse, 0));
+        CK(cudaMemsetAsync(ctx->d_status, 0, n * sizeof(uint32_t), ctx->stream));
+        CK(cudaMemsetAsync(c->d_ustatus, 0, m * sizeof(uint32_t), ctx->stream));
+        CK(cudaMemcpyAsync(c->d_meta, c->h_meta, (3 * n + kCellsPerExtBlob + 1) * 4, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(c->d_uc, c->h_uc, m * 48, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(c->d_goff, goff.data(), (k + 1) * 4, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(c->d_gbad, gbad.data(), k * 4, cudaMemcpyHostToDevice, ctx->stream));
+        if (copy_inputs) {
+            CK(cudaMemcpyAsync(c->d_p, hp, n * 48, cudaMemcpyHostToDevice, ctx->stream));
+            CK(cudaMemcpyAsync(c->d_cells, hcells, n * kBytesPerCell, cudaMemcpyHostToDevice, ctx->stream));
+            d_cells = c->d_cells; d_p = c->d_p;
+        }
+        phase_begin(ctx, kPhParse, ctx->stream);
+        cell_points_kernel<<<(mi + 127) / 128, 128, 0, ctx->stream>>>(c->d_uc, mi, c->d_U, c->d_ustatus, kErrCommitment);
+        cell_points_kernel<<<(ni + 127) / 128, 128, 0, ctx->stream>>>(d_p, ni, ctx->d_P, ctx->d_status, kErrProof);
+        cell_check_kernel<<<(unsigned)(((size_t)n * kFieldElementsPerCell + 255) / 256), 256, 0, ctx->stream>>>(d_cells, ni, ctx->d_status);
+        cell_scalars_kernel<<<(ni + 127) / 128, 128, 0, ctx->stream>>>(c->d_meta, ni, c->d_U, c->d_ustatus, c->tables, ctx->d_z_mont, ctx->d_zy,
+                                                                        ctx->d_C, ctx->d_status);
+        many_group_status_kernel<<<(ni + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_status, ni, c->d_goff, ki, c->d_gbad);
+        phase_end(ctx, kPhParse, ctx->stream);
+        CK(cudaGetLastError());
+        return KZGB200_OK;
+    }();
+    for (auto& t : pool) t.join();
+    const float hash_ms = std::chrono::duration<float, std::milli>(std::chrono::steady_clock::now() - t0).count();
+    if (rc) return rc;
+    many_rho(rg, off, k, rg + 32 * k);
+    c->many_k = k;
+    c->many_done = true;
+    // the combined check: the single-call pipeline with the weights (in d_rk) in place of r^k
+    phase_begin(ctx, kPhTranscript, ctx->stream);
+    CK(cudaMemcpyAsync(c->d_rg, rg, 32 * (k + 1), cudaMemcpyHostToDevice, ctx->stream));
+    many_weights_kernel<<<(ni + 127) / 128, 128, 0, ctx->stream>>>(ni, c->d_goff, ki, c->d_rg, c->d_gbad, c->d_rk, ctx->d_status);
+    phase_end(ctx, kPhTranscript, ctx->stream);
+    CK(cudaEventRecord(c->ev_r, ctx->stream));
+    CK(cudaStreamWaitEvent(ctx->s_aux, c->ev_r, 0));
+    cell_agg_kernel<<<dim3(kCellsPerExtBlob, kCellAggSlices), kFieldElementsPerCell, 0, ctx->s_aux>>>(d_cells, c->d_meta, ni, c->d_rk, c->d_agg);
+    cell_interp_kernel<<<kCellsPerExtBlob, kFieldElementsPerCell, 0, ctx->s_aux>>>(c->d_agg, c->d_meta, ni, c->tables, c->d_coeffs);
+    cell_rli_kernel<<<1, 256, 0, ctx->s_aux>>>(c->d_coeffs, c->tables, c->d_part + 1);
+    CK(cudaGetLastError());
+    CK(cudaEventRecord(c->ev_rli, ctx->s_aux));
+    ctx->cur_c = nullptr; ctx->cur_p = d_p; ctx->cur_n = n; ctx->subgroup_pending = false;
+    if ((rc = launch_lincomb(ctx, 0, c->d_part, false, nullptr, 0, c->d_rk))) return rc;
+    CK(cudaStreamWaitEvent(ctx->stream, c->ev_rli, 0));
+    phase_begin(ctx, kPhFinal, ctx->stream);
+    launch_batch_final(ctx->stream, c->d_part, 2, ctx->tables, ctx->d_result, ctx->d_scratch, false, c->tables->lines29);
+    phase_end(ctx, kPhFinal, ctx->stream);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(gbad.data(), c->d_gbad, k * 4, cudaMemcpyDeviceToHost, ctx->stream));
+    int ok = 0;
+    rc = read_result(ctx, &ok);
+    if (rc != KZGB200_OK && rc != KZGB200_BAD_ARGS) return rc;
+    if (rc == KZGB200_OK && ok) for (size_t g = 0; g < k; g++) verdicts[g] = gbad[g] ? kBadArgs : kTrue;
+    else if ((rc = cell_many_fallback(ctx, d_cells, n, off, goff, gbad, k, verdicts))) return rc;
+    collect_phase_times(ctx);
+    ctx->phase_ms[1] = hash_ms;
+    ctx->phase_ms[2] = (float)pool.size();
+    return KZGB200_OK;
+}
+// argument checks shared by both forms; n_out = the number of cells
+static int many_args(kzgb200_ctx* ctx, const void* a, const void* b, const void* cc, const void* d, const uint64_t* off, size_t k,
+                     const uint8_t* verdicts, size_t* n_out) {
+    if (!ctx || (k && (!off || !verdicts)) || k > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
+    size_t n = 0;
+    if (k) {
+        if (off[0] != 0) return KZGB200_BAD_ARGS;
+        for (size_t g = 0; g < k; g++) if (off[g + 1] < off[g] || off[g + 1] > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
+        n = off[k];
+    }
+    if (n && (!a || !b || !cc || !d)) return KZGB200_BAD_ARGS;
+    if (!ctx->cells) return KZGB200_INVALID_SETUP;
+    *n_out = n;
+    return KZGB200_OK;
+}
+// a call without cells: every group is empty (true); r_g = 0 and rho as for any call
+static void many_empty(kzgb200_ctx* ctx, const uint64_t* off, size_t k, uint8_t* verdicts) {
+    CellCtx* c = ctx->cells;
+    c->many_rg.assign(32 * (k + 1), 0);
+    many_rho(c->many_rg.data(), off, k, c->many_rg.data() + 32 * k);
+    c->many_k = k;
+    c->many_done = true;
+    if (k) memset(verdicts, kTrue, k);
+}
+
+extern "C" int kzgb200_verify_cell_kzg_proof_batch_many(kzgb200_ctx* ctx, const uint8_t* commitments, const uint64_t* cell_indices, const uint8_t* cells,
+                                                        const uint8_t* proofs, const uint64_t* group_offsets, size_t n_groups, uint8_t* verdicts) {
+    size_t n = 0;
+    int rc = many_args(ctx, commitments, cell_indices, cells, proofs, group_offsets, n_groups, verdicts, &n);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    if (n == 0) { many_empty(ctx, group_offsets, n_groups, verdicts); return KZGB200_OK; }
+    DeviceGuard dev(ctx->device);
+    if ((rc = cell_capacity(ctx, n, true, false))) return rc;
+    return cell_many_locked(ctx, commitments, cell_indices, cells, proofs, nullptr, nullptr, group_offsets, n_groups, verdicts, true);
+}
+
+extern "C" int kzgb200_verify_cell_kzg_proof_batch_many_device(kzgb200_ctx* ctx, const uint8_t* d_commitments, const uint64_t* d_cell_indices,
+                                                               const uint8_t* d_cells, const uint8_t* d_proofs, const uint64_t* group_offsets,
+                                                               size_t n_groups, uint8_t* verdicts) {
+    size_t n = 0;
+    int rc = many_args(ctx, d_commitments, d_cell_indices, d_cells, d_proofs, group_offsets, n_groups, verdicts, &n);
+    if (rc) return rc;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    if (n == 0) { many_empty(ctx, group_offsets, n_groups, verdicts); return KZGB200_OK; }
+    DeviceGuard dev(ctx->device);
+    if ((rc = cell_capacity(ctx, n, false, true))) return rc;
+    CellCtx* c = ctx->cells;
+    // the exact transcripts are host chains over every input byte: the inputs come back to pinned memory once
+    CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_parse, 0));
+    CK(cudaMemcpyAsync(c->h_idx, d_cell_indices, n * 8, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaMemcpyAsync(c->h_c, d_commitments, n * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaMemcpyAsync(c->h_p, d_proofs, n * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaMemcpyAsync(c->h_cells, d_cells, n * kBytesPerCell, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaStreamSynchronize(ctx->s_d2h));
+    return cell_many_locked(ctx, c->h_c, c->h_idx, c->h_cells, c->h_p, d_cells, d_proofs, group_offsets, n_groups, verdicts, false);
+}
+
+// test hook: r_g of every group of the last _many call (zeros for empty groups) and rho, canonical big-endian
+extern "C" int kzgb200_last_cell_many_r(kzgb200_ctx* ctx, uint8_t* r_out, size_t n_groups, uint8_t* rho_out32) {
+    if (!ctx || !rho_out32 || (n_groups && !r_out)) return KZGB200_BAD_ARGS;
+    if (!ctx->cells) return KZGB200_INVALID_SETUP;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    CellCtx* c = ctx->cells;
+    if (!c->many_done || n_groups != c->many_k) return KZGB200_BAD_ARGS;
+    if (n_groups) memcpy(r_out, c->many_rg.data(), 32 * n_groups);
+    memcpy(rho_out32, c->many_rg.data() + 32 * n_groups, 32);
+    return KZGB200_OK;
 }
 
 static int compute_cells_locked(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8_t* d_out) {

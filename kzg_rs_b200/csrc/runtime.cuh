@@ -72,6 +72,17 @@ struct CellCtx {
     int* d_pos = nullptr;                                          // recovery: input position of each cell index (-1: missing)
     uint32_t* d_missing = nullptr;
     Fr* d_z = nullptr;                                             // see recover_z_kernel
+    // verify_cell_kzg_proof_batch_many: per-group buffers for gcap groups, the fallback's workspace (per cell, per (group, index)
+    // run), and the last call's r_g (32 bytes each, canonical big-endian) followed by rho
+    size_t gcap = 0, fmeta_cap = 0, terms_cap = 0, rcoef_cap = 0;
+    uint32_t *d_goff = nullptr, *d_gbad = nullptr, *d_fmeta = nullptr;   // group offsets (k + 1), BadArgs flags (k), see many_run_interp_kernel
+    uint8_t *d_rg = nullptr, *d_gv = nullptr;                      // r_g and rho (k + 1 x 32 bytes), fallback verdicts (k)
+    G1 *d_terms = nullptr, *d_AB = nullptr;                        // fallback: per-cell terms (2 per cell), per-group A_g, B'_g
+    G1Affine* d_gX = nullptr;                                      // fallback: X_g (k), then A_g (k)
+    Fr* d_rcoef = nullptr;                                         // fallback: interpolated coefficients per run (64 each)
+    std::vector<uint8_t> many_rg;
+    size_t many_k = 0;
+    bool many_done = false;
 };
 
 }  // namespace kzgb200
@@ -194,7 +205,9 @@ int transcript_progress(kzgb200_ctx* ctx, bool block);
 int transcript_finish(kzgb200_ctx* ctx);
 // upload a 32-byte transcript digest computed elsewhere (multi-GPU: the group leader) and derive r from it
 int upload_r_digest(kzgb200_ctx* ctx, const uint8_t digest[32]);
-int launch_lincomb(kzgb200_ctx* ctx, size_t offset, Partial* d_out, bool wait_subgroup, uint32_t* d_flag = nullptr, uint32_t epoch = 0);
+// d_weights: per-entry scalars in place of r^(offset + i) (cell groups), nullptr = the powers of r
+int launch_lincomb(kzgb200_ctx* ctx, size_t offset, Partial* d_out, bool wait_subgroup, uint32_t* d_flag = nullptr, uint32_t epoch = 0,
+                   const Fr* d_weights = nullptr);
 int read_result(kzgb200_ctx* ctx, int* ok);
 int export_zy(kzgb200_ctx* ctx, size_t n, uint8_t* d_z, uint8_t* d_y);
 void phase_begin(kzgb200_ctx* ctx, int ph, cudaStream_t st);

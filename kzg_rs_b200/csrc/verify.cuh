@@ -48,29 +48,31 @@ KZG_NI G1Affine kzg_lhs_point(const G1Affine& C, const Fr& z_raw, const Fr& y_ra
     acc = acc.add(scalar_mul_affine(pi, z_raw.l, 255));
     return g1_to_affine(acc);
 }
+// [k]P by the GLV split k = k1 + k2 x^2 (glv.cuh) with Shamir's trick over {P, -phi(P), P - phi(P)}: 128 doublings and ~96
+// additions instead of 2 x (255 + 128).  k: canonical raw limbs.
+KZG_HD G1 glv_mul(const G1Affine& p, const Fr& k_raw) {
+    uint32_t k1[4], k2[4];
+    glv_split(k_raw.l, k1, k2);
+    G1Affine q = glv_endo_neg(p);
+    G1 both = G1::from_affine(p).add_mixed(q), acc = G1::identity();
+    for (int i = 127; i >= 0; i--) {
+        acc = acc.dbl();
+        uint32_t b1 = (k1[i >> 5] >> (i & 31)) & 1u, b2 = (k2[i >> 5] >> (i & 31)) & 1u;
+        if (b1 & b2) acc = acc.add(both);
+        else if (b1) acc = acc.add_mixed(p);
+        else if (b2) acc = acc.add_mixed(q);
+    }
+    return acc;
+}
 // The same point for the batched per-tuple path (BASELINE config 5): [y]G from the fixed-base table of the generator
-// (gen_table[w][d-1] = [d 16^w]G: 64 mixed additions, no doublings) and [z]pi by the GLV split z = k1 + k2 x^2 (glv.cuh) with
-// Shamir's trick over {pi, -phi(pi), pi - phi(pi)}: 128 doublings and ~96 additions instead of 2 x (255 + 128).
+// (gen_table[w][d-1] = [d 16^w]G: 64 mixed additions, no doublings) and [z]pi by glv_mul.
 KZG_NI G1 kzg_lhs_point_fast(const G1Affine& C, const Fr& z_raw, const Fr& y_raw, const G1Affine& pi, const G1Affine (*gen_table)[15]) {
     G1 acc = G1::from_affine(C);
     for (int w = 0; w < 64; w++) {
         uint32_t d = (y_raw.l[w >> 3] >> (4 * (w & 7))) & 15u;
         if (d) { G1Affine t = gen_table[w][d - 1]; t.y = t.y.neg(); acc = acc.add_mixed(t); }
     }
-    if (!pi.inf) {
-        uint32_t k1[4], k2[4];
-        glv_split(z_raw.l, k1, k2);
-        G1Affine q = glv_endo_neg(pi);
-        G1 both = G1::from_affine(pi).add_mixed(q), zp = G1::identity();
-        for (int i = 127; i >= 0; i--) {
-            zp = zp.dbl();
-            uint32_t b1 = (k1[i >> 5] >> (i & 31)) & 1u, b2 = (k2[i >> 5] >> (i & 31)) & 1u;
-            if (b1 & b2) zp = zp.add(both);
-            else if (b1) zp = zp.add_mixed(pi);
-            else if (b2) zp = zp.add_mixed(q);
-        }
-        acc = acc.add(zp);
-    }
+    if (!pi.inf) acc = acc.add(glv_mul(pi, z_raw));
     return acc;
 }
 // parse order z, y, commitment, proof as kzg_proof.rs:360-383
