@@ -190,7 +190,7 @@ int kzgb200_compute_blob_kzg_proof_batch(kzgb200_ctx* ctx, const uint8_t* d_blob
  *   n == 0 -> Ok(true); an index >= 128, a non-canonical cell element, or a commitment / proof that is not a valid compressed
  *   point of the G1 subgroup -> KZGB200_BAD_ARGS.  The batch challenge r is the spec's (commitments deduplicated by their bytes),
  *   hashed by a host thread over the caller's buffers while the GPU parses the inputs; kzgb200_last_r returns it afterwards.
- *   The _device form takes device pointers; the inputs are copied back to pinned host memory once for the hash.
+ *   The call is the one-group case of kzgb200_verify_cell_kzg_proof_batch_many below.  The _device form takes device pointers; the inputs are copied back to pinned host memory once for the hash.
  * kzgb200_compute_cells: the 128 cells of one host blob (cells_out: 128 x 2048 bytes, host);
  * kzgb200_compute_cells_batch_device: n device blobs -> n x 128 cells (device, blob-major).  Non-canonical element -> BAD_ARGS. */
 int kzgb200_load_cell_setup(kzgb200_ctx* ctx, const uint8_t* g1_monomial48, size_t n_points, const uint8_t* g2_tau64_96);
@@ -215,15 +215,17 @@ int kzgb200_harness_generate_cells(kzgb200_ctx* ctx, uint64_t seed, size_t n_blo
  *   r_g is the spec's, hashed over that group's bytes alone (its own deduplication of commitments) by up to 16 host threads while
  *   the GPU parses.  All groups are checked together first (weights rho^g r_g^j, one MSM and one pairing; a false group passes it
  *   with probability <= n_groups / q); only if that fails does every group get its own check (one extra pass for any number of bad
- *   groups).  Returns BAD_ARGS only for a malformed call (a null pointer with n > 0 or n_groups > 0, bad offsets, n or n_groups
+ *   groups; with one group the combined check is that group's own, and there is no second pass).  Returns BAD_ARGS only for a malformed call (a null pointer with n > 0 or n_groups > 0, bad offsets, n or n_groups
  *   above 0x7fffffff / 2), INVALID_SETUP without the cell setup; n_groups == 0 -> OK.
  *   The _device form takes device pointers for the four data arrays (group_offsets and verdicts stay host memory); the inputs are
  *   copied back to pinned host memory once for the transcripts.
- *   kzgb200_get_phase_ms after a _many call: {parse, host hashing (wall ms, every call), hasher threads (every call), r_g upload and
- *   weights, lincomb, reduce, combined pairing, per-group fallback}; the device slots with kzgb200_set_profiling on.
- * kzgb200_last_cell_many_r: the last _many call's r_g (r_out: n_groups x 32, zeros for empty groups) and rho (rho_out32), canonical
- *   big-endian; n_groups must be that call's (else BAD_ARGS).  A _many call leaves what kzgb200_last_r and kzgb200_last_partial
- *   report untouched. */
+ *   kzgb200_get_phase_ms after any cell verification call (single or _many, either form): {parse, host hashing (wall ms, every
+ *   call), hasher threads (every call), r_g upload and weights, lincomb, reduce, combined pairing, per-group fallback}; the device
+ *   slots with kzgb200_set_profiling on.
+ * kzgb200_last_cell_many_r: r_g of the last cell verification call (a single call is one group; r_out: n_groups x 32, zeros for
+ *   empty groups) and rho (rho_out32), canonical big-endian; n_groups must be that call's (else BAD_ARGS).  A call with one group
+ *   sets what kzgb200_last_r reports to r_0, as the single call does; a call with more groups leaves it untouched.  No cell call
+ *   changes what kzgb200_last_partial reports. */
 int kzgb200_verify_cell_kzg_proof_batch_many(kzgb200_ctx* ctx, const uint8_t* commitments, const uint64_t* cell_indices, const uint8_t* cells,
                                              const uint8_t* proofs, const uint64_t* group_offsets, size_t n_groups, uint8_t* verdicts);
 int kzgb200_verify_cell_kzg_proof_batch_many_device(kzgb200_ctx* ctx, const uint8_t* d_commitments, const uint64_t* d_cell_indices,

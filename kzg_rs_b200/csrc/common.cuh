@@ -239,7 +239,6 @@ __global__ void cell_check_kernel(const uint8_t* __restrict__ cells, int n, uint
 __global__ void cell_scalars_kernel(const uint32_t* __restrict__ meta, int n, const G1Affine* __restrict__ U, const uint32_t* __restrict__ ustatus,
                                     const CellTables* __restrict__ T, Fr* __restrict__ z_mont, ZY* __restrict__ zy, G1Affine* __restrict__ C,
                                     uint32_t* __restrict__ status);
-__global__ void cell_rpow_kernel(const Fr* __restrict__ r_mont, int n, Fr* __restrict__ rk);
 __global__ void cell_agg_kernel(const uint8_t* __restrict__ cells, const uint32_t* __restrict__ meta, int n, const Fr* __restrict__ rk, Fr* __restrict__ agg);
 __global__ void cell_interp_kernel(const Fr* __restrict__ agg, const uint32_t* __restrict__ meta, int n, const CellTables* __restrict__ T,
                                    Fr* __restrict__ coeffs);

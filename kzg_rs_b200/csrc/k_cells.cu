@@ -174,14 +174,7 @@ __global__ void __launch_bounds__(128) cell_scalars_kernel(const uint32_t* __res
     C[k] = U[u];
     if (ustatus[u]) atomicOr(&status[k], kErrCommitment);
 }
-// r^k, Montgomery
-__global__ void __launch_bounds__(128) cell_rpow_kernel(const Fr* __restrict__ r_mont, int n, Fr* __restrict__ rk) {
-    const int k = blockIdx.x * blockDim.x + threadIdx.x;
-    if (k >= n) return;
-    const uint32_t e = (uint32_t)k;
-    rk[k] = r_mont->pow(&e, 32);
-}
-// r-weighted sums of the cell values per cell index: CTA (index i, slice s) sums its share of the cells with that index
+// weighted sums (rk: the per-cell weights) of the cell values per cell index: CTA (index i, slice s) sums its share of the cells with that index
 // (order / start: the cells grouped by index, built by the host); thread j = element j
 __global__ void __launch_bounds__(kFieldElementsPerCell) cell_agg_kernel(const uint8_t* __restrict__ cells, const uint32_t* __restrict__ meta, int n,
                                                                         const Fr* __restrict__ rk, Fr* __restrict__ agg) {
@@ -256,10 +249,10 @@ __global__ void __launch_bounds__(256) cell_rli_kernel(const Fr* __restrict__ co
     }
 }
 
-// ---- verify_cell_kzg_proof_batch_many: k independent groups of cells, one verdict each ------------------------------------
-// Group g = cells [goff[g], goff[g + 1]).  Every cell gets the weight w_k = rho^g r_g^j (j = its position in the group); the groups
-// are first checked together by the single-call pipeline with these weights in place of r^k, and only if that fails, each group on
-// its own (the fallback below).  gbad[g] != 0: group g fails an assertion of the spec (BadArgs).
+// ---- verify_cell_kzg_proof_batch[_many]: k independent groups of cells, one verdict each ----------------------------------
+// Group g = cells [goff[g], goff[g + 1]).  Every cell gets the weight w_k = rho^g r_g^j (j = its position in the group; with one
+// group, r^j); the groups are first checked together by the pipeline above with these weights, and only if that fails (and k > 1),
+// each group on its own (the fallback below).  gbad[g] != 0: group g fails an assertion of the spec (BadArgs).
 __device__ __forceinline__ uint32_t group_of(const uint32_t* __restrict__ goff, int k, uint32_t cell) {
     int lo = 0, hi = k - 1;                        // the last g with goff[g] <= cell (empty groups before it are skipped)
     while (lo < hi) { const int mid = (lo + hi + 1) >> 1; if (__ldg(goff + mid) <= cell) lo = mid; else hi = mid - 1; }

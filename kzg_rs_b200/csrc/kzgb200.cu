@@ -1117,103 +1117,11 @@ static void cell_transcript(uint8_t digest[32], const uint8_t* uc, size_t m, con
     host_sha256_final(&s, digest);
 }
 
-// verify_cell_kzg_proof_batch.  hc / hidx / hcells / hp: host copies (the caller's, or the pinned read-back of device inputs);
-// d_cells / d_p: the cells / proofs on the device.
-static int cell_verify_locked(kzgb200_ctx* ctx, const uint8_t* hc, const uint64_t* hidx, const uint8_t* hcells, const uint8_t* hp,
-                              const uint8_t* d_cells, const uint8_t* d_p, size_t n, int* ok, bool copy_inputs) {
-    CellCtx* c = ctx->cells;
-    for (size_t k = 0; k < n; k++) if (hidx[k] >= (uint64_t)kCellsPerExtBlob) return KZGB200_BAD_ARGS;
-    const size_t m = cell_plan(c, hc, hidx, n);
-    // the host hashes the transcript while the GPU parses
-    uint8_t digest[32];
-    std::thread hasher(cell_transcript, digest, c->h_uc, m, c->h_meta + n, hidx, hcells, hp, n);
-    const int ni = (int)n, mi = (int)m;
-    int rc = [&]() -> int {
-        for (int i = 0; i < 8; i++) ctx->ph_started[i] = false;
-        CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_parse, 0));       // a previous call's deferred subgroup checks still write status
-        CK(cudaMemsetAsync(ctx->d_status, 0, n * sizeof(uint32_t), ctx->stream));
-        CK(cudaMemsetAsync(c->d_ustatus, 0, m * sizeof(uint32_t), ctx->stream));
-        CK(cudaMemcpyAsync(c->d_meta, c->h_meta, (3 * n + kCellsPerExtBlob + 1) * 4, cudaMemcpyHostToDevice, ctx->stream));
-        CK(cudaMemcpyAsync(c->d_uc, c->h_uc, m * 48, cudaMemcpyHostToDevice, ctx->stream));
-        if (copy_inputs) {
-            CK(cudaMemcpyAsync(c->d_p, hp, n * 48, cudaMemcpyHostToDevice, ctx->stream));
-            CK(cudaMemcpyAsync(c->d_cells, hcells, n * kBytesPerCell, cudaMemcpyHostToDevice, ctx->stream));
-            d_cells = c->d_cells; d_p = c->d_p;
-        }
-        phase_begin(ctx, kPhParse, ctx->stream);
-        cell_points_kernel<<<(mi + 127) / 128, 128, 0, ctx->stream>>>(c->d_uc, mi, c->d_U, c->d_ustatus, kErrCommitment);
-        cell_points_kernel<<<(ni + 127) / 128, 128, 0, ctx->stream>>>(d_p, ni, ctx->d_P, ctx->d_status, kErrProof);
-        cell_check_kernel<<<(unsigned)(((size_t)n * kFieldElementsPerCell + 255) / 256), 256, 0, ctx->stream>>>(d_cells, ni, ctx->d_status);
-        cell_scalars_kernel<<<(ni + 127) / 128, 128, 0, ctx->stream>>>(c->d_meta, ni, c->d_U, c->d_ustatus, c->tables, ctx->d_z_mont, ctx->d_zy,
-                                                                        ctx->d_C, ctx->d_status);
-        phase_end(ctx, kPhParse, ctx->stream);
-        CK(cudaGetLastError());
-        return KZGB200_OK;
-    }();
-    hasher.join();
-    if (rc) return rc;
-    phase_begin(ctx, kPhTranscript, ctx->stream);
-    if ((rc = upload_r_digest(ctx, digest))) return rc;
-    phase_end(ctx, kPhTranscript, ctx->stream);
-    // RLI depends only on r: on the aux stream beside the big MSM
-    CK(cudaEventRecord(c->ev_r, ctx->stream));
-    CK(cudaStreamWaitEvent(ctx->s_aux, c->ev_r, 0));
-    cell_rpow_kernel<<<(ni + 127) / 128, 128, 0, ctx->s_aux>>>(ctx->d_r, ni, c->d_rk);
-    cell_agg_kernel<<<dim3(kCellsPerExtBlob, kCellAggSlices), kFieldElementsPerCell, 0, ctx->s_aux>>>(d_cells, c->d_meta, ni, c->d_rk, c->d_agg);
-    cell_interp_kernel<<<kCellsPerExtBlob, kFieldElementsPerCell, 0, ctx->s_aux>>>(c->d_agg, c->d_meta, ni, c->tables, c->d_coeffs);
-    cell_rli_kernel<<<1, 256, 0, ctx->s_aux>>>(c->d_coeffs, c->tables, c->d_part + 1);
-    CK(cudaGetLastError());
-    CK(cudaEventRecord(c->ev_rli, ctx->s_aux));
-    // LL and RLC + RLP: the blob batch's MSM with z_k = h_k^64, y_k = 0
-    ctx->cur_c = nullptr; ctx->cur_p = d_p; ctx->cur_n = n; ctx->subgroup_pending = false;
-    if ((rc = launch_lincomb(ctx, 0, c->d_part, false))) return rc;
-    CK(cudaStreamWaitEvent(ctx->stream, c->ev_rli, 0));
-    phase_begin(ctx, kPhFinal, ctx->stream);
-    launch_batch_final(ctx->stream, c->d_part, 2, ctx->tables, ctx->d_result, ctx->d_scratch, false, c->tables->lines29);
-    phase_end(ctx, kPhFinal, ctx->stream);
-    CK(cudaGetLastError());
-    rc = read_result(ctx, ok);
-    collect_phase_times(ctx);
-    return rc;
-}
-
-extern "C" int kzgb200_verify_cell_kzg_proof_batch(kzgb200_ctx* ctx, const uint8_t* commitments, const uint64_t* cell_indices, const uint8_t* cells,
-                                                   const uint8_t* proofs, size_t n, int* ok) {
-    if (!ctx || !ok || (n && (!commitments || !cell_indices || !cells || !proofs)) || n > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
-    if (!ctx->cells) return KZGB200_INVALID_SETUP;
-    if (n == 0) { *ok = 1; return KZGB200_OK; }
-    std::lock_guard<std::mutex> g(ctx->lock);
-    DeviceGuard dev(ctx->device);
-    int rc = cell_capacity(ctx, n, true, false);
-    if (rc) return rc;
-    return cell_verify_locked(ctx, commitments, cell_indices, cells, proofs, nullptr, nullptr, n, ok, true);
-}
-
-extern "C" int kzgb200_verify_cell_kzg_proof_batch_device(kzgb200_ctx* ctx, const uint8_t* d_commitments, const uint64_t* d_cell_indices,
-                                                          const uint8_t* d_cells, const uint8_t* d_proofs, size_t n, int* ok) {
-    if (!ctx || !ok || (n && (!d_commitments || !d_cell_indices || !d_cells || !d_proofs)) || n > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
-    if (!ctx->cells) return KZGB200_INVALID_SETUP;
-    if (n == 0) { *ok = 1; return KZGB200_OK; }
-    std::lock_guard<std::mutex> g(ctx->lock);
-    DeviceGuard dev(ctx->device);
-    int rc = cell_capacity(ctx, n, false, true);
-    if (rc) return rc;
-    CellCtx* c = ctx->cells;
-    // the exact transcript is a host chain over every input byte: the inputs come back to pinned memory once
-    CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_parse, 0));
-    CK(cudaMemcpyAsync(c->h_idx, d_cell_indices, n * 8, cudaMemcpyDeviceToHost, ctx->s_d2h));
-    CK(cudaMemcpyAsync(c->h_c, d_commitments, n * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
-    CK(cudaMemcpyAsync(c->h_p, d_proofs, n * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
-    CK(cudaMemcpyAsync(c->h_cells, d_cells, n * kBytesPerCell, cudaMemcpyDeviceToHost, ctx->s_d2h));
-    CK(cudaStreamSynchronize(ctx->s_d2h));
-    return cell_verify_locked(ctx, c->h_c, c->h_idx, c->h_cells, c->h_p, d_cells, d_proofs, n, ok, false);
-}
-
-// ---- verify_cell_kzg_proof_batch_many: k independent cell batches (groups), one verdict each ---------------------------------
+// ---- verify_cell_kzg_proof_batch[_many]: k independent cell batches (groups), one verdict each -------------------------------
 // The spec's check of a group is linear in its per-cell weights r^j.  With w = rho^g r_g^j on the cells of group g, all groups are
-// checked at once by the single-call pipeline above (one MSM, one pairing); only if that fails is every group checked on its own
-// (many_*_kernel, k_cells.cu, and one pairing check per group on the many-check engine).  Each r_g is the spec's challenge of
-// group g alone: its own transcript with its own deduplication of commitments, hashed by a small pool of host threads.
+// checked at once (one MSM, one pairing); only if that fails is every group checked on its own (many_*_kernel, k_cells.cu, and one
+// pairing check per group on the many-check engine).  Each r_g is the spec's challenge of group g alone: its own transcript with its
+// own deduplication of commitments, hashed by a small pool of host threads.  verify_cell_kzg_proof_batch is the case k = 1.
 
 // x mod q for a 32-byte big-endian x (hash_to_bls_field): x < 2^256 < 3q, at most two subtractions
 static void fr_reduce_be(uint8_t v[32]) {
@@ -1330,9 +1238,10 @@ static int cell_many_fallback(kzgb200_ctx* ctx, const uint8_t* d_cells, size_t n
     return KZGB200_OK;
 }
 
-// n = off[k] >= 1 cells in k groups.  hc / hidx / hcells / hp, d_cells / d_p, copy_inputs: as cell_verify_locked.
-static int cell_many_locked(kzgb200_ctx* ctx, const uint8_t* hc, const uint64_t* hidx, const uint8_t* hcells, const uint8_t* hp,
-                            const uint8_t* d_cells, const uint8_t* d_p, const uint64_t* off, size_t k, uint8_t* verdicts, bool copy_inputs) {
+// n = off[k] >= 1 cells in k groups.  hc / hidx / hcells / hp: host copies (the caller's, or the pinned read-back of device inputs);
+// d_cells / d_p: the cells / proofs on the device, or (copy_inputs) copied there from the host copies.
+static int cell_verify_groups(kzgb200_ctx* ctx, const uint8_t* hc, const uint64_t* hidx, const uint8_t* hcells, const uint8_t* hp,
+                              const uint8_t* d_cells, const uint8_t* d_p, const uint64_t* off, size_t k, uint8_t* verdicts, bool copy_inputs) {
     CellCtx* c = ctx->cells;
     const size_t n = off[k];
     // an index >= 128 fails its group's first assertion; the plan sees index 0 in its place (the group's weights are 0)
@@ -1401,10 +1310,11 @@ static int cell_many_locked(kzgb200_ctx* ctx, const uint8_t* hc, const uint64_t*
     many_rho(rg, off, k, rg + 32 * k);
     c->many_k = k;
     c->many_done = true;
-    // the combined check: the single-call pipeline with the weights (in d_rk) in place of r^k
+    // the combined check: the weights (in d_rk), then RLI on the aux stream beside the big MSM
     phase_begin(ctx, kPhTranscript, ctx->stream);
     CK(cudaMemcpyAsync(c->d_rg, rg, 32 * (k + 1), cudaMemcpyHostToDevice, ctx->stream));
     many_weights_kernel<<<(ni + 127) / 128, 128, 0, ctx->stream>>>(ni, c->d_goff, ki, c->d_rg, c->d_gbad, c->d_rk, ctx->d_status);
+    if (k == 1) r_from_digest_kernel<<<1, 1, 0, ctx->stream>>>(reinterpret_cast<const uint32_t*>(c->d_rg), ctx->d_r);   // for kzgb200_last_r
     phase_end(ctx, kPhTranscript, ctx->stream);
     CK(cudaEventRecord(c->ev_r, ctx->stream));
     CK(cudaStreamWaitEvent(ctx->s_aux, c->ev_r, 0));
@@ -1413,6 +1323,7 @@ static int cell_many_locked(kzgb200_ctx* ctx, const uint8_t* hc, const uint64_t*
     cell_rli_kernel<<<1, 256, 0, ctx->s_aux>>>(c->d_coeffs, c->tables, c->d_part + 1);
     CK(cudaGetLastError());
     CK(cudaEventRecord(c->ev_rli, ctx->s_aux));
+    // LL and RLC + RLP: the blob batch's MSM with z_k = h_k^64, y_k = 0
     ctx->cur_c = nullptr; ctx->cur_p = d_p; ctx->cur_n = n; ctx->subgroup_pending = false;
     if ((rc = launch_lincomb(ctx, 0, c->d_part, false, nullptr, 0, c->d_rk))) return rc;
     CK(cudaStreamWaitEvent(ctx->stream, c->ev_rli, 0));
@@ -1425,15 +1336,16 @@ static int cell_many_locked(kzgb200_ctx* ctx, const uint8_t* hc, const uint64_t*
     rc = read_result(ctx, &ok);
     if (rc != KZGB200_OK && rc != KZGB200_BAD_ARGS) return rc;
     if (rc == KZGB200_OK && ok) for (size_t g = 0; g < k; g++) verdicts[g] = gbad[g] ? kBadArgs : kTrue;
+    else if (k == 1) verdicts[0] = gbad[0] || rc ? kBadArgs : kFalse;      // rho^0 = 1: the combined check is the group's own
     else if ((rc = cell_many_fallback(ctx, d_cells, n, off, goff, gbad, k, verdicts))) return rc;
     collect_phase_times(ctx);
     ctx->phase_ms[1] = hash_ms;
     ctx->phase_ms[2] = (float)pool.size();
     return KZGB200_OK;
 }
-// argument checks shared by both forms; n_out = the number of cells
-static int many_args(kzgb200_ctx* ctx, const void* a, const void* b, const void* cc, const void* d, const uint64_t* off, size_t k,
-                     const uint8_t* verdicts, size_t* n_out) {
+// The four entry points: the argument checks, then the k groups of n = off[k] cells, from host or (device_inputs) device pointers.
+static int cell_verify(kzgb200_ctx* ctx, const uint8_t* cm, const uint64_t* idx, const uint8_t* cells, const uint8_t* p, const uint64_t* off,
+                       size_t k, uint8_t* verdicts, bool device_inputs) {
     if (!ctx || (k && (!off || !verdicts)) || k > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
     size_t n = 0;
     if (k) {
@@ -1441,55 +1353,63 @@ static int many_args(kzgb200_ctx* ctx, const void* a, const void* b, const void*
         for (size_t g = 0; g < k; g++) if (off[g + 1] < off[g] || off[g + 1] > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
         n = off[k];
     }
-    if (n && (!a || !b || !cc || !d)) return KZGB200_BAD_ARGS;
+    if (n && (!cm || !idx || !cells || !p)) return KZGB200_BAD_ARGS;
     if (!ctx->cells) return KZGB200_INVALID_SETUP;
-    *n_out = n;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    CellCtx* c = ctx->cells;
+    if (n == 0) {                                     // every group is empty (true); r_g = 0 and rho as for any call
+        c->many_rg.assign(32 * (k + 1), 0);
+        many_rho(c->many_rg.data(), off, k, c->many_rg.data() + 32 * k);
+        c->many_k = k;
+        c->many_done = true;
+        if (k) memset(verdicts, kTrue, k);
+        return KZGB200_OK;
+    }
+    DeviceGuard dev(ctx->device);
+    int rc = cell_capacity(ctx, n, !device_inputs, device_inputs);
+    if (rc) return rc;
+    if (!device_inputs) return cell_verify_groups(ctx, cm, idx, cells, p, nullptr, nullptr, off, k, verdicts, true);
+    // the exact transcripts are host chains over every input byte: the inputs come back to pinned memory once
+    CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_parse, 0));
+    CK(cudaMemcpyAsync(c->h_idx, idx, n * 8, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaMemcpyAsync(c->h_c, cm, n * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaMemcpyAsync(c->h_p, p, n * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaMemcpyAsync(c->h_cells, cells, n * kBytesPerCell, cudaMemcpyDeviceToHost, ctx->s_d2h));
+    CK(cudaStreamSynchronize(ctx->s_d2h));
+    return cell_verify_groups(ctx, c->h_c, c->h_idx, c->h_cells, c->h_p, cells, p, off, k, verdicts, false);
+}
+// one group: its verdict 2 (an assertion of the spec fails) is the call's BAD_ARGS
+static int cell_verify_one(kzgb200_ctx* ctx, const uint8_t* cm, const uint64_t* idx, const uint8_t* cells, const uint8_t* p, size_t n, int* ok,
+                           bool device_inputs) {
+    if (!ok) return KZGB200_BAD_ARGS;
+    const uint64_t off[2] = {0, n};
+    uint8_t v = kFalse;
+    int rc = cell_verify(ctx, cm, idx, cells, p, off, 1, &v, device_inputs);
+    if (rc) return rc;
+    if (v == kBadArgs) return KZGB200_BAD_ARGS;
+    *ok = v == kTrue;
     return KZGB200_OK;
 }
-// a call without cells: every group is empty (true); r_g = 0 and rho as for any call
-static void many_empty(kzgb200_ctx* ctx, const uint64_t* off, size_t k, uint8_t* verdicts) {
-    CellCtx* c = ctx->cells;
-    c->many_rg.assign(32 * (k + 1), 0);
-    many_rho(c->many_rg.data(), off, k, c->many_rg.data() + 32 * k);
-    c->many_k = k;
-    c->many_done = true;
-    if (k) memset(verdicts, kTrue, k);
-}
 
+extern "C" int kzgb200_verify_cell_kzg_proof_batch(kzgb200_ctx* ctx, const uint8_t* commitments, const uint64_t* cell_indices, const uint8_t* cells,
+                                                   const uint8_t* proofs, size_t n, int* ok) {
+    return cell_verify_one(ctx, commitments, cell_indices, cells, proofs, n, ok, false);
+}
+extern "C" int kzgb200_verify_cell_kzg_proof_batch_device(kzgb200_ctx* ctx, const uint8_t* d_commitments, const uint64_t* d_cell_indices,
+                                                          const uint8_t* d_cells, const uint8_t* d_proofs, size_t n, int* ok) {
+    return cell_verify_one(ctx, d_commitments, d_cell_indices, d_cells, d_proofs, n, ok, true);
+}
 extern "C" int kzgb200_verify_cell_kzg_proof_batch_many(kzgb200_ctx* ctx, const uint8_t* commitments, const uint64_t* cell_indices, const uint8_t* cells,
                                                         const uint8_t* proofs, const uint64_t* group_offsets, size_t n_groups, uint8_t* verdicts) {
-    size_t n = 0;
-    int rc = many_args(ctx, commitments, cell_indices, cells, proofs, group_offsets, n_groups, verdicts, &n);
-    if (rc) return rc;
-    std::lock_guard<std::mutex> g(ctx->lock);
-    if (n == 0) { many_empty(ctx, group_offsets, n_groups, verdicts); return KZGB200_OK; }
-    DeviceGuard dev(ctx->device);
-    if ((rc = cell_capacity(ctx, n, true, false))) return rc;
-    return cell_many_locked(ctx, commitments, cell_indices, cells, proofs, nullptr, nullptr, group_offsets, n_groups, verdicts, true);
+    return cell_verify(ctx, commitments, cell_indices, cells, proofs, group_offsets, n_groups, verdicts, false);
 }
-
 extern "C" int kzgb200_verify_cell_kzg_proof_batch_many_device(kzgb200_ctx* ctx, const uint8_t* d_commitments, const uint64_t* d_cell_indices,
                                                                const uint8_t* d_cells, const uint8_t* d_proofs, const uint64_t* group_offsets,
                                                                size_t n_groups, uint8_t* verdicts) {
-    size_t n = 0;
-    int rc = many_args(ctx, d_commitments, d_cell_indices, d_cells, d_proofs, group_offsets, n_groups, verdicts, &n);
-    if (rc) return rc;
-    std::lock_guard<std::mutex> g(ctx->lock);
-    if (n == 0) { many_empty(ctx, group_offsets, n_groups, verdicts); return KZGB200_OK; }
-    DeviceGuard dev(ctx->device);
-    if ((rc = cell_capacity(ctx, n, false, true))) return rc;
-    CellCtx* c = ctx->cells;
-    // the exact transcripts are host chains over every input byte: the inputs come back to pinned memory once
-    CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_parse, 0));
-    CK(cudaMemcpyAsync(c->h_idx, d_cell_indices, n * 8, cudaMemcpyDeviceToHost, ctx->s_d2h));
-    CK(cudaMemcpyAsync(c->h_c, d_commitments, n * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
-    CK(cudaMemcpyAsync(c->h_p, d_proofs, n * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
-    CK(cudaMemcpyAsync(c->h_cells, d_cells, n * kBytesPerCell, cudaMemcpyDeviceToHost, ctx->s_d2h));
-    CK(cudaStreamSynchronize(ctx->s_d2h));
-    return cell_many_locked(ctx, c->h_c, c->h_idx, c->h_cells, c->h_p, d_cells, d_proofs, group_offsets, n_groups, verdicts, false);
+    return cell_verify(ctx, d_commitments, d_cell_indices, d_cells, d_proofs, group_offsets, n_groups, verdicts, true);
 }
 
-// test hook: r_g of every group of the last _many call (zeros for empty groups) and rho, canonical big-endian
+// test hook: r_g of every group of the last cell verification call (zeros for empty groups) and rho, canonical big-endian
 extern "C" int kzgb200_last_cell_many_r(kzgb200_ctx* ctx, uint8_t* r_out, size_t n_groups, uint8_t* rho_out32) {
     if (!ctx || !rho_out32 || (n_groups && !r_out)) return KZGB200_BAD_ARGS;
     if (!ctx->cells) return KZGB200_INVALID_SETUP;

@@ -255,6 +255,23 @@ def test_shapes(K, settings, lib, ctx, block21):
     assert lib.kzgb200_verify_cell_kzg_proof_batch_many(ctx, None, None, None, None, C.cast(off, C.c_void_p), 1, out) == 1
 
 
+def test_one_false_group_skips_fallback(K, settings, lib, ctx, block21):
+    """with one group the combined check is that group's own (rho^0 = 1): a false group gets 0 without the per-group pass"""
+    g = block21.sidecar(61)
+    g[3][4] = g1_plus_gen(g[3][4])
+    ms = (C.c_float * 8)()
+    assert lib.kzgb200_set_profiling(ctx, 1) == 0
+    try:
+        assert many(lib, ctx, [g])[0] == [0]
+        assert lib.kzgb200_get_phase_ms(ctx, ms) == 0
+        assert ms[6] > 0 and ms[7] == 0, list(ms)
+        assert single(lib, ctx, g)[0] == 0
+        assert lib.kzgb200_get_phase_ms(ctx, ms) == 0
+        assert ms[6] > 0 and ms[7] == 0, list(ms)
+    finally:
+        lib.kzgb200_set_profiling(ctx, 0)
+
+
 def test_large_group_beside_small_ones(K, settings, lib, ctx):
     blk = Block(K, settings, 128, 11)
     whole = group([blk.entry(b, i) for b in range(128) for i in range(128)])

@@ -96,7 +96,8 @@ def main():
         out = (C.c_float * 8)()
         lib.kzgb200_get_phase_ms(ctx, out)
         lib.kzgb200_set_profiling(ctx, 0)
-        names = ["parse", "challenge", "eval", "transcript_upload", "lincomb", "reduce", "final", "deferred_subgroup"]
+        # the slot layout of a cell verification call (kzgb200.h): slots 1 and 2 are the host hashing's wall ms and thread count
+        names = ["parse", "host_hash_wall", "hasher_threads", "weights", "lincomb", "reduce", "final", "fallback"]
         yield {k: round(v, 4) for k, v in zip(names, out) if v}
 
     def record(name, desc, n, call, host_bytes, extra=None):
