@@ -5,7 +5,7 @@
 //   kzg_rs::KzgSettings::load_trusted_setup_file                                                src/trusted_setup.rs:94-98
 //   kzg_rs::Blob / Bytes32 / Bytes48 (from_slice length check, as_slice)                        src/dtypes.rs:7-46
 //   kzg_rs::KzgError                                                                            src/enums.rs:6-18
-// plus EIP-7594 cells: kzg_rs::Cell, KzgProof::verify_cell_kzg_proof_batch[_many], kzg_rs::compute_cells, kzg_rs::compute_cells_and_kzg_proofs,
+// plus the EIP-4844 publisher calls kzg_rs::blob_to_kzg_commitment / compute_kzg_proof / compute_blob_kzg_proof, and EIP-7594 cells: kzg_rs::Cell, KzgProof::verify_cell_kzg_proof_batch[_many], kzg_rs::compute_cells, kzg_rs::compute_cells_and_kzg_proofs,
 // kzg_rs::recover_cells_and_kzg_proofs (c-kzg-4844 / rust-kzg names).
 // Result<bool, KzgError> is kzg_rs::Result<bool>: either a value or an error.
 #pragma once
@@ -71,6 +71,7 @@ class KzgSettings {
     std::shared_ptr<kzgb200_ctx> ctx_;
 public:
     std::vector<uint8_t> g2_points;   // compressed, 96 bytes each; the verification path reads [0] and [1]
+    std::vector<uint8_t> g1_lagrange; // compressed, 48 bytes each, file order; read by load_commit_setup
     // setup file: "KZGS" | u32 n1 | u32 n2 | n1*48 G1 Lagrange | n2*96 G2 monomial (kzg_rs_b200/data/mainnet_setup.bin)
     static Result<KzgSettings> load_trusted_setup_file(const std::string& path, int device = 0) {
         std::ifstream f(path, std::ios::binary);
@@ -81,6 +82,7 @@ public:
         if (n2 < 2 || raw.size() != 12 + size_t(n1) * 48 + size_t(n2) * 96) return KzgError{KzgError::InvalidTrustedSetup, "Invalid trusted setup"};
         KzgSettings s;
         s.g2_points.assign(raw.begin() + 12 + size_t(n1) * 48, raw.end());
+        s.g1_lagrange.assign(raw.begin() + 12, raw.begin() + 12 + size_t(n1) * 48);
         kzgb200_ctx* c = nullptr;
         int rc = kzgb200_create(&c, device, s.g2_points.data(), 192);
         if (rc) return KzgError{rc == KZGB200_INVALID_SETUP ? KzgError::InvalidTrustedSetup : KzgError::InternalError, "kzgb200_create failed"};
@@ -94,6 +96,13 @@ public:
         if (g2_points.size() < 65 * 96) return KzgError{KzgError::InvalidTrustedSetup, "the setup has no G2 point 64"};
         int rc = kzgb200_load_cell_setup(ctx(), g1_monomial48, n_points, g2_points.data() + 64 * 96);
         if (rc) return KzgError{rc == KZGB200_INVALID_SETUP ? KzgError::InvalidTrustedSetup : KzgError::InternalError, "kzgb200_load_cell_setup failed"};
+        return true;
+    }
+    // commitments and proofs (EIP-4844 publisher calls): the window table of the 4096 Lagrange points (4.8 GB of device memory);
+    // once, before the calls
+    Result<bool> load_commit_setup() const {
+        int rc = kzgb200_load_g1_lagrange(ctx(), g1_lagrange.data(), g1_lagrange.size() / 48);
+        if (rc) return KzgError{rc == KZGB200_INVALID_SETUP ? KzgError::InvalidTrustedSetup : KzgError::InternalError, "kzgb200_load_g1_lagrange failed"};
         return true;
     }
 };
@@ -166,6 +175,28 @@ struct KzgProof {
         return verdicts;
     }
 };
+
+// EIP-4844 publisher calls (need load_commit_setup).  BadArgs for a non-canonical blob element or z, and for a commitment that is not
+// a valid compressed point of the G1 subgroup.
+inline Result<Bytes48> blob_to_kzg_commitment(const Blob& blob, const KzgSettings& kzg_settings) {
+    Bytes48 c;
+    int rc = kzgb200_blob_to_kzg_commitment(kzg_settings.ctx(), blob.as_slice(), c.bytes.data());
+    if (rc) return detail::to_result(rc, 0).unwrap_err();
+    return c;
+}
+// (proof, y) with y = p(z); z may be a point of the evaluation domain
+inline Result<std::pair<Bytes48, Bytes32>> compute_kzg_proof(const Blob& blob, const Bytes32& z_bytes, const KzgSettings& kzg_settings) {
+    std::pair<Bytes48, Bytes32> out;
+    int rc = kzgb200_compute_kzg_proof(kzg_settings.ctx(), blob.as_slice(), z_bytes.as_slice(), out.first.bytes.data(), out.second.bytes.data());
+    if (rc) return detail::to_result(rc, 0).unwrap_err();
+    return out;
+}
+inline Result<Bytes48> compute_blob_kzg_proof(const Blob& blob, const Bytes48& commitment_bytes, const KzgSettings& kzg_settings) {
+    Bytes48 p;
+    int rc = kzgb200_compute_blob_kzg_proof(kzg_settings.ctx(), blob.as_slice(), commitment_bytes.as_slice(), p.bytes.data());
+    if (rc) return detail::to_result(rc, 0).unwrap_err();
+    return p;
+}
 
 // EIP-7594 compute_cells: the 128 cells of the blob's extension
 inline Result<std::vector<Cell>> compute_cells(const Blob& blob, const KzgSettings& kzg_settings) {

@@ -170,12 +170,29 @@ int kzgb200_last_partial(kzgb200_ctx* ctx, uint8_t* out352);
  * [tau^j]G1, j < degree, are given compressed in tau_powers48 (host, degree x 48 bytes). */
 int kzgb200_harness_generate(kzgb200_ctx* ctx, uint64_t seed, size_t n, int degree, const uint8_t* tau_powers48,
                              uint8_t* d_blobs, uint8_t* d_commitments, uint8_t* d_proofs);
-/* ---- commit / prove (SURVEY.md 8f-1; EIP-4844 blob_to_kzg_commitment / compute_blob_kzg_proof) -------------------
- * kzg-rs has no commit/prove path (its g1_points are loaded but never read); these are the companion operations used
- * to make test data for arbitrary blobs, pinned by the commitment / proof bytes of the reference's valid vectors.
- * kzgb200_load_g1_lagrange: the setup's 4096 Lagrange G1 points, compressed, FILE order (host, 4096 x 48 bytes);
- * builds a 4.8 GB fixed-base window table on the device (once per context).  The batch calls take DEVICE pointers. */
+/* ---- commit / prove: EIP-4844 blob_to_kzg_commitment, compute_kzg_proof, compute_blob_kzg_proof (c-kzg-4844 semantics) ------
+ * The publisher side of EIP-4844 (kzg-rs itself has none).  All outputs are compressed G1 points (48 bytes; the identity is 0xc0
+ * then 47 zero bytes) and 32-byte big-endian scalars.
+ * kzgb200_load_g1_lagrange: the setup's 4096 Lagrange G1 points, compressed, FILE order (host, 4096 x 48 bytes); builds a 4.8 GB
+ *   fixed-base window table on the device (once per context; later calls return OK).  Every call below returns
+ *   KZGB200_INVALID_SETUP before it.
+ * kzgb200_blob_to_kzg_commitment: one host blob -> its commitment.  A non-canonical blob element -> BAD_ARGS.
+ * kzgb200_compute_kzg_proof: one host blob and a host z -> the proof of p(z) = y and y.  z may be any canonical scalar, a point of
+ *   the evaluation domain included.  A non-canonical blob element or z -> BAD_ARGS.
+ * kzgb200_compute_blob_kzg_proof: one host blob and its commitment -> the proof at the Fiat-Shamir challenge of (blob, commitment).
+ *   BAD_ARGS for a non-canonical blob element and for a commitment that is not a valid compressed point of the G1 subgroup
+ *   (bad encoding, off the curve, outside the subgroup), as the spec's bytes_to_kzg_commitment.
+ * kzgb200_compute_kzg_proof_batch_device: n device blobs and n device z (n x 32) -> n proofs (n x 48) and n y (n x 32), device
+ *   pointers; n == 0 -> OK; any bad blob element or z -> BAD_ARGS for the whole call (outputs undefined).
+ * kzgb200_blob_to_kzg_commitment_batch / kzgb200_compute_blob_kzg_proof_batch: the device-pointer batch forms (n >= 1); a bad blob
+ *   element -> BAD_ARGS for the whole call.  The proof batch takes its commitments as given: it does not decompress or check them
+ *   (the single-blob kzgb200_compute_blob_kzg_proof does). */
 int kzgb200_load_g1_lagrange(kzgb200_ctx* ctx, const uint8_t* g1_lagrange, size_t n_points);
+int kzgb200_blob_to_kzg_commitment(kzgb200_ctx* ctx, const uint8_t* blob, uint8_t* commitment_out48);
+int kzgb200_compute_kzg_proof(kzgb200_ctx* ctx, const uint8_t* blob, const uint8_t* z32, uint8_t* proof_out48, uint8_t* y_out32);
+int kzgb200_compute_blob_kzg_proof(kzgb200_ctx* ctx, const uint8_t* blob, const uint8_t* commitment48, uint8_t* proof_out48);
+int kzgb200_compute_kzg_proof_batch_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t* d_zs, size_t n,
+                                           uint8_t* d_proofs_out, uint8_t* d_ys_out);
 int kzgb200_blob_to_kzg_commitment_batch(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8_t* d_commitments_out);
 int kzgb200_compute_blob_kzg_proof_batch(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t* d_commitments, size_t n,
                                          uint8_t* d_proofs_out);

@@ -101,6 +101,10 @@ class Library:
         d.kzgb200_load_g1_lagrange.argtypes = [p, C.c_char_p, sz]
         d.kzgb200_blob_to_kzg_commitment_batch.argtypes = [p, p, sz, p]
         d.kzgb200_compute_blob_kzg_proof_batch.argtypes = [p, p, p, sz, p]
+        d.kzgb200_blob_to_kzg_commitment.argtypes = [p, C.c_char_p, p]
+        d.kzgb200_compute_kzg_proof.argtypes = [p, C.c_char_p, C.c_char_p, p, p]
+        d.kzgb200_compute_blob_kzg_proof.argtypes = [p, C.c_char_p, C.c_char_p, p]
+        d.kzgb200_compute_kzg_proof_batch_device.argtypes = [p, p, p, sz, p, p]
         u64 = C.c_uint64
         d.kzgb200_pipeline_create.argtypes = [C.POINTER(p), C.c_int, C.c_char_p, sz, C.c_int]
         d.kzgb200_pipeline_destroy.argtypes = [p]
@@ -202,6 +206,7 @@ class KzgSettings:
         self._ctx = {}
         self._cells = set()
         self._proofs = set()
+        self._commit = set()
         self._lock = threading.Lock()
 
     @classmethod
@@ -287,6 +292,20 @@ class KzgSettings:
                 self._proofs.add(device)
         return ctx
 
+    def commit_context(self, device=0):
+        """The device context with the Lagrange window table loaded (blob_to_kzg_commitment, compute_kzg_proof,
+        compute_blob_kzg_proof): 4.8 GB of device memory, built once from g1_lagrange_bytes."""
+        ctx = self.context(device)
+        with self._lock:
+            if device not in self._commit:
+                if len(self.g1_lagrange_bytes) != 4096 * 48:
+                    raise KzgError("InvalidTrustedSetup", "commitments and proofs need the setup's 4096 Lagrange G1 points")
+                rc = Library.get().dll.kzgb200_load_g1_lagrange(ctx, self.g1_lagrange_bytes, 4096)
+                if rc:
+                    _raise(rc, ctx)
+                self._commit.add(device)
+        return ctx
+
     def close(self):
         with self._lock:
             for h in self._ctx.values():
@@ -294,6 +313,7 @@ class KzgSettings:
             self._ctx = {}
             self._cells = set()
             self._proofs = set()
+            self._commit = set()
 
 
 def mainnet_g1_monomial():
@@ -491,6 +511,39 @@ def recover_cells_and_kzg_proofs(cell_indices, cells, kzg_settings, device=0):
     if rc:
         _raise(rc, ctx, "Invalid cell indices / cells" if rc == 1 else None)
     return _cells_and_proofs(out_cells.raw, out_proofs.raw)
+
+
+def blob_to_kzg_commitment(blob, kzg_settings, device=0):
+    """EIP-4844 blob_to_kzg_commitment: the blob's commitment, 48 bytes compressed; BadArgs on a non-canonical element."""
+    b = _b(blob, BYTES_PER_BLOB, "blob")
+    ctx, out = kzg_settings.commit_context(device), C.create_string_buffer(48)
+    rc = Library.get().dll.kzgb200_blob_to_kzg_commitment(ctx, b, out)
+    if rc:
+        _raise(rc, ctx, "Failed to parse blob" if rc == 1 else None)
+    return out.raw
+
+
+def compute_kzg_proof(blob, z_bytes, kzg_settings, device=0):
+    """EIP-4844 compute_kzg_proof: (proof, y) for the blob's polynomial at z, y = p(z) (48 and 32 bytes); z may be a point of
+    the evaluation domain.  BadArgs on a non-canonical blob element or z."""
+    b, z = _b(blob, BYTES_PER_BLOB, "blob"), _b(z_bytes, 32, "z")
+    ctx = kzg_settings.commit_context(device)
+    proof, y = C.create_string_buffer(48), C.create_string_buffer(32)
+    rc = Library.get().dll.kzgb200_compute_kzg_proof(ctx, b, z, proof, y)
+    if rc:
+        _raise(rc, ctx, "Failed to parse blob / z" if rc == 1 else None)
+    return proof.raw, y.raw
+
+
+def compute_blob_kzg_proof(blob, commitment_bytes, kzg_settings, device=0):
+    """EIP-4844 compute_blob_kzg_proof: the proof at the Fiat-Shamir challenge of (blob, commitment), 48 bytes.  BadArgs on a
+    non-canonical blob element or a commitment that is not a valid compressed point of the G1 subgroup."""
+    b, c = _b(blob, BYTES_PER_BLOB, "blob"), _b(commitment_bytes, 48, "commitment")
+    ctx, out = kzg_settings.commit_context(device), C.create_string_buffer(48)
+    rc = Library.get().dll.kzgb200_compute_blob_kzg_proof(ctx, b, c, out)
+    if rc:
+        _raise(rc, ctx, "Failed to parse blob / commitment" if rc == 1 else None)
+    return out.raw
 
 
 def compute_challenge(blob, commitment_bytes, kzg_settings, device=0):

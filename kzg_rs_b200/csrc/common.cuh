@@ -58,6 +58,9 @@ constexpr int kManyCtasPerSm = 1;                     // (two CTAs of 14 checks 
 constexpr int kManyWarps = 4;         // many_pairing_warp_kernel (identity inputs): one check per warp
 constexpr int kHarnessMaxDegree = 16;
 constexpr int kLagWindows = 32, kLagEntries = 255;
+constexpr int kLagTerms = kFieldElementsPerBlob * kLagWindows;   // (point, window) terms of a blob's commitment MSM
+constexpr int kLagMsmThreads = 256, kLagMaxSlices = kLagTerms / kLagMsmThreads / 2;   // lag_msm_slice_kernel: >= 2 terms per thread
+constexpr int kLagFinishThreads = 64;                             // lag_msm_finish_kernel
 // EIP-7594 cells (k_cells.cu)
 constexpr int kCellsPerExtBlob = 128, kFieldElementsPerCell = 64, kBytesPerCell = 2048;
 constexpr int kCellNttThreads = 512;                              // compute_cells_kernel: one CTA per blob, 4096 values in shared memory
@@ -205,7 +208,9 @@ __global__ void lag_table_kernel(const G1Affine* __restrict__ L, G1* __restrict_
 __global__ void blob_scalars_kernel(const uint8_t* __restrict__ blobs, int n, Fr* __restrict__ scalars, uint32_t* __restrict__ status);
 __global__ void quotient_kernel(const uint8_t* __restrict__ blobs, int n, const Fr* __restrict__ z_mont, const ZY* __restrict__ zy,
                                 const DeviceTables* __restrict__ T, Fr* __restrict__ scalars);
-__global__ void lag_msm_kernel(const Fr* __restrict__ scalars, int n, const G1* __restrict__ table, uint8_t* __restrict__ out48);
+__global__ void lag_msm_slice_kernel(const Fr* __restrict__ scalars, int n, int slices, const G1* __restrict__ table, G1* __restrict__ partials,
+                                     uint8_t* __restrict__ out48);
+__global__ void lag_msm_finish_kernel(const G1* __restrict__ partials, int n, int slices, uint8_t* __restrict__ out48);
 __global__ void cell_setup_kernel(CellTables* T, const uint8_t* __restrict__ g2_tau64);
 __global__ void cell_setup_points_kernel(CellTables* T, const uint8_t* __restrict__ g1_monomial48);
 __global__ void cell_setup_lines29_kernel(CellTables* T);

@@ -110,8 +110,9 @@ __global__ void __launch_bounds__(128) blob_scalars_kernel(const uint8_t* __rest
     scalars[i] = f;
 }
 // quotient q_i = (f_i - y) / (w_i - z) in evaluation form (one CTA of 128 threads per blob, Montgomery batch inversion
-// across the CTA); if z = w_m the m-th entry is sum_{i != m} (f_i - y) w_i / (z (z - w_i))
-__global__ void __launch_bounds__(kEvalThreads) quotient_kernel(const uint8_t* __restrict__ blobs, int n, const Fr* __restrict__ z_mont,
+// across the CTA); if z = w_m the m-th entry is sum_{i != m} (f_i - y) w_i / (z (z - w_i)) = -(1/z) sum_{i != m} q_i w_i, summed
+// by every thread over its own 32 entries, then tree-summed in shared memory
+__global__ void __launch_bounds__(kEvalThreads, 5) quotient_kernel(const uint8_t* __restrict__ blobs, int n, const Fr* __restrict__ z_mont,
                                                                 const ZY* __restrict__ zy, const DeviceTables* __restrict__ T,
                                                                 Fr* __restrict__ scalars) {
     __shared__ Fr s_tot[kEvalThreads], s_pre[kEvalThreads], s_inv;
@@ -152,39 +153,61 @@ __global__ void __launch_bounds__(kEvalThreads) quotient_kernel(const uint8_t* _
         Fr f = Fr::from_raw(load_fe_be(base + 2 * j));
         out[j] = ((f - y_m).mul_inl(inv_d)).to_raw();
     }
+    const int special = s_special;      // z in the domain (probability 2^-243 for hashed z; a real input of compute_kzg_proof)
+    if (special < 0) return;            // uniform across the CTA
+    Fr qw = Fr::zero();                 // sum of q_i w_i over this thread's entries i != special (its own stores, read back)
+    for (int j = 0; j < kLeavesPerThread; j++)
+        if (t * kLeavesPerThread + j != special) qw = qw + Fr::from_raw(out[j]).mul_inl(den[j] + z);   // den[j] + z = w_i
+    __syncthreads();                    // every thread has read s_tot / s_pre
+    s_tot[t] = qw;
     __syncthreads();
-    if (s_special >= 0 && t == 0) {   // z in the domain (probability 2^-243 for hashed z): direct formula
-        int m = s_special;
-        Fr zi = fr_inv(z), sum = Fr::zero();
-        Fr* row = scalars + (size_t)blob * kFieldElementsPerBlob;
-        for (int i = 0; i < kFieldElementsPerBlob; i++) {
-            if (i == m) continue;
-            Fr w = T->twiddle[i >> 1];
-            if (i & 1) w = w.neg();
-            sum = sum - Fr::from_raw(row[i]) * w * zi;    // (f_i-y)/(w_i-z) = -(f_i-y)/(z-w_i)
-        }
-        row[m] = sum.to_raw();
+    for (int span = kEvalThreads / 2; span >= 1; span >>= 1) {
+        if (t < span) s_tot[t] = s_tot[t] + s_tot[t + span];
+        __syncthreads();
     }
+    if (t == 0) scalars[(size_t)blob * kFieldElementsPerBlob + special] = (s_tot[0] * fr_inv(z)).neg().to_raw();
 }
-// one CTA (256 threads) per blob: sum_j [s_j] L_j through the window table, tree-summed in shared memory, compressed
-__global__ void __launch_bounds__(256) lag_msm_kernel(const Fr* __restrict__ scalars, int n, const G1* __restrict__ table, uint8_t* __restrict__ out48) {
-    __shared__ G1 sm[256];
-    int blob = blockIdx.x, t = threadIdx.x;
+// Sliced fixed-base MSM sum_j [s_j] L_j through the window table.  Term i = 32 j + w of a blob (point j, window w) is row i of the
+// table, so a blob is 131072 terms in table order; CTA (s, blob) of a (slices x blobs) grid sums the s-th of `slices` equal ranges (thread t takes
+// every kLagMsmThreads-th term from t), tree-sums its threads' partials in shared memory and stores one Jacobian partial, which
+// lag_msm_finish_kernel sums.  Many slices spread a small batch over the whole GPU (kzgb200.cu, lag_slices); with one slice per blob
+// the CTA compresses its sum itself (out48), so that each blob's affine conversion overlaps the MSM of later CTAs.
+__global__ void __launch_bounds__(kLagMsmThreads) lag_msm_slice_kernel(const Fr* __restrict__ scalars, int n, int slices, const G1* __restrict__ table,
+                                                                       G1* __restrict__ partials, uint8_t* __restrict__ out48) {
+    __shared__ G1 sm[kLagMsmThreads];
+    int s = blockIdx.x, blob = blockIdx.y, t = threadIdx.x;
     if (blob >= n) return;
-    const Fr* row = scalars + (size_t)blob * kFieldElementsPerBlob;
+    const uint32_t* row = reinterpret_cast<const uint32_t*>(scalars + (size_t)blob * kFieldElementsPerBlob);
+    const int lo = (int)((int64_t)s * kLagTerms / slices), hi = (int)((int64_t)(s + 1) * kLagTerms / slices);
     G1 acc = G1::identity();
-    for (int j = t; j < kFieldElementsPerBlob; j += 256) {
-        Fr s = row[j];
-        const G1* tj = table + (size_t)j * kLagWindows * kLagEntries;
-        for (int w = 0; w < kLagWindows; w++) {
-            uint32_t d = (s.l[w >> 2] >> (8 * (w & 3))) & 0xffu;
-            if (d) acc = acc.add(tj[(size_t)w * kLagEntries + d - 1]);
-        }
+    for (int i = lo + t; i < hi; i += kLagMsmThreads) {
+        uint32_t d = (__ldg(row + 8 * (i >> 5) + ((i & 31) >> 2)) >> (8 * (i & 3))) & 0xffu;   // byte w of s_j
+        if (d) acc = acc.add(table[(size_t)i * kLagEntries + d - 1]);
     }
     sm[t] = acc;
     __syncthreads();
-    for (int span = 128; span >= 1; span >>= 1) {
+    for (int span = kLagMsmThreads / 2; span >= 1; span >>= 1) {
         if (t < span) sm[t] = sm[t].add(sm[t + span]);
+        __syncthreads();
+    }
+    if (t != 0) return;
+    if (slices > 1) { partials[(size_t)blob * slices + s] = sm[0]; return; }
+    uint8_t enc[48];
+    g1_to_compressed(enc, g1_to_affine(sm[0]));
+    for (int k = 0; k < 48; k++) out48[(size_t)blob * 48 + k] = enc[k];
+}
+// slices > 1: one CTA per blob, the sum of its slice partials (thread t takes every kLagFinishThreads-th, then a tree in shared memory), compressed.
+// Affine compression is canonical: the bytes do not depend on how the sum was split.
+__global__ void __launch_bounds__(kLagFinishThreads) lag_msm_finish_kernel(const G1* __restrict__ partials, int n, int slices, uint8_t* __restrict__ out48) {
+    __shared__ G1 sm[kLagFinishThreads];
+    int blob = blockIdx.x, t = threadIdx.x;
+    if (blob >= n) return;
+    G1 acc = G1::identity();
+    for (int s = t; s < slices; s += kLagFinishThreads) acc = acc.add(partials[(size_t)blob * slices + s]);
+    sm[t] = acc;
+    __syncthreads();
+    for (int span = kLagFinishThreads / 2; span >= 1; span >>= 1) {
+        if (t < span && t + span < slices) sm[t] = sm[t].add(sm[t + span]);
         __syncthreads();
     }
     if (t == 0) {

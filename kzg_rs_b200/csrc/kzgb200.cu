@@ -529,7 +529,7 @@ extern "C" void kzgb200_destroy(kzgb200_ctx* ctx) {
     for (auto e : ctx->ev_stage) if (e) cudaEventDestroy(e);
     void* ptrs[] = {ctx->tables, ctx->d_blobs, ctx->d_c, ctx->d_p, ctx->d_z_mont, ctx->d_zy, ctx->d_C, ctx->d_P, ctx->d_status,
                     ctx->d_ry, ctx->d_r, ctx->d_partial, ctx->d_result, ctx->d_zout, ctx->d_yout, ctx->d_many, ctx->d_wk,
-                    ctx->d_digits, ctx->d_order, ctx->d_start, ctx->d_buckets, ctx->d_halfsum, ctx->d_part, ctx->d_windows, ctx->d_lag_table, ctx->d_scalars, ctx->d_zpow,
+                    ctx->d_digits, ctx->d_order, ctx->d_start, ctx->d_buckets, ctx->d_halfsum, ctx->d_part, ctx->d_windows, ctx->d_lag_table, ctx->d_scalars, ctx->d_lag_part, ctx->d_zpow,
                     ctx->d_chain_state, ctx->d_scratch, ctx->d_digest};
     for (void* p : ptrs) if (p) cudaFree(p);
     void* hptrs[] = {ctx->h_flags, ctx->h_result, ctx->h_digest, ctx->h_partial, ctx->h_zy, ctx->h_c, ctx->h_p, ctx->h_stage[0], ctx->h_stage[1], ctx->h_stage[2], ctx->h_stage[3]};
@@ -897,26 +897,52 @@ extern "C" int kzgb200_load_g1_lagrange(kzgb200_ctx* ctx, const uint8_t* g1_lagr
     if (bad) { cudaFree(ctx->d_lag_table); ctx->d_lag_table = nullptr; return KZGB200_INVALID_SETUP; }
     return KZGB200_OK;
 }
-// shared driver: want_proof == 0 -> commitments of the blobs; 1 -> proofs at the Fiat-Shamir challenge of (blob, commitment)
-static int commit_or_prove(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t* d_commitments, size_t n, uint8_t* d_out, int want_proof) {
+// Slices per blob of the commitment MSM for a chunk of cnt blobs: as many as keep the grid within one wave of one CTA per SM
+// (lag_msm_slice_kernel uses 180 registers: two 256-thread CTAs do not fit one SM).  One blob then spreads over every SM; from
+// num_sms / 2 + 1 blobs on it is one CTA per blob, the batch throughput form.
+static int lag_slices(const kzgb200_ctx* ctx, int cnt) {
+    int s = ctx->num_sms / cnt;
+    return s < 1 ? 1 : (s > kLagMaxSlices ? kLagMaxSlices : s);
+}
+enum ProveMode { kProveCommit, kProveBlob, kProveAtZ };
+// Shared driver of every commit / prove entry point, in chunks of 1024 blobs:
+//   kProveCommit  commitments of the blobs (d_in unused);
+//   kProveBlob    proofs at the Fiat-Shamir challenge of (blob, commitment), d_in = the commitments (n x 48); check_commitments also
+//                 decompresses them and checks the subgroup (the spec's bytes_to_kzg_commitment);
+//   kProveAtZ     proofs at caller-given points, d_in = z (n x 32 big-endian); d_y_out (nullable) receives y = p(z) (n x 32).
+// BAD_ARGS when any blob element, z or checked commitment is invalid; the outputs are then undefined.
+static int commit_or_prove(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t* d_in, size_t n, uint8_t* d_out, ProveMode mode,
+                           bool check_commitments = false, uint8_t* d_y_out = nullptr) {
     if (!ctx->d_lag_table) return KZGB200_INVALID_SETUP;
     const size_t kChunk = 1024;
     int rc = ensure_capacity(ctx, n < kChunk ? n : kChunk, false);
     if (rc) return rc;
     if (!ctx->d_scalars) CK(cudaMalloc(&ctx->d_scalars, kChunk * (size_t)kFieldElementsPerBlob * sizeof(Fr)));
+    if (!ctx->d_lag_part) CK(cudaMalloc(&ctx->d_lag_part, (kChunk > (size_t)ctx->num_sms ? kChunk : (size_t)ctx->num_sms) * sizeof(G1)));
     uint32_t any_bad = 0;
     for (size_t lo = 0; lo < n; lo += kChunk) {
         int cnt = (int)(n - lo < kChunk ? n - lo : kChunk);
         const uint8_t* blobs = d_blobs + lo * kBytesPerBlob;
         CK(cudaMemsetAsync(ctx->d_status, 0, cnt * sizeof(uint32_t), ctx->stream));
-        if (!want_proof) {
+        if (mode == kProveCommit) {
             blob_scalars_kernel<<<(unsigned)(((size_t)cnt * kFieldElementsPerBlob + 127) / 128), 128, 0, ctx->stream>>>(blobs, cnt, ctx->d_scalars, ctx->d_status);
         } else {
-            launch_challenge(ctx->sha_stages, ctx->stream, blobs, d_commitments + lo * 48, cnt, ctx->d_z_mont, ctx->d_zy, ctx->d_zpow);
+            if (mode == kProveBlob) {
+                const uint8_t* cs = d_in + lo * 48;
+                launch_challenge(ctx->sha_stages, ctx->stream, blobs, cs, cnt, ctx->d_z_mont, ctx->d_zy, ctx->d_zpow);
+                if (check_commitments)   // each commitment as both point arguments: one kernel, flags in d_status
+                    g1_decompress_kernel<<<(2 * cnt + 127) / 128, 128, 0, ctx->stream>>>(cs, cs, cnt, ctx->d_C, ctx->d_P, ctx->d_status, true);
+            } else {
+                z_setup_kernel<<<(cnt + 127) / 128, 128, 0, ctx->stream>>>(d_in + lo * 32, cnt, ctx->d_z_mont, ctx->d_zy, ctx->d_zpow, ctx->d_status);
+            }
             eval_kernel<<<cnt, kEvalThreads, 0, ctx->stream>>>(blobs, cnt, ctx->d_zpow, ctx->tables, ctx->d_zy, ctx->d_status);
             quotient_kernel<<<cnt, kEvalThreads, 0, ctx->stream>>>(blobs, cnt, ctx->d_z_mont, ctx->d_zy, ctx->tables, ctx->d_scalars);
+            if (d_y_out) export_scalars_kernel<<<(cnt + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_zy, cnt, nullptr, d_y_out + lo * 32);
         }
-        lag_msm_kernel<<<cnt, 256, 0, ctx->stream>>>(ctx->d_scalars, cnt, ctx->d_lag_table, d_out + lo * 48);
+        const int slices = lag_slices(ctx, cnt);
+        lag_msm_slice_kernel<<<dim3(slices, cnt), kLagMsmThreads, 0, ctx->stream>>>(ctx->d_scalars, cnt, slices, ctx->d_lag_table, ctx->d_lag_part,
+                                                                                     d_out + lo * 48);
+        if (slices > 1) lag_msm_finish_kernel<<<cnt, kLagFinishThreads, 0, ctx->stream>>>(ctx->d_lag_part, cnt, slices, d_out + lo * 48);
         status_or_kernel<<<1, 256, 0, ctx->stream>>>(ctx->d_status, cnt, ctx->d_result);
         CK(cudaGetLastError());
         CK(cudaMemcpyAsync(ctx->h_result, ctx->d_result, 4, cudaMemcpyDeviceToHost, ctx->stream));
@@ -929,14 +955,51 @@ extern "C" int kzgb200_blob_to_kzg_commitment_batch(kzgb200_ctx* ctx, const uint
     if (!ctx || !d_blobs || !d_commitments_out || n == 0) return KZGB200_BAD_ARGS;
     std::lock_guard<std::mutex> g(ctx->lock);
     DeviceGuard dev(ctx->device);
-    return commit_or_prove(ctx, d_blobs, nullptr, n, d_commitments_out, 0);
+    return commit_or_prove(ctx, d_blobs, nullptr, n, d_commitments_out, kProveCommit);
 }
 extern "C" int kzgb200_compute_blob_kzg_proof_batch(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t* d_commitments, size_t n,
                                                     uint8_t* d_proofs_out) {
     if (!ctx || !d_blobs || !d_commitments || !d_proofs_out || n == 0) return KZGB200_BAD_ARGS;
     std::lock_guard<std::mutex> g(ctx->lock);
     DeviceGuard dev(ctx->device);
-    return commit_or_prove(ctx, d_blobs, d_commitments, n, d_proofs_out, 1);
+    return commit_or_prove(ctx, d_blobs, d_commitments, n, d_proofs_out, kProveBlob);
+}
+extern "C" int kzgb200_compute_kzg_proof_batch_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t* d_zs, size_t n,
+                                                      uint8_t* d_proofs_out, uint8_t* d_ys_out) {
+    if (!ctx || (n && (!d_blobs || !d_zs || !d_proofs_out || !d_ys_out)) || n > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
+    if (!ctx->d_lag_table) return KZGB200_INVALID_SETUP;
+    if (n == 0) return KZGB200_OK;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    return commit_or_prove(ctx, d_blobs, d_zs, n, d_proofs_out, kProveAtZ, false, d_ys_out);
+}
+// one host blob through commit_or_prove on the context's staging buffers: the blob in d_blobs, the 48-byte commitment or the
+// 32-byte z in d_c, the point out of d_p and y out of d_yout
+static int prove_host(kzgb200_ctx* ctx, const uint8_t* blob, const uint8_t* in, size_t in_bytes, ProveMode mode, uint8_t* out48, uint8_t* y_out32) {
+    if (!ctx->d_lag_table) return KZGB200_INVALID_SETUP;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    int rc = ensure_capacity(ctx, 1, true);
+    if (rc) return rc;
+    CK(cudaMemcpyAsync(ctx->d_blobs, blob, kBytesPerBlob, cudaMemcpyHostToDevice, ctx->stream));
+    if (in) CK(cudaMemcpyAsync(ctx->d_c, in, in_bytes, cudaMemcpyHostToDevice, ctx->stream));
+    if ((rc = commit_or_prove(ctx, ctx->d_blobs, ctx->d_c, 1, ctx->d_p, mode, mode == kProveBlob, y_out32 ? ctx->d_yout : nullptr))) return rc;
+    CK(cudaMemcpyAsync(out48, ctx->d_p, 48, cudaMemcpyDeviceToHost, ctx->stream));
+    if (y_out32) CK(cudaMemcpyAsync(y_out32, ctx->d_yout, 32, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return KZGB200_OK;
+}
+extern "C" int kzgb200_blob_to_kzg_commitment(kzgb200_ctx* ctx, const uint8_t* blob, uint8_t* commitment_out48) {
+    if (!ctx || !blob || !commitment_out48) return KZGB200_BAD_ARGS;
+    return prove_host(ctx, blob, nullptr, 0, kProveCommit, commitment_out48, nullptr);
+}
+extern "C" int kzgb200_compute_kzg_proof(kzgb200_ctx* ctx, const uint8_t* blob, const uint8_t* z32, uint8_t* proof_out48, uint8_t* y_out32) {
+    if (!ctx || !blob || !z32 || !proof_out48 || !y_out32) return KZGB200_BAD_ARGS;
+    return prove_host(ctx, blob, z32, 32, kProveAtZ, proof_out48, y_out32);
+}
+extern "C" int kzgb200_compute_blob_kzg_proof(kzgb200_ctx* ctx, const uint8_t* blob, const uint8_t* commitment48, uint8_t* proof_out48) {
+    if (!ctx || !blob || !commitment48 || !proof_out48) return KZGB200_BAD_ARGS;
+    return prove_host(ctx, blob, commitment48, 48, kProveBlob, proof_out48, nullptr);
 }
 // clock64() stamps of the last single-GPU batch_final_kernel: start, prelude end, Miller loop end, easy part end, hard part end, done
 extern "C" int kzgb200_debug_final_ticks(kzgb200_ctx* ctx, long long* out14) {

@@ -110,6 +110,7 @@ struct kzgb200_ctx {
     uint8_t* d_many = nullptr;
     kzgb200::G1* d_lag_table = nullptr;      // [4096][32][255] window table of the Lagrange G1 points (commit / prove only)
     kzgb200::Fr* d_scalars = nullptr;
+    kzgb200::G1* d_lag_part = nullptr;      // slice partials of the commitment MSM (lag_msm_slice_kernel)
     uint32_t* d_wk = nullptr;       // device transcript scratch: W+K words (exact-device) / entry words + leaf digests (tree)
     size_t wk_cap = 0;
     uint32_t* h_result = nullptr;   // pinned
