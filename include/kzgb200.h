@@ -290,6 +290,10 @@ int kzgb200_set_slab_tail(kzgb200_ctx* ctx, int on);
 int kzgb200_get_phase_ms(kzgb200_ctx* ctx, float* out8);
 /* profiling aid: SM clock stamps of the sections of the last single-GPU final pairing kernel */
 int kzgb200_debug_final_ticks(kzgb200_ctx* ctx, long long* out14);
+/* f^(3(p^12-1)/r) of the last single-GPU batch check, 12 canonical Fp coefficients of 48 little-endian bytes (the verdict is true iff
+ * it is 1), and the split tail's shifted line tables ([256^w]G2, [256^w tau]G2, w = 1..15; len = 783360).  Test aids. */
+int kzgb200_debug_last_gt(kzgb200_ctx* ctx, uint8_t* out576);
+int kzgb200_debug_lines29w(kzgb200_ctx* ctx, uint8_t* out, size_t len);
 /* Self-test of the pairing engine's 16-lane instructions (csrc/vliw29.cuh): every engine program is run `rounds` times on the
  * cooperative executors and on the sequential reference executors from the same seeded register files; mismatches[i] receives
  * the number of registers of program i whose canonical values differ (all zero = pass).  n_programs receives their count. */

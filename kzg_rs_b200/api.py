@@ -98,6 +98,8 @@ class Library:
         d.kzgb200_set_transcript_mode.argtypes = [p, C.c_int]
         d.kzgb200_last_r.argtypes = [p, C.c_char_p]
         d.kzgb200_last_partial.argtypes = [p, C.c_char_p]
+        d.kzgb200_debug_last_gt.argtypes = [p, C.c_char_p]
+        d.kzgb200_debug_lines29w.argtypes = [p, C.c_char_p, sz]
         d.kzgb200_load_g1_lagrange.argtypes = [p, C.c_char_p, sz]
         d.kzgb200_blob_to_kzg_commitment_batch.argtypes = [p, p, sz, p]
         d.kzgb200_compute_blob_kzg_proof_batch.argtypes = [p, p, p, sz, p]

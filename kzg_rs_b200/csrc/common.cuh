@@ -31,6 +31,9 @@ struct DeviceTables {
     PairingTables pairing;
     // the same line triples in the representation of the cooperative pairing engine (vliw29.cuh): [0] = G2 generator, [1] = [tau]G2
     vliw29::LineCoeffs29 lines29[2][kMillerSteps];
+    // ... and of their multiples by 256^w, w = 1..15 ([0] = [256^w]G2, [1] = [256^w tau]G2): the batch verifier's split tail pairs MSM
+    // window w with them (window_miller_kernel), so the window weights need no Horner chain on the G1 side
+    vliw29::LineCoeffs29 lines29w[2][15][kMillerSteps];
     // fixed-base table of the G1 generator: gen_table[w][d-1] = [d * 16^w] G, d = 1..15, w < 64
     G1Affine gen_table[64][15];
     uint32_t setup_ok;
@@ -46,10 +49,12 @@ constexpr int kLeavesPerThread = kFieldElementsPerBlob / kEvalThreads;  // 32
 constexpr int kTreeGroup = 16;      // transcript entries (160 B each) per leaf hash: 40 compressions
 constexpr int kTreeMid = 32;        // leaf digests per middle-level hash: 17 compressions
 constexpr int kWindows = 16, kBuckets = 256, kMsmSets = 3, kDigitRows = 4 * kWindows;   // rows: (kind r|rz) x (half lo|hi) x window
+static_assert(kWindows - 1 == sizeof(DeviceTables::lines29w[0]) / sizeof(DeviceTables::lines29w[0][0]), "one shifted line table per window > 0");
 constexpr int kMinSlice = 8, kMsmRows = kMsmSets * 2 * kWindows;   // bucket accumulation: fewest entries per thread (msm_slice_len); rows = (set, GLV half, window)
 constexpr int kWinLanes = kBuckets;                                 // window sums: one thread per bucket (suffix scan + tree in shared memory)
 constexpr int kWinSmemBytes = kWinLanes * 144;                      // one Jacobian point per thread
 constexpr int kCombineThreads = 544;    // msm_combine_kernel: 384 engine threads (three Horner chains in lockstep) + 160 helpers
+constexpr int kCombHelpers = 160;       // ... of which helpers ([s]G, flags; alone: msm_sg_kernel)
 constexpr int kCombineSmemBytes = 48 * 1024;
 constexpr int kFinalThreads = 64;       // G1 prelude of the final check (sums, [s]G, affine conversion)
 constexpr int kPairThreads = 768;       // pairing engine: 24 warps = 24 products (one per warp) or 48 sums (16 lanes each) at a time
@@ -103,6 +108,16 @@ struct PairSmem {                        // pairing_check_kernel
 // hand-over from the prelude kernel to the pairing kernel (device memory, 256 bytes into the context's 512-byte scratch)
 struct FinalPts { G1Affine pts[2]; uint32_t go; };
 
+// hand-over buffer of the split tail of a batch (kzgb200_ctx::d_split; see window_miller_kernel)
+struct SplitTail {
+    G1 sg;                                  // [s]G, s = sum r_i y_i (msm_sg_kernel)
+    uint32_t err;                           // OR of the per-blob error flags (msm_sg_kernel)
+    uint32_t pad[3];
+    G1Affine pts[kWindows][2];              // per window: -W0_w, B_w (window_prelude_kernel)
+    alignas(16) f29::F29 f[kWindows][12];   // per-window Miller values (window_miller_kernel)
+    Fp gt[12];                              // f^(3(p^12-1)/r) of the last batch check, canonical integers (kzgb200_debug_last_gt)
+};
+
 constexpr int kManyStride = vliw::kTotalRegsThr * 12 + 1;     // words between the register files of consecutive groups (odd: bank skew)
 constexpr int kManySmemBytes = kManyGroups * kManyStride * 4 + (int)sizeof(vliw::SharedTables) + vliw::kNumSharedRegs * (int)sizeof(Fp) +
                                kManyGroups * (2 * (int)sizeof(G1Affine) + 2) + 64;
@@ -136,6 +151,7 @@ struct ProofTables {
 // ---- kernels (k_*.cu) ----------------------------------------------------------------------------------------
 __global__ void setup_tables_kernel(DeviceTables* T, const uint8_t* g2_points);
 __global__ void setup_lines29_kernel(DeviceTables* T);
+__global__ void setup_lines29w_kernel(DeviceTables* T, const uint8_t* g2_points, LineCoeffs* scratch);
 constexpr int kChallengeSlabs = 8;   // slab-wise arrival of the last host chunk (k_challenge.cu)
 void launch_challenge(int stages, cudaStream_t st, const uint8_t* blobs, const uint8_t* commitments, int n, Fr* z_mont, ZY* zy, Fr* zpow,
                       const uint8_t* slab_flags = nullptr);   // K2
@@ -168,6 +184,11 @@ void launch_msm_bucket_join(int lanes, int n, int slice, cudaStream_t st, const 
 __global__ void msm_window_kernel(const G1* __restrict__ buckets, G1* __restrict__ windows);
 __global__ void msm_combine_kernel(const G1* __restrict__ windows, const Fr* __restrict__ ry, const uint32_t* __restrict__ status, int n,
                                    const DeviceTables* __restrict__ T, Partial* __restrict__ out, uint32_t* flag, uint32_t epoch);
+__global__ void msm_sg_kernel(const Fr* __restrict__ ry, const uint32_t* __restrict__ status, int n, const DeviceTables* __restrict__ T,
+                              SplitTail* __restrict__ out);
+__global__ void window_prelude_kernel(const G1* __restrict__ windows, SplitTail* __restrict__ io);
+__global__ void window_miller_kernel(const DeviceTables* __restrict__ T, SplitTail* __restrict__ io, long long* __restrict__ ticks);
+__global__ void split_final_kernel(const SplitTail* __restrict__ io, uint32_t* __restrict__ result, Fp* __restrict__ gt, long long* __restrict__ ticks);
 __global__ void wait_flags_kernel(const uint32_t* flags, int count, uint32_t epoch, uint32_t* __restrict__ timed_out);
 __global__ void batch_final_kernel(const Partial* __restrict__ parts, int nparts, const DeviceTables* __restrict__ T, uint32_t* __restrict__ result,
                                    FinalPts* __restrict__ out);
@@ -175,16 +196,17 @@ __global__ void single_final_kernel(const G1Affine* __restrict__ C, const G1Affi
                                     const uint32_t* __restrict__ status, const DeviceTables* __restrict__ T, uint32_t* __restrict__ result,
                                     FinalPts* __restrict__ out);
 // lines_b: line table of the G2 point paired with pts[0]; nullptr = [tau]G2 (T->lines29[1], the blob checks)
+// gt (nullable): receives f^(3(p^12-1)/r) as 12 canonical integers
 __global__ void pairing_check_kernel(const FinalPts* __restrict__ in, const DeviceTables* __restrict__ T, const vliw29::LineCoeffs29* __restrict__ lines_b,
-                                     uint32_t* __restrict__ result, long long* __restrict__ ticks);
+                                     uint32_t* __restrict__ result, long long* __restrict__ ticks, Fp* __restrict__ gt);
 __global__ void engine_selftest_kernel(uint32_t seed, int rounds, f29::F29* __restrict__ ref, uint32_t* __restrict__ mismatches);
 // final check of a batch = G1 prelude + pairing engine, back to back on `st`; scratch512 = the context's 512-byte device scratch
 // (ticks at +128 when profiling, the hand-over points at +256); lines_b: see pairing_check_kernel (cells: [tau^64]G2)
 inline void launch_batch_final(cudaStream_t st, const Partial* parts, int nparts, const DeviceTables* T, uint32_t* result, unsigned char* scratch512,
-                               bool ticks, const vliw29::LineCoeffs29* lines_b = nullptr) {
+                               bool ticks, const vliw29::LineCoeffs29* lines_b = nullptr, Fp* gt = nullptr) {
     FinalPts* fp = reinterpret_cast<FinalPts*>(scratch512 + 256);
     batch_final_kernel<<<1, kFinalThreads, sizeof(FinalSmem), st>>>(parts, nparts, T, result, fp);
-    pairing_check_kernel<<<1, kPairThreads, sizeof(PairSmem), st>>>(fp, T, lines_b, result, ticks ? reinterpret_cast<long long*>(scratch512 + 128) : nullptr);
+    pairing_check_kernel<<<1, kPairThreads, sizeof(PairSmem), st>>>(fp, T, lines_b, result, ticks ? reinterpret_cast<long long*>(scratch512 + 128) : nullptr, gt);
 }
 __global__ void many_lhs_kernel(const uint8_t* __restrict__ z32, const uint8_t* __restrict__ y32, const G1Affine* __restrict__ C,
                                 const G1Affine* __restrict__ P, size_t m, const DeviceTables* __restrict__ T, G1Affine* __restrict__ X,

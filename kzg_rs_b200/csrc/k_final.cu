@@ -43,7 +43,7 @@ __global__ void __launch_bounds__(kFinalThreads) batch_final_kernel(const Partia
 // point whose line table lines_b is (cell proofs: [tau^64]G2).
 __global__ void __launch_bounds__(kPairThreads) pairing_check_kernel(const FinalPts* __restrict__ in, const DeviceTables* __restrict__ T,
                                                                      const vliw29::LineCoeffs29* __restrict__ lines_b, uint32_t* __restrict__ result,
-                                                                     long long* __restrict__ ticks) {
+                                                                     long long* __restrict__ ticks, Fp* __restrict__ gt) {
     extern __shared__ __align__(16) unsigned char dyn_smem[];
     PairSmem& S = *reinterpret_cast<PairSmem*>(dyn_smem);
     const int t = threadIdx.x;
@@ -52,7 +52,82 @@ __global__ void __launch_bounds__(kPairThreads) pairing_check_kernel(const Final
     vliw29::Tables tab = vliw29::load_tables(&S.stab, t, kPairThreads);
     vliw29::Lanes L{t, kPairThreads, tab, ticks, S.stab.p29};
     const G1Affine p0 = in->pts[0], p1 = in->pts[1];
-    bool ok = vliw29::coop_pairing_product_is_one(S.regs, p1, T->lines29[0], p0, lines_b ? lines_b : T->lines29[1], L);
+    bool ok = vliw29::coop_pairing_product_is_one(S.regs, p1, T->lines29[0], p0, lines_b ? lines_b : T->lines29[1], L, gt);
+    L.tick(5);
+    if (t == 0) { result[0] = ok ? kTrue : kFalse; result[1] = 0; }
+}
+
+// Split tail of a single-GPU batch (kzgb200_ctx::final_split).  With A = sum_w 256^w W0_w and B = sum_w 256^w B_w (W*_w: the
+// MSM window sums of the three point sets, B_w = W1_w + W2_w, B_0 also - [s]G), bilinearity gives
+//   e(-A, [tau]G2) e(B, G2) = prod_w e(-W0_w, [256^w tau]G2) e(B_w, [256^w]G2),
+// and the final exponentiation is a homomorphism, so FE(prod_w Miller_w) is the very GT element of the combined check.  The G2
+// multiples are setup constants (lines29w), so the Horner chain of msm_combine_kernel (120 doublings + 16 additions) leaves the
+// critical path: window_prelude_kernel forms every window's two affine points, CTA w of window_miller_kernel runs its Miller loop,
+// split_final_kernel multiplies the 16 values and runs the final exponentiation.
+// Prelude: one CTA of kFinalThreads threads per window (a kernel of its own, as batch_final_kernel: the G1 sums and the inversion
+// inside the 768-thread engine kernel would spill); lane 0 of warps 0 and 1 run the two inversions side by side.
+__global__ void __launch_bounds__(kFinalThreads) window_prelude_kernel(const G1* __restrict__ windows, SplitTail* __restrict__ io) {
+    const int t = threadIdx.x, w = blockIdx.x;
+    if (io->err || (t & 31) != 0) return;         // BadArgs: split_final_kernel writes the result
+    const int k = t >> 5;
+    G1 acc;
+    if (k == 0) acc = windows[w].neg();                                       // -W0_w
+    else {
+        acc = windows[kWindows + w].add(windows[2 * kWindows + w]);           // B_w
+        if (w == 0) acc = acc.add(io->sg.neg());
+    }
+    Fp zi = vliw::fp_inv_bingcd(acc.z), zi2 = zi.sqr();
+    io->pts[w][k] = acc.is_identity() ? G1Affine{Fp::zero(), Fp::zero(), 1} : G1Affine{acc.x * zi2, acc.y * zi2 * zi, 0};
+}
+// Miller loop of window w = blockIdx.x on the lines of [256^w]G2 and [256^w tau]G2 (one-pair script for an identity point, f = 1
+// for two).  ticks (profiling, nullable): ticks[2] receives the longest Miller time over the CTAs (split_final_kernel rebases it).
+__global__ void __launch_bounds__(kPairThreads) window_miller_kernel(const DeviceTables* __restrict__ T, SplitTail* __restrict__ io,
+                                                                     long long* __restrict__ ticks) {
+    extern __shared__ __align__(16) unsigned char dyn_smem[];
+    PairSmem& S = *reinterpret_cast<PairSmem*>(dyn_smem);
+    const int t = threadIdx.x, w = blockIdx.x;
+    if (io->err) return;
+    const long long c0 = clock64();
+    vliw29::Tables tab = vliw29::load_tables(&S.stab, t, kPairThreads);
+    vliw29::Lanes L{t, kPairThreads, tab, nullptr, S.stab.p29};
+    const vliw29::LineCoeffs29* lg = w ? T->lines29w[0][w - 1] : T->lines29[0];
+    const vliw29::LineCoeffs29* lt = w ? T->lines29w[1][w - 1] : T->lines29[1];
+    vliw29::coop_miller(S.regs, io->pts[w][1], lg, io->pts[w][0], lt, L);
+    uint4* dst = reinterpret_cast<uint4*>(io->f[w]);
+    const uint4* src = reinterpret_cast<const uint4*>(S.regs + vliw29::kRegF);
+    for (int i = t; i < 12 * 4; i += kPairThreads) dst[i] = src[i];
+    if (ticks && t == 0) atomicMax(&ticks[2], clock64() - c0);
+}
+// product of the 16 window Miller values (15 f12_mul in a row: the program has 3 levels, a 4-level tree over 8 register files
+// would run more passes of its wider levels than it saves), final exponentiation, == 1.  Same result words as pairing_check_kernel.
+__global__ void __launch_bounds__(kPairThreads) split_final_kernel(const SplitTail* __restrict__ io, uint32_t* __restrict__ result, Fp* __restrict__ gt,
+                                                                   long long* __restrict__ ticks) {
+    extern __shared__ __align__(16) unsigned char dyn_smem[];
+    PairSmem& S = *reinterpret_cast<PairSmem*>(dyn_smem);
+    const int t = threadIdx.x;
+    if (io->err) { if (t == 0) { result[0] = kBadArgs; result[1] = io->err; } return; }
+    if (ticks && t == 0) {              // stamps on this SM's clock: the longest window Miller loop ends at this start
+        const long long c0 = clock64(), mil = ticks[2];
+        ticks[0] = c0 - mil; ticks[1] = c0 - mil; ticks[2] = c0;
+        for (int i = 6; i < 14; i++) ticks[i] = 0;
+    }
+    vliw29::Tables tab = vliw29::load_tables(&S.stab, t, kPairThreads);
+    vliw29::Lanes L{t, kPairThreads, tab, ticks, S.stab.p29};
+    {
+        uint4* dst = reinterpret_cast<uint4*>(S.regs + vliw29::kRegF);
+        const uint4* src = reinterpret_cast<const uint4*>(io->f[0]);
+        for (int i = t; i < 12 * 4; i += kPairThreads) dst[i] = src[i];
+        for (int i = t; i < 10; i += kPairThreads) S.regs[vliw29::kRegConst + i] = vliw29::frob_const(i);
+    }
+    for (int w = 1; w < kWindows; w++) {
+        uint4* dst = reinterpret_cast<uint4*>(S.regs + vliw29::kRegG);
+        const uint4* src = reinterpret_cast<const uint4*>(io->f[w]);
+        for (int i = t; i < 12 * 4; i += kPairThreads) dst[i] = src[i];
+        L.sync();
+        vliw29::run(vliw29::kProg_f12_mul, S.regs, L);      // F <- F * G
+    }
+    L.sync();
+    const bool ok = vliw29::coop_final_exp_is_one(S.regs, L, gt);
     L.tick(5);
     if (t == 0) { result[0] = ok ? kTrue : kFalse; result[1] = 0; }
 }

@@ -221,9 +221,36 @@ __global__ void __launch_bounds__(kWinLanes) msm_window_kernel(const G1* __restr
 // table (64 lookups, a 6-level tree); the partial carries B' - [s]G and ry = 0, so the final check has no fixed-base work left.
 // `out` may be a peer-mapped pointer into the group leader's exchange buffer (multi-GPU: the partial-sum gather is this kernel's
 // last store, over NVLink); then `flag` (same buffer) receives `epoch` after the partial, with a system-scope fence in between.
-constexpr int kCombEngine = 384, kCombHelpers = 160;          // kCombineThreads = 544 (common.cuh)
+constexpr int kCombEngine = 384;                              // kCombineThreads = 544, kCombHelpers = 160 (common.cuh)
 constexpr int kCombRegs = 96;                                  // registers per chain: g1_add needs 83; 90..92 = saved accumulator
 static_assert(kCombEngine + kCombHelpers == kCombineThreads, "thread split of msm_combine_kernel");
+// kCombHelpers threads (h = 0..kCombHelpers-1, meeting at `bar`): OR of the per-blob error flags into *err (shared), s = sum r_i y_i
+// tree-summed in sry[kCombHelpers], [s]G from the fixed-base table (64 lookups, a 6-level tree) into sg[0] (sg: 64 shared points)
+template <class Bar>
+__device__ __forceinline__ void sum_s_sg(int h, const Fr* __restrict__ ry, const uint32_t* __restrict__ status, int n, const DeviceTables* __restrict__ T,
+                                         uint32_t* err, Fr* sry, G1* sg, Bar bar) {
+    uint32_t e = 0;
+    Fr acc_ry = Fr::zero();
+    for (int i = h; i < n; i += kCombHelpers) { e |= status[i]; acc_ry = acc_ry.add_inl(ry[i]); }
+    if (e) atomicOr(err, e);
+    sry[h] = acc_ry;
+    bar();
+    for (int span = 128; span >= 1; span >>= 1) {
+        if (h < span && h + span < kCombHelpers) sry[h] = sry[h].add_inl(sry[h + span]);
+        bar();
+    }
+    // [s]G: helper h < 64 takes the h-th 4-bit digit of s (normal form), then a tree over the 64 table points
+    if (h < 64) {
+        const Fr sv = sry[0];
+        const uint32_t d = (sv.l[h / 8] >> (4 * (h % 8))) & 15u;
+        sg[h] = d ? G1::from_affine(T->gen_table[h][d - 1]) : G1::identity();
+    }
+    bar();
+    for (int span = 32; span >= 1; span >>= 1) {
+        if (h < span) sg[h] = sg[h].add(sg[h + span]);
+        bar();
+    }
+}
 struct CombineSmem {
     f29::F29 regs[kMsmSets][kCombRegs];
     f29::F29 win[kMsmSets][kWindows][3];
@@ -310,28 +337,7 @@ __global__ void __launch_bounds__(kCombineThreads) msm_combine_kernel(const G1* 
         }
     } else {
         // helpers, beside the chains: OR of the per-blob error flags, s = sum r_i y_i, [s]G
-        const int h = t - kCombEngine;
-        uint32_t e = 0;
-        Fr acc_ry = Fr::zero();
-        for (int i = h; i < n; i += kCombHelpers) { e |= status[i]; acc_ry = acc_ry.add_inl(ry[i]); }
-        if (e) atomicOr(&s_err, e);
-        s_ry[h] = acc_ry;
-        asm volatile("bar.sync 1, %0;" ::"n"(kCombHelpers) : "memory");
-        for (int span = 128; span >= 1; span >>= 1) {
-            if (h < span && h + span < kCombHelpers) s_ry[h] = s_ry[h].add_inl(s_ry[h + span]);
-            asm volatile("bar.sync 1, %0;" ::"n"(kCombHelpers) : "memory");
-        }
-        // [s]G: helper h < 64 takes the h-th 4-bit digit of s (normal form), then a tree over the 64 table points
-        if (h < 64) {
-            const Fr sv = s_ry[0];
-            const uint32_t d = (sv.l[h / 8] >> (4 * (h % 8))) & 15u;
-            s_sg[h] = d ? G1::from_affine(T->gen_table[h][d - 1]) : G1::identity();
-        }
-        asm volatile("bar.sync 1, %0;" ::"n"(kCombHelpers) : "memory");
-        for (int span = 32; span >= 1; span >>= 1) {
-            if (h < span) s_sg[h] = s_sg[h].add(s_sg[h + span]);
-            asm volatile("bar.sync 1, %0;" ::"n"(kCombHelpers) : "memory");
-        }
+        sum_s_sg(t - kCombEngine, ry, status, n, T, &s_err, s_ry, s_sg, [] { asm volatile("bar.sync 1, %0;" ::"n"(kCombHelpers) : "memory"); });
     }
     __syncthreads();
     const int warp = t >> 5, lane = t & 31;
@@ -347,6 +353,20 @@ __global__ void __launch_bounds__(kCombineThreads) msm_combine_kernel(const G1* 
         __syncthreads();
         if (t == 0) { *reinterpret_cast<volatile uint32_t*>(flag) = epoch; __threadfence_system(); }
     }
+}
+
+// the helpers' work of msm_combine_kernel on their own CTA (kCombHelpers threads), for the split tail: launched beside the bucket
+// phase, it hands [s]G and the flags to window_miller_kernel off the critical path
+__global__ void __launch_bounds__(kCombHelpers) msm_sg_kernel(const Fr* __restrict__ ry, const uint32_t* __restrict__ status, int n,
+                                                              const DeviceTables* __restrict__ T, SplitTail* __restrict__ out) {
+    __shared__ uint32_t s_err;
+    __shared__ Fr s_ry[kCombHelpers];
+    __shared__ G1 s_sg[64];
+    const int t = threadIdx.x;
+    if (t == 0) s_err = 0;
+    __syncthreads();
+    sum_s_sg(t, ry, status, n, T, &s_err, s_ry, s_sg, [] { __syncthreads(); });
+    if (t == 0) { out->sg = s_sg[0]; out->err = s_err; }
 }
 
 }  // namespace kzgb200

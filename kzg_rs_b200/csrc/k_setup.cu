@@ -54,4 +54,24 @@ __global__ void setup_lines29_kernel(DeviceTables* T) {
     T->lines29[q][k].v[e] = f29::from_fp((e & 1) ? f2.c1 : f2.c0);
 }
 
+// line tables of [256^w]Q, Q in {G2, [tau]G2}, w = 1..15, for the split tail of the batch check (one thread per table: 8w doublings,
+// affine conversion, the 68 line triples into `scratch` (30 x kMillerSteps), then the engine's representation).  Built from the
+// context's own G2 points, so a custom setup gets its own tables.
+__global__ void setup_lines29w_kernel(DeviceTables* T, const uint8_t* g2_points /* 2 x 96 B */, LineCoeffs* scratch) {
+    const int tid = blockIdx.x * blockDim.x + threadIdx.x;
+    if (tid >= 2 * (kWindows - 1)) return;
+    const int q = tid / (kWindows - 1), w = tid % (kWindows - 1) + 1;
+    G2Affine base;
+    if (!g2_from_compressed_unchecked(base, g2_points + 96 * q) || base.inf) return;    // setup_tables_kernel reports the failure
+    G2 acc = G2::from_affine(base);
+    for (int k = 0; k < 8 * w; k++) acc = acc.dbl();
+    LineCoeffs* lc = scratch + (size_t)tid * kMillerSteps;
+    prepare_g2(lc, g2_to_affine(acc));
+    for (int k = 0; k < kMillerSteps; k++)
+        for (int e = 0; e < 6; e++) {
+            const Fp2& f2 = e < 2 ? lc[k].A : (e < 4 ? lc[k].B : lc[k].C);
+            T->lines29w[q][w - 1][k].v[e] = f29::from_fp((e & 1) ? f2.c1 : f2.c0);
+        }
+}
+
 }  // namespace kzgb200

@@ -389,10 +389,18 @@ static int msm_slice_len(const kzgb200_ctx* ctx, int n) {
     return slice < kMinSlice ? kMinSlice : slice;
 }
 // K6: digits, counting sort, buckets, window sums, Horner -> partial (optionally stored into a peer's exchange buffer + flag)
-int launch_lincomb(kzgb200_ctx* ctx, size_t offset, Partial* d_out, bool wait_subgroup, uint32_t* d_flag, uint32_t epoch, const Fr* d_weights) {
+int launch_lincomb(kzgb200_ctx* ctx, size_t offset, Partial* d_out, bool wait_subgroup, uint32_t* d_flag, uint32_t epoch, const Fr* d_weights,
+                   bool split) {
     int n = (int)ctx->cur_n;
     phase_begin(ctx, kPhLincomb, ctx->stream);
     msm_scalars_kernel<<<(n + 127) / 128, 128, 0, ctx->stream>>>(ctx->d_z_mont, ctx->d_zy, ctx->d_r, (uint64_t)offset, n, ctx->d_digits, ctx->d_ry, d_weights);
+    if (split) {        // s = sum r_i y_i, [s]G and the flags on one CTA beside the bucket phase
+        CK(cudaEventRecord(ctx->ev_sg, ctx->stream));
+        CK(cudaStreamWaitEvent(ctx->s_tail, ctx->ev_sg, 0));
+        if (wait_subgroup) CK(cudaStreamWaitEvent(ctx->s_tail, ctx->ev_parse, 0));
+        msm_sg_kernel<<<1, kCombHelpers, 0, ctx->s_tail>>>(ctx->d_ry, ctx->d_status, n, ctx->tables, ctx->d_split);
+        CK(cudaEventRecord(ctx->ev_sg, ctx->s_tail));
+    }
     msm_sort_kernel<<<kDigitRows, 256, 0, ctx->stream>>>(ctx->d_digits, n, ctx->d_order, ctx->d_start);
     {
         const int slice = msm_slice_len(ctx, n);
@@ -411,14 +419,45 @@ int launch_lincomb(kzgb200_ctx* ctx, size_t offset, Partial* d_out, bool wait_su
         CK(cudaEventRecord(ctx->ev_bucket, ctx->stream));
         CK(cudaStreamWaitEvent(ctx->s_aux, ctx->ev_bucket, 0));
         if (ctx->profile) cudaEventRecord(ctx->ev_s[7], ctx->s_aux);
-        g1_subgroup_kernel<<<ctx->num_sms - kTailSms, 256, kTailHogSmem, ctx->s_aux>>>(ctx->d_C, ctx->d_P, n, ctx->d_status);
+        g1_subgroup_kernel<<<ctx->num_sms - (split ? kTailSmsSplit : kTailSms), 256, kTailHogSmem, ctx->s_aux>>>(ctx->d_C, ctx->d_P, n, ctx->d_status);
         if (ctx->profile) { cudaEventRecord(ctx->ev_e[7], ctx->s_aux); ctx->ph_started[7] = true; }
         CK(cudaEventRecord(ctx->ev_parse, ctx->s_aux));
         ctx->subgroup_pending = false;
     }
+    if (split) {        // the combined partial (kzgb200_last_partial) beside the window Miller CTAs: off the critical path
+        phase_end(ctx, kPhReduce, ctx->stream);
+        CK(cudaEventRecord(ctx->ev_comb, ctx->stream));
+        CK(cudaStreamWaitEvent(ctx->s_tail, ctx->ev_comb, 0));
+        msm_combine_kernel<<<1, kCombineThreads, kCombineSmemBytes, ctx->s_tail>>>(ctx->d_windows, ctx->d_ry, ctx->d_status, n, ctx->tables, d_out, d_flag, epoch);
+        CK(cudaEventRecord(ctx->ev_comb, ctx->s_tail));
+        CK(cudaGetLastError());
+        return KZGB200_OK;
+    }
     if (wait_subgroup) CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_parse, 0));    // combine ORs the per-blob error flags
     msm_combine_kernel<<<1, kCombineThreads, kCombineSmemBytes, ctx->stream>>>(ctx->d_windows, ctx->d_ry, ctx->d_status, n, ctx->tables, d_out, d_flag, epoch);
     phase_end(ctx, kPhReduce, ctx->stream);
+    CK(cudaGetLastError());
+    return KZGB200_OK;
+}
+// K6 + K7 of a single-GPU batch against [tau]G2 (batch verdict in d_result, f^(3(p^12-1)/r) in d_split->gt): the split tail
+// (window_miller_kernel) or, with final_split = 0, the Horner combination + one pairing check.  phase_final: open the final phase
+// (closed by the caller); ticks: kzgb200_debug_final_ticks stamps.
+int launch_batch_check(kzgb200_ctx* ctx, bool wait_subgroup, bool phase_final, bool ticks) {
+    int rc;
+    const bool split = ctx->final_split != 0;
+    if ((rc = launch_lincomb(ctx, 0, ctx->d_partial, wait_subgroup, nullptr, 0, nullptr, split))) return rc;
+    if (phase_final) phase_begin(ctx, kPhFinal, ctx->stream);
+    if (!split) {
+        launch_batch_final(ctx->stream, ctx->d_partial, 1, ctx->tables, ctx->d_result, ctx->d_scratch, ticks, nullptr, ctx->d_split->gt);
+    } else {
+        long long* tk = ticks ? reinterpret_cast<long long*>(ctx->d_scratch + 128) : nullptr;
+        if (tk) CK(cudaMemsetAsync(tk, 0, 14 * sizeof(long long), ctx->stream));
+        CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_sg, 0));
+        window_prelude_kernel<<<kWindows, kFinalThreads, sizeof(FinalSmem), ctx->stream>>>(ctx->d_windows, ctx->d_split);
+        window_miller_kernel<<<kWindows, kPairThreads, sizeof(PairSmem), ctx->stream>>>(ctx->tables, ctx->d_split, tk);
+        split_final_kernel<<<1, kPairThreads, sizeof(PairSmem), ctx->stream>>>(ctx->d_split, ctx->d_result, ctx->d_split->gt, tk);
+        CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_comb, 0));     // the combined partial is in place when the call returns
+    }
     CK(cudaGetLastError());
     return KZGB200_OK;
 }
@@ -463,12 +502,14 @@ extern "C" int kzgb200_create(kzgb200_ctx** out, int device, const uint8_t* g2_p
         if (const char* v = getenv("KZGB200_MSM_SLICE")) ctx->msm_slice = atoi(v);
         if (const char* v = getenv("KZGB200_MSM_JOIN")) ctx->msm_join = atoi(v);
         if (const char* v = getenv("KZGB200_MSM_OCC")) { int o = atoi(v); if (o >= 2 && o <= 4) ctx->msm_occ = o; }
+        if (const char* v = getenv("KZGB200_FINAL_SPLIT")) ctx->final_split = atoi(v) != 0;
         if (const char* v = getenv("KZGB200_TRANSCRIPT")) ctx->transcript_mode = !strcmp(v, "tree") ? KZGB200_TRANSCRIPT_TREE : (!strcmp(v, "device") ? KZGB200_TRANSCRIPT_EXACT_DEVICE : KZGB200_TRANSCRIPT_EXACT);
         CK(cudaFuncSetAttribute(g1_subgroup_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kTailHogSmem));
         CK(cudaStreamCreateWithFlags(&ctx->s_copy, cudaStreamNonBlocking));
         CK(cudaStreamCreateWithPriority(&ctx->s_d2h, cudaStreamNonBlocking, prio_hi));
         for (auto& w : ctx->s_work) CK(cudaStreamCreateWithPriority(&w, cudaStreamNonBlocking, prio_hi));
-        for (cudaEvent_t* e : {&ctx->ev_begin, &ctx->ev_parse, &ctx->ev_decomp, &ctx->ev_bucket, &ctx->ev_sha_all, &ctx->ev_leaf})
+        CK(cudaStreamCreateWithPriority(&ctx->s_tail, cudaStreamNonBlocking, prio_hi));
+        for (cudaEvent_t* e : {&ctx->ev_begin, &ctx->ev_parse, &ctx->ev_decomp, &ctx->ev_bucket, &ctx->ev_sha_all, &ctx->ev_leaf, &ctx->ev_sg, &ctx->ev_comb})
             CK(cudaEventCreateWithFlags(e, cudaEventDisableTiming));
         for (auto& e : ctx->ev_h2d) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
         for (auto& e : ctx->ev_zy) CK(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
@@ -479,12 +520,17 @@ extern "C" int kzgb200_create(kzgb200_ctx** out, int device, const uint8_t* g2_p
         CK(cudaFuncSetAttribute(batch_final_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FinalSmem)));
         CK(cudaFuncSetAttribute(single_final_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FinalSmem)));
         CK(cudaFuncSetAttribute(pairing_check_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PairSmem)));
+        CK(cudaFuncSetAttribute(window_prelude_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(FinalSmem)));
+        CK(cudaFuncSetAttribute(window_miller_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PairSmem)));
+        CK(cudaFuncSetAttribute(split_final_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(PairSmem)));
         CK(cudaFuncSetAttribute(msm_combine_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCombineSmemBytes));
         CK(cudaFuncSetAttribute(many_pairing_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kManySmemBytes));
         CK(cudaFuncSetAttribute(many_pairing_warp_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kManySmemBytes));
         CK(cudaMalloc(&ctx->tables, sizeof(DeviceTables)));
         CK(cudaMalloc(&ctx->d_r, sizeof(Fr)));
         CK(cudaMalloc(&ctx->d_partial, sizeof(Partial)));
+        CK(cudaMalloc(&ctx->d_split, sizeof(SplitTail)));
+        CK(cudaMemsetAsync(ctx->d_split, 0, sizeof(SplitTail), ctx->stream));
         CK(cudaMalloc(&ctx->d_result, 16));
         CK(cudaMalloc(&ctx->d_start, kDigitRows * (kBuckets + 1) * sizeof(uint32_t)));
         CK(cudaMalloc(&ctx->d_buckets, kMsmSets * kWindows * kBuckets * sizeof(G1)));
@@ -500,11 +546,15 @@ extern "C" int kzgb200_create(kzgb200_ctx** out, int device, const uint8_t* g2_p
         CK(cudaMemcpyAsync(d_g2, g2_points, 192, cudaMemcpyHostToDevice, ctx->stream));
         setup_tables_kernel<<<(8192 + 4096) / 128, 128, 0, ctx->stream>>>(ctx->tables, d_g2);
         setup_lines29_kernel<<<(2 * kMillerSteps * 6 + 127) / 128, 128, 0, ctx->stream>>>(ctx->tables);
+        LineCoeffs* d_lines_tmp = nullptr;
+        CK(cudaMalloc(&d_lines_tmp, 2 * (kWindows - 1) * kMillerSteps * sizeof(LineCoeffs)));
+        setup_lines29w_kernel<<<1, 32, 0, ctx->stream>>>(ctx->tables, d_g2, d_lines_tmp);
         CK(cudaGetLastError());
         uint32_t ok = 0;
         CK(cudaMemcpyAsync(&ok, &ctx->tables->setup_ok, 4, cudaMemcpyDeviceToHost, ctx->stream));
         CK(cudaStreamSynchronize(ctx->stream));
         cudaFree(d_g2);
+        cudaFree(d_lines_tmp);
         return ok ? KZGB200_OK : KZGB200_INVALID_SETUP;
     }();
     if (rc != KZGB200_OK) return fail(rc);
@@ -519,8 +569,8 @@ extern "C" void kzgb200_destroy(kzgb200_ctx* ctx) {
     cudaDeviceSynchronize();
     cell_destroy(ctx);
     delete ctx->pool;
-    for (cudaStream_t st : {ctx->s_aux, ctx->s_copy, ctx->s_d2h, ctx->s_work[0], ctx->s_work[1], ctx->s_work[2], ctx->s_work[3]}) if (st) cudaStreamDestroy(st);
-    for (cudaEvent_t e : {ctx->ev_begin, ctx->ev_parse, ctx->ev_decomp, ctx->ev_bucket, ctx->ev_sha_all, ctx->ev_leaf}) if (e) cudaEventDestroy(e);
+    for (cudaStream_t st : {ctx->s_tail, ctx->s_aux, ctx->s_copy, ctx->s_d2h, ctx->s_work[0], ctx->s_work[1], ctx->s_work[2], ctx->s_work[3]}) if (st) cudaStreamDestroy(st);
+    for (cudaEvent_t e : {ctx->ev_begin, ctx->ev_parse, ctx->ev_decomp, ctx->ev_bucket, ctx->ev_sha_all, ctx->ev_leaf, ctx->ev_sg, ctx->ev_comb}) if (e) cudaEventDestroy(e);
     for (auto e : ctx->ev_h2d) if (e) cudaEventDestroy(e);
     for (auto e : ctx->ev_zy) if (e) cudaEventDestroy(e);
     for (auto e : ctx->ev_zyh) if (e) cudaEventDestroy(e);
@@ -530,7 +580,7 @@ extern "C" void kzgb200_destroy(kzgb200_ctx* ctx) {
     void* ptrs[] = {ctx->tables, ctx->d_blobs, ctx->d_c, ctx->d_p, ctx->d_z_mont, ctx->d_zy, ctx->d_C, ctx->d_P, ctx->d_status,
                     ctx->d_ry, ctx->d_r, ctx->d_partial, ctx->d_result, ctx->d_zout, ctx->d_yout, ctx->d_many, ctx->d_wk,
                     ctx->d_digits, ctx->d_order, ctx->d_start, ctx->d_buckets, ctx->d_halfsum, ctx->d_part, ctx->d_windows, ctx->d_lag_table, ctx->d_scalars, ctx->d_lag_part, ctx->d_zpow,
-                    ctx->d_chain_state, ctx->d_scratch, ctx->d_digest};
+                    ctx->d_chain_state, ctx->d_scratch, ctx->d_digest, ctx->d_split};
     for (void* p : ptrs) if (p) cudaFree(p);
     void* hptrs[] = {ctx->h_flags, ctx->h_result, ctx->h_digest, ctx->h_partial, ctx->h_zy, ctx->h_c, ctx->h_p, ctx->h_stage[0], ctx->h_stage[1], ctx->h_stage[2], ctx->h_stage[3]};
     for (void* p : hptrs) if (p) cudaFreeHost(p);
@@ -568,13 +618,11 @@ static int batch_locked(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t*
         CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_parse, 0));
         FinalPts* fp = reinterpret_cast<FinalPts*>(ctx->d_scratch + 256);
         single_final_kernel<<<1, kFinalThreads, sizeof(FinalSmem), ctx->stream>>>(ctx->d_C, ctx->d_P, ctx->d_zy, ctx->d_status, ctx->tables, ctx->d_result, fp);
-        pairing_check_kernel<<<1, kPairThreads, sizeof(PairSmem), ctx->stream>>>(fp, ctx->tables, nullptr, ctx->d_result, nullptr);
+        pairing_check_kernel<<<1, kPairThreads, sizeof(PairSmem), ctx->stream>>>(fp, ctx->tables, nullptr, ctx->d_result, nullptr, nullptr);
     } else {
         if ((rc = transcript_progress(ctx, true))) return rc;     // the host hashes the transcript behind the evaluation chunks
         if ((rc = transcript_finish(ctx))) return rc;
-        if ((rc = launch_lincomb(ctx, 0, ctx->d_partial, !defer))) return rc;   // deferred: the flags are merged by status_or below
-        phase_begin(ctx, kPhFinal, ctx->stream);
-        launch_batch_final(ctx->stream, ctx->d_partial, 1, ctx->tables, ctx->d_result, ctx->d_scratch, true);
+        if ((rc = launch_batch_check(ctx, !defer, true, true))) return rc;   // deferred: the flags are merged by status_or below
     }
     phase_end(ctx, kPhFinal, ctx->stream);
     // the deferred subgroup checks may still be running beside the pairing: their flags are merged last
@@ -648,8 +696,7 @@ extern "C" int kzgb200_verify_blob_kzg_proof_batch_each(kzgb200_ctx* ctx, const 
     if (n >= 2) {
         if ((rc = transcript_progress(ctx, true))) return rc;
         if ((rc = transcript_finish(ctx))) return rc;
-        if ((rc = launch_lincomb(ctx, 0, ctx->d_partial, true))) return rc;
-        launch_batch_final(ctx->stream, ctx->d_partial, 1, ctx->tables, ctx->d_result, ctx->d_scratch, false);
+        if ((rc = launch_batch_check(ctx, true, false, false))) return rc;
         status_or_kernel<<<1, 256, 0, ctx->stream>>>(ctx->d_status, (int)n, ctx->d_result + 2);
         CK(cudaGetLastError());
         rc = read_result(ctx, &ok);
@@ -701,8 +748,7 @@ extern "C" int kzgb200_verify_kzg_proof_batch(kzgb200_ctx* ctx, const uint8_t* c
     if ((rc = transcript_enqueue_chunk(ctx, 0, ctx->d_c, ctx->d_p))) return rc;
     if ((rc = transcript_progress(ctx, true))) return rc;
     if ((rc = transcript_finish(ctx))) return rc;
-    if ((rc = launch_lincomb(ctx, 0, ctx->d_partial, false))) return rc;
-    launch_batch_final(ctx->stream, ctx->d_partial, 1, ctx->tables, ctx->d_result, ctx->d_scratch, false);
+    if ((rc = launch_batch_check(ctx, false, false, false))) return rc;
     CK(cudaMemsetAsync(ctx->d_result + 2, 0, 4, ctx->stream));
     CK(cudaGetLastError());
     return read_result(ctx, ok);
@@ -1001,7 +1047,28 @@ extern "C" int kzgb200_compute_blob_kzg_proof(kzgb200_ctx* ctx, const uint8_t* b
     if (!ctx || !blob || !commitment48 || !proof_out48) return KZGB200_BAD_ARGS;
     return prove_host(ctx, blob, commitment48, 48, kProveBlob, proof_out48, nullptr);
 }
-// clock64() stamps of the last single-GPU batch_final_kernel: start, prelude end, Miller loop end, easy part end, hard part end, done
+// f^(3(p^12-1)/r) of the last single-GPU batch check (either tail): 12 canonical Fp values, 48 little-endian bytes each, in the
+// order c0.c0.c0, c0.c0.c1, c0.c1.c0, ... of the engine's F slot
+extern "C" int kzgb200_debug_last_gt(kzgb200_ctx* ctx, uint8_t* out576) {
+    if (!ctx || !out576) return KZGB200_BAD_ARGS;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    CK(cudaMemcpyAsync(out576, ctx->d_split->gt, 12 * sizeof(Fp), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return KZGB200_OK;
+}
+// the shifted line tables of the split tail (DeviceTables::lines29w: [2][15][68][6] values of 16 little-endian 32-bit words)
+extern "C" int kzgb200_debug_lines29w(kzgb200_ctx* ctx, uint8_t* out, size_t len) {
+    if (!ctx || !out || len != sizeof(DeviceTables::lines29w)) return KZGB200_BAD_ARGS;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    CK(cudaMemcpyAsync(out, ctx->tables->lines29w, len, cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    return KZGB200_OK;
+}
+// clock64() stamps of the last single-GPU batch check: start, prelude end, Miller loop end, easy part end, hard part end, done.  With the
+// split tail the first three are rebased onto the product CTA's clock from the longest window CTA, and the product of the 16
+// Miller values counts into the easy part.
 extern "C" int kzgb200_debug_final_ticks(kzgb200_ctx* ctx, long long* out14) {
     if (!ctx || !out14) return KZGB200_BAD_ARGS;
     std::lock_guard<std::mutex> g(ctx->lock);

@@ -16,6 +16,7 @@
 namespace kzgb200 {
 
 constexpr int kTailSms = 8;                    // SMs kept free of deferred subgroup checks for the latency-bound tail kernels
+constexpr int kTailSmsSplit = 20;              // ... with the split tail: 16 window Miller CTAs, msm_combine_kernel, the product CTA
 constexpr int kTailHogSmem = 200 * 1024;       // dynamic shared memory of a subgroup-check CTA in deferred mode (never touched)
 constexpr int kTailPadSmem = 28 * 1024;        // ... and of the tail kernels: 200 KB + 28 KB do not fit one SM
 static_assert(sizeof(FinalSmem) >= (size_t)kTailPadSmem && sizeof(PairSmem) >= (size_t)kTailPadSmem, "the final-check kernels must not fit beside a subgroup-check CTA");
@@ -143,6 +144,10 @@ struct kzgb200_ctx {
     int pageable_mode = 0;          // 0 = pinned staging ring, 1 = plain cudaMemcpyAsync (driver staging), 2 = cudaHostRegister in place
     bool subgroup_pending = false;
     int parse_first = 0;            // tuning: launch G1 parsing before the first hash launch (env KZGB200_PARSE_FIRST)
+    int final_split = 1;            // batch check against [tau]G2: per-window Miller loops on the [256^w]-scaled G2 lines (env KZGB200_FINAL_SPLIT=0: Horner + one pairing)
+    kzgb200::SplitTail* d_split = nullptr;
+    cudaStream_t s_tail = nullptr;  // split tail: msm_sg_kernel, then msm_combine_kernel
+    cudaEvent_t ev_sg = nullptr, ev_comb = nullptr;
     cudaStream_t s_aux = nullptr, s_copy = nullptr, s_d2h = nullptr, s_work[kzgb200::kWorkStreams] = {nullptr, nullptr, nullptr, nullptr};
     cudaEvent_t ev_begin = nullptr, ev_parse = nullptr, ev_decomp = nullptr, ev_bucket = nullptr, ev_sha_all = nullptr, ev_leaf = nullptr;
     cudaEvent_t ev_h2d[kzgb200::kMaxChunks] = {nullptr}, ev_zy[kzgb200::kMaxChunks] = {nullptr}, ev_zyh[kzgb200::kMaxChunks] = {nullptr};
@@ -207,8 +212,10 @@ int transcript_finish(kzgb200_ctx* ctx);
 // upload a 32-byte transcript digest computed elsewhere (multi-GPU: the group leader) and derive r from it
 int upload_r_digest(kzgb200_ctx* ctx, const uint8_t digest[32]);
 // d_weights: per-entry scalars in place of r^(offset + i) (cell groups), nullptr = the powers of r
+// split: the split tail follows (kzgb200_ctx::final_split): [s]G and the flags go to d_split beside the bucket phase (ev_sg), and
+// msm_combine_kernel runs on s_tail beside the window Miller CTAs (ev_comb)
 int launch_lincomb(kzgb200_ctx* ctx, size_t offset, Partial* d_out, bool wait_subgroup, uint32_t* d_flag = nullptr, uint32_t epoch = 0,
-                   const Fr* d_weights = nullptr);
+                   const Fr* d_weights = nullptr, bool split = false);
 int read_result(kzgb200_ctx* ctx, int* ok);
 int export_zy(kzgb200_ctx* ctx, size_t n, uint8_t* d_z, uint8_t* d_y);
 void phase_begin(kzgb200_ctx* ctx, int ph, cudaStream_t st);

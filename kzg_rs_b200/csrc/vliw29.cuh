@@ -378,31 +378,9 @@ constexpr int kSave0 = kMaxRegs;            // each save slot = 12 registers (th
 constexpr int kNumSaves = 5;
 constexpr int kTotalRegs = kMaxRegs + 12 * kNumSaves;
 
-// e(P1, Q1) e(P2, Q2) == 1 with the lines of Q1, Q2 precomputed (c1, c2).  All cooperating threads call it with the same
-// arguments; returns the same verdict to all.  regs: kTotalRegs values shared by the threads.  The sequence of engine steps
-// (Miller loop, final exponentiation) is the generated script (vliw29_programs.cuh: script2 = both pairs live, script1 = one).
-KZG_HD bool coop_pairing_product_is_one(F29* regs, const G1Affine& P1, const LineCoeffs29* c1, const G1Affine& P2, const LineCoeffs29* c2,
-                                        const Lanes& L) {
-    const bool live1 = !P1.inf, live2 = !P2.inf;
-    if (!live1 && !live2) return true;
-    const G1Affine& Pa = live1 ? P1 : P2;       // with a single live pair it takes slot 0
-    const LineCoeffs29* ca = live1 ? c1 : c2;
-    const LineCoeffs29* cb = (live1 && live2) ? c2 : nullptr;
-    for (int i = L.tid; i < 26; i += L.n) {
-        if (i < 10) regs[kRegConst + i] = frob_const(i);
-        else if (i < 14) {
-            const int j = i - 10;
-            if (j < 2) regs[kRegP + j] = f29::from_fp(j == 0 ? Pa.x : Pa.y);
-            else regs[kRegP + j] = cb ? f29::from_fp(j == 2 ? P2.x : P2.y) : f29::f29_zero();
-        } else regs[kRegF + (i - 14)] = i == 14 ? f29::f29_one() : f29::f29_zero();
-    }
-    L.sync();
-#ifdef __CUDA_ARCH__
-    const uint32_t* script = cb ? d_script2 : d_script1;
-#else
-    const uint32_t* script = cb ? h_script2 : h_script1;
-#endif
-    const int n_steps = cb ? kLen_script2 : kLen_script1;
+// The engine steps of a generated script (vliw29_programs.cuh): run a program, copy an Fp12 slot, load the lines of Miller step a
+// (ca: slot-0 pair, cb: slot-1 pair, nullptr = none), invert one register, stamp a profiling tick.
+KZG_HD void run_script(F29* regs, const uint32_t* script, int n_steps, const LineCoeffs29* ca, const LineCoeffs29* cb, const Lanes& L) {
     for (int s = 0; s < n_steps; s++) {
         const uint32_t w = script[s];
         const int op = (int)(w & 0xffu), a = (int)((w >> 8) & 0xfffu), b = (int)(w >> 20);
@@ -418,9 +396,36 @@ KZG_HD bool coop_pairing_product_is_one(F29* regs, const G1Affine& P1, const Lin
         if (L.ticks && L.tid == 0 && (op == kOpCopy || op == kOpLines)) L.ticks[op == kOpCopy ? 6 : 7] += clock64() - s0;   // profiling aid
 #endif
     }
-    // == 1 ?  (each coefficient canonicalised by its own thread; the verdict words land in the padding of the G slot)
+}
+// Miller loop of e(P1, Q1) e(P2, Q2) with the lines of Q1, Q2 precomputed (c1, c2): leaves prod f_{|x|,Q_i}(P_i), conjugated, in
+// the F slot (registers kRegF..+11) and the Frobenius constants in kRegConst.  Pairs whose P is the identity contribute 1.
+KZG_HD void coop_miller(F29* regs, const G1Affine& P1, const LineCoeffs29* c1, const G1Affine& P2, const LineCoeffs29* c2, const Lanes& L) {
+    const bool live1 = !P1.inf, live2 = !P2.inf;
+    const G1Affine& Pa = live1 ? P1 : P2;       // with a single live pair it takes slot 0
+    const LineCoeffs29* ca = live1 ? c1 : c2;
+    const LineCoeffs29* cb = (live1 && live2) ? c2 : nullptr;
+    for (int i = L.tid; i < 26; i += L.n) {
+        if (i < 10) regs[kRegConst + i] = frob_const(i);
+        else if (i < 14) {
+            const int j = i - 10;
+            if (j < 2) regs[kRegP + j] = f29::from_fp(j == 0 ? Pa.x : Pa.y);
+            else regs[kRegP + j] = cb ? f29::from_fp(j == 2 ? P2.x : P2.y) : f29::f29_zero();
+        } else regs[kRegF + (i - 14)] = i == 14 ? f29::f29_one() : f29::f29_zero();
+    }
+    L.sync();
+    if (!live1 && !live2) return;
+#ifdef __CUDA_ARCH__
+    run_script(regs, cb ? d_miller2 : d_miller1, cb ? kLen_miller2 : kLen_miller1, ca, cb, L);
+#else
+    run_script(regs, cb ? h_miller2 : h_miller1, cb ? kLen_miller2 : kLen_miller1, ca, cb, L);
+#endif
+}
+// F slot == 1 ?  (each coefficient canonicalised by its own thread; the verdict words land in the padding of the G slot).
+// gt (nullable): the 12 coefficients as canonical integers (c0.c0.c0, c0.c0.c1, ...: the register order of the F slot).
+KZG_HD bool f_is_one(F29* regs, const Lanes& L, Fp* gt = nullptr) {
     for (int i = L.tid; i < 12; i += L.n) {
         Fp x = canonical_signed(regs[kRegF + i]);
+        if (gt) gt[i] = x;
         bool good = i == 0 ? (x.l[0] == 1u) : (x.l[0] == 0u);
         for (int w = 1; w < 12; w++) good = good && x.l[w] == 0u;
         regs[kRegG + i].l[15] = good ? 1u : 0u;
@@ -432,6 +437,45 @@ KZG_HD bool coop_pairing_product_is_one(F29* regs, const G1Affine& P1, const Lin
     for (int i = L.tid; i < 12; i += L.n) regs[kRegG + i].l[15] = 0;
     L.sync();
     return ok;
+}
+// final exponentiation f^(3(p^12-1)/r) of the F slot (Frobenius constants in kRegConst), then == 1 ?  Same verdict to all threads.
+KZG_HD bool coop_final_exp_is_one(F29* regs, const Lanes& L, Fp* gt = nullptr) {
+#ifdef __CUDA_ARCH__
+    run_script(regs, d_final_exp, kLen_final_exp, nullptr, nullptr, L);
+#else
+    run_script(regs, h_final_exp, kLen_final_exp, nullptr, nullptr, L);
+#endif
+    return f_is_one(regs, L, gt);
+}
+
+// e(P1, Q1) e(P2, Q2) == 1 with the lines of Q1, Q2 precomputed (c1, c2).  All cooperating threads call it with the same
+// arguments; returns the same verdict to all.  regs: kTotalRegs values shared by the threads.  The sequence of engine steps
+// (Miller loop, final exponentiation) is the generated script (vliw29_programs.cuh: script2 = both pairs live, script1 = one).
+KZG_HD bool coop_pairing_product_is_one(F29* regs, const G1Affine& P1, const LineCoeffs29* c1, const G1Affine& P2, const LineCoeffs29* c2,
+                                        const Lanes& L, Fp* gt = nullptr) {
+    const bool live1 = !P1.inf, live2 = !P2.inf;
+    if (!live1 && !live2) {
+        if (gt) for (int i = L.tid; i < 12; i += L.n) { Fp x = Fp::zero(); x.l[0] = i == 0 ? 1u : 0u; gt[i] = x; }
+        return true;
+    }
+    const G1Affine& Pa = live1 ? P1 : P2;       // with a single live pair it takes slot 0
+    const LineCoeffs29* ca = live1 ? c1 : c2;
+    const LineCoeffs29* cb = (live1 && live2) ? c2 : nullptr;
+    for (int i = L.tid; i < 26; i += L.n) {
+        if (i < 10) regs[kRegConst + i] = frob_const(i);
+        else if (i < 14) {
+            const int j = i - 10;
+            if (j < 2) regs[kRegP + j] = f29::from_fp(j == 0 ? Pa.x : Pa.y);
+            else regs[kRegP + j] = cb ? f29::from_fp(j == 2 ? P2.x : P2.y) : f29::f29_zero();
+        } else regs[kRegF + (i - 14)] = i == 14 ? f29::f29_one() : f29::f29_zero();
+    }
+    L.sync();
+#ifdef __CUDA_ARCH__
+    run_script(regs, cb ? d_script2 : d_script1, cb ? kLen_script2 : kLen_script1, ca, cb, L);
+#else
+    run_script(regs, cb ? h_script2 : h_script1, cb ? kLen_script2 : kLen_script1, ca, cb, L);
+#endif
+    return f_is_one(regs, L, gt);
 }
 
 }  // namespace vliw29

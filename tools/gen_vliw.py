@@ -893,12 +893,14 @@ OP_RUN, OP_COPY, OP_LINES, OP_INV, OP_TICK = range(5)
 BLS_X_ABS = 0xd201000000010000
 
 
-def pairing_script(names, max_regs, two_pairs):
+def pairing_script(names, max_regs, two_pairs, part="all"):
     """The pairing check e(P1, Q1) e(P2, Q2) == 1 (one pair when the other G1 argument is the identity) as a straight list of
     engine steps -- run a program, copy an Fp12 slot, load the line coefficients of Miller step k, invert one register, stamp a
     profiling tick -- so that the kernel contains ONE interpreter loop with the two instruction executors inlined once.
     Same sequence as vliw.cuh coop_pairing_product_is_one: Miller loop with precomputed lines, then f^(3(p^12-1)/r) with the
-    hard part (x-1)^2 (x+p)(x^2+p^2-1) + 3 on cyclotomic squarings."""
+    hard part (x-1)^2 (x+p)(x^2+p^2-1) + 3 on cyclotomic squarings.
+    part = "miller": the Miller loop alone, up to and including tick 2 (f left in the F slot, conjugated); part = "fe": the final
+    exponentiation alone, from the F slot (the batch verifier's split tail multiplies per-window Miller values in between)."""
     P = {n: i for i, n in enumerate(names)}
     S = [max_regs + 12 * i for i in range(5)]
     F, G = 0, RG
@@ -941,6 +943,8 @@ def pairing_script(names, max_regs, two_pairs):
     copy(G, S[2]); run("conj_g"); run("f12_mul"); copy(S[4], F)                           # c = b^(x^2+p^2-1)
     copy(F, S[0]); run("f12_sqr"); copy(G, S[0]); run("f12_mul")                          # f^3
     copy(G, S[4]); run("f12_mul"); tick(4)                                                # c f^3
+    cut = s.index((OP_TICK, 2, 0)) + 1
+    s = s[:cut] if part == "miller" else (s[cut:] if part == "fe" else s)
     return [op | a << 8 | b << 20 for op, a, b in s]
 
 
@@ -991,8 +995,9 @@ def emit29(progs, path):
         out.append("%s uint32_t %s_term[%d] = {%s};" % (qual, pre, len(term_tab), ",".join("%du" % t for t in term_tab)))
         out.append("%s Level %s_level[%d] = {%s};" % (qual, pre, len(level_tab), ",".join(row(l) for l in level_tab)))
         out.append("%s Program %s_prog[%d] = {%s};" % (qual, pre, len(prog_tab), ",".join(row(p) for p in prog_tab)))
-        for tag, two in (("script2", True), ("script1", False)):
-            sc = pairing_script(names, max(p[2] for p in prog_tab), two)
+        for tag, two, part in (("script2", True, "all"), ("script1", False, "all"),
+                               ("miller2", True, "miller"), ("miller1", False, "miller"), ("final_exp", True, "fe")):
+            sc = pairing_script(names, max(p[2] for p in prog_tab), two, part)
             if pre == "d":
                 out.append("constexpr int kLen_%s = %d;" % (tag, len(sc)))
             out.append("%s uint32_t %s_%s[%d] = {%s};" % (qual, pre, tag, len(sc), ",".join(str(x) for x in sc)))
