@@ -174,6 +174,33 @@ struct KzgProof {
         if (rc) return detail::to_result(rc, 0).unwrap_err();
         return verdicts;
     }
+    // The cell proofs of a blob transaction: its blobs, one commitment per blob and 128 cell proofs per blob (proof j of blob b at
+    // 128 b + j).  The verdict of verify_cell_kzg_proof_batch on the expanded lists; the cells are computed on the GPU.
+    static Result<bool> verify_blob_cell_kzg_proof_batch(const std::vector<Blob>& blobs, const std::vector<Bytes48>& commitments_bytes,
+                                                         const std::vector<Bytes48>& cell_proofs_bytes, const KzgSettings& kzg_settings) {
+        int ok = 0;
+        int rc = kzgb200_verify_blob_cell_kzg_proof_batch(kzg_settings.ctx(), reinterpret_cast<const uint8_t*>(blobs.data()), blobs.size(),
+                                                          reinterpret_cast<const uint8_t*>(commitments_bytes.data()), commitments_bytes.size(),
+                                                          reinterpret_cast<const uint8_t*>(cell_proofs_bytes.data()), cell_proofs_bytes.size(), &ok);
+        return detail::to_result(rc, ok, "Invalid blobs / commitments / cell proofs length");
+    }
+    // Many transactions in one call, contiguous: transaction g = blobs and commitments [blob_offsets[g], blob_offsets[g + 1]) and the
+    // 128 cell proofs of each of those blobs (k + 1 offsets, the first 0, the last blobs.size()).  One verdict per transaction: 1 = true,
+    // 0 = false, 2 = the transaction alone would give BadArgs.  An error only for the call itself (lengths, offsets, setup).
+    static Result<std::vector<uint8_t>> verify_blob_cell_kzg_proof_batch_many(const std::vector<Blob>& blobs, const std::vector<Bytes48>& commitments_bytes,
+                                                                              const std::vector<Bytes48>& cell_proofs_bytes,
+                                                                              const std::vector<uint64_t>& blob_offsets, const KzgSettings& kzg_settings) {
+        const size_t n = blobs.size();
+        if (commitments_bytes.size() != n || cell_proofs_bytes.size() != CELLS_PER_EXT_BLOB * n || blob_offsets.empty() || blob_offsets.back() != n)
+            return KzgError{KzgError::InvalidBytesLength, "Invalid blobs / commitments / cell proofs / blob offsets length"};
+        std::vector<uint8_t> verdicts(blob_offsets.size() - 1);
+        int rc = kzgb200_verify_blob_cell_kzg_proof_batch_many(kzg_settings.ctx(), reinterpret_cast<const uint8_t*>(blobs.data()),
+                                                               reinterpret_cast<const uint8_t*>(commitments_bytes.data()),
+                                                               reinterpret_cast<const uint8_t*>(cell_proofs_bytes.data()), blob_offsets.data(),
+                                                               verdicts.size(), verdicts.data());
+        if (rc) return detail::to_result(rc, 0).unwrap_err();
+        return verdicts;
+    }
 };
 
 // EIP-4844 publisher calls (need load_commit_setup).  BadArgs for a non-canonical blob element or z, and for a commitment that is not

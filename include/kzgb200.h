@@ -250,6 +250,35 @@ int kzgb200_verify_cell_kzg_proof_batch_many_device(kzgb200_ctx* ctx, const uint
                                                     size_t n_groups, uint8_t* verdicts);
 int kzgb200_last_cell_many_r(kzgb200_ctx* ctx, uint8_t* r_out, size_t n_groups, uint8_t* rho_out32);
 
+/* ---- cell proofs of whole blobs, one verdict per blob transaction (EIP-7594 network form of a blob transaction) ---------------
+ * A blob transaction carries its blobs, their commitments and 128 cell proofs per blob.  An execution-layer node checks it as
+ * verify_cell_kzg_proof_batch on the expanded lists: per blob b in order and j < 128, (commitment b, index j, cell j of
+ * compute_cells(blob b), proof 128 b + j).  These calls run that composition on the GPU: the cells are computed on the device and
+ * never handed to the caller.  Only the cell setup is needed (kzgb200_load_cell_setup), else INVALID_SETUP.
+ * kzgb200_verify_blob_cell_kzg_proof_batch: blobs n_blobs x 131072, commitments n_commitments x 48, cell_proofs n_cell_proofs x 48
+ *   (blob-major: proof j of blob b at 128 b + j), host.  n_commitments != n_blobs or n_cell_proofs != 128 n_blobs -> INVALID_LENGTH;
+ *   n_blobs == 0 -> Ok(true); a non-canonical blob element (compute_cells fails) or a commitment / proof that is not a valid
+ *   compressed point of the G1 subgroup -> BAD_ARGS.  The _device form takes the three arrays in device memory (n_blobs each).
+ * kzgb200_verify_blob_cell_kzg_proof_batch_many: n_groups transactions in one call; blob_offsets[0..n_groups] (host, blobs: offsets[0]
+ *   = 0, never decreasing) split the blobs, commitments (one per blob) and cell proofs (128 per blob) into groups.  verdicts[g] (host)
+ *   = 1 / 0 / 2 for true / false / BadArgs of group g alone, exactly as the single call on that group; an empty group gets 1; a bad
+ *   group never changes another group's verdict.  BAD_ARGS only for a malformed call (a null pointer with work to do, bad offsets,
+ *   128 x blobs or n_groups above 0x7fffffff / 2).  The _device form takes the three data arrays in device memory.
+ *   The single calls are its one-group case.  It is kzgb200_verify_cell_kzg_proof_batch_many on the expanded groups (cell offsets =
+ *   128 x blob offsets): r_g is the spec's r of group g's expanded call, bit for bit (kzgb200_last_cell_many_r reports it; a one-group
+ *   call also sets kzgb200_last_r), and kzgb200_get_phase_ms reports the same slots.  The computed cells (256 KiB per blob) are read
+ *   back to pinned host memory once, for the exact transcripts. */
+int kzgb200_verify_blob_cell_kzg_proof_batch(kzgb200_ctx* ctx, const uint8_t* blobs, size_t n_blobs, const uint8_t* commitments,
+                                             size_t n_commitments, const uint8_t* cell_proofs, size_t n_cell_proofs, int* ok);
+int kzgb200_verify_blob_cell_kzg_proof_batch_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t* d_commitments,
+                                                    const uint8_t* d_cell_proofs, size_t n_blobs, int* ok);
+int kzgb200_verify_blob_cell_kzg_proof_batch_many(kzgb200_ctx* ctx, const uint8_t* blobs, const uint8_t* commitments,
+                                                  const uint8_t* cell_proofs, const uint64_t* blob_offsets, size_t n_groups,
+                                                  uint8_t* verdicts);
+int kzgb200_verify_blob_cell_kzg_proof_batch_many_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t* d_commitments,
+                                                         const uint8_t* d_cell_proofs, const uint64_t* blob_offsets, size_t n_groups,
+                                                         uint8_t* verdicts);
+
 /* ---- EIP-7594 cell proofs and recovery (FK20; consensus-specs Fulu compute_cells_and_kzg_proofs / recover_cells_and_kzg_proofs) --
  * kzgb200_load_cell_proof_setup: the setup's 4096 Lagrange G1 points (host, 4096 x 48 compressed, file order: point j pairs with
  *   omega4096^j; KzgSettings.g1_lagrange_bytes).  n_points must be 4096 and the cell setup must be loaded, else INVALID_SETUP.  Derives

@@ -125,6 +125,10 @@ class Library:
         d.kzgb200_verify_cell_kzg_proof_batch_many.argtypes = [p, p, p, p, p, p, sz, p]
         d.kzgb200_verify_cell_kzg_proof_batch_many_device.argtypes = [p, p, p, p, p, p, sz, p]
         d.kzgb200_last_cell_many_r.argtypes = [p, p, sz, p]
+        d.kzgb200_verify_blob_cell_kzg_proof_batch.argtypes = [p, p, sz, p, sz, p, sz, ip]
+        d.kzgb200_verify_blob_cell_kzg_proof_batch_device.argtypes = [p, p, p, p, sz, ip]
+        d.kzgb200_verify_blob_cell_kzg_proof_batch_many.argtypes = [p, p, p, p, p, sz, p]
+        d.kzgb200_verify_blob_cell_kzg_proof_batch_many_device.argtypes = [p, p, p, p, p, sz, p]
         d.kzgb200_compute_cells.argtypes = [p, C.c_char_p, p]
         d.kzgb200_compute_cells_batch_device.argtypes = [p, p, sz, p]
         d.kzgb200_harness_generate_cells.argtypes = [p, C.c_uint64, sz, C.c_int, C.c_char_p, p, p, p]
@@ -463,6 +467,50 @@ class KzgProof:
         if rc:
             _raise(rc, ctx)
         return [{0: False, 1: True, 2: None}[v] for v in out.raw[:k]]
+
+    @staticmethod
+    def verify_blob_cell_kzg_proof_batch(blobs, commitments_bytes, cell_proofs_bytes, kzg_settings, device=0):
+        """The cell proofs of a blob transaction (EIP-7594 network form): blobs, one commitment per blob and 128 cell proofs per blob
+        (proof j of blob b at 128 b + j).  Returns what verify_cell_kzg_proof_batch returns on the expanded lists (commitment b,
+        index j, cell j of compute_cells(blob b), proof 128 b + j); the cells are computed on the GPU.  Wrong list or byte lengths ->
+        KzgError(InvalidBytesLength); a non-canonical blob element or an invalid point -> KzgError(BadArgs)."""
+        bl, cs, ps = KzgProof._blob_cell_inputs(blobs, commitments_bytes, cell_proofs_bytes)
+        ctx, ok = kzg_settings.cell_context(device), C.c_int(0)
+        n = len(blobs)
+        rc = Library.get().dll.kzgb200_verify_blob_cell_kzg_proof_batch(ctx, _ptr(bl), n, _ptr(cs), n, _ptr(ps), CELLS_PER_EXT_BLOB * n,
+                                                                        C.byref(ok))
+        if rc:
+            _raise(rc, ctx, "Failed to parse blob / G1Affine" if rc == 1 else None)
+        return bool(ok.value)
+
+    @staticmethod
+    def verify_blob_cell_kzg_proof_batch_many(transactions, kzg_settings, device=0):
+        """Many verify_blob_cell_kzg_proof_batch checks in one GPU call (e.g. the blob transactions entering a mempool):
+        transactions is a sequence of (blobs, commitments_bytes, cell_proofs_bytes).  Returns one verdict per transaction:
+        True / False / None, None = that transaction alone would raise BadArgs; a bad transaction does not change another's verdict.
+        Wrong list or byte lengths in any transaction -> KzgError(InvalidBytesLength) for the whole call."""
+        bl, cs, ps, offs = [], [], [], [0]
+        for blobs, commitments_bytes, cell_proofs_bytes in transactions:
+            b, c, p = KzgProof._blob_cell_inputs(blobs, commitments_bytes, cell_proofs_bytes)
+            bl.append(b); cs.append(c); ps.append(p)
+            offs.append(offs[-1] + len(blobs))
+        k = len(offs) - 1
+        ctx = kzg_settings.cell_context(device)
+        out = C.create_string_buffer(max(k, 1))
+        off = (C.c_uint64 * (k + 1))(*offs)
+        rc = Library.get().dll.kzgb200_verify_blob_cell_kzg_proof_batch_many(ctx, _ptr(b"".join(bl)), _ptr(b"".join(cs)), _ptr(b"".join(ps)),
+                                                                             C.cast(off, C.c_void_p), k, out)
+        if rc:
+            _raise(rc, ctx)
+        return [{0: False, 1: True, 2: None}[v] for v in out.raw[:k]]
+
+    @staticmethod
+    def _blob_cell_inputs(blobs, commitments_bytes, cell_proofs_bytes):
+        n = len(blobs)
+        if len(commitments_bytes) != n or len(cell_proofs_bytes) != CELLS_PER_EXT_BLOB * n:
+            raise KzgError("InvalidBytesLength", "Invalid blobs / commitments / cell proofs length")
+        return (b"".join(_b(x, BYTES_PER_BLOB, "blob") for x in blobs), b"".join(_b(x, 48, "commitment") for x in commitments_bytes),
+                b"".join(_b(x, 48, "proof") for x in cell_proofs_bytes))
 
 
 def compute_cells(blob, kzg_settings, device=0):

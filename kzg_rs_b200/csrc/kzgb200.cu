@@ -1539,6 +1539,96 @@ extern "C" int kzgb200_verify_cell_kzg_proof_batch_many_device(kzgb200_ctx* ctx,
     return cell_verify(ctx, d_commitments, d_cell_indices, d_cells, d_proofs, group_offsets, n_groups, verdicts, true);
 }
 
+// ---- verify_blob_cell_kzg_proof_batch[_many]: the cell proofs of whole blobs (EIP-7594 blob transactions), one verdict per group ---
+// Group g = blobs [boff[g], boff[g + 1]) with their commitments and 128 cell proofs each.  Its verdict and r_g are those of
+// verify_cell_kzg_proof_batch on the expanded call: per blob b in order and j < 128, (C_b, j, cell j of compute_cells(blob_b),
+// proof 128 b + j).  The cells are computed on the device straight into d_cells, whose blob-major layout is already that per-cell
+// order, and read back once to pinned memory: the exact transcripts are host chains over every cell byte.  The expanded commitments
+// and indices are built on the host; then the cell pipeline (cell_verify_groups) runs unchanged with cell offsets = 128 x blob offsets.
+static int blob_cell_verify(kzgb200_ctx* ctx, const uint8_t* blobs, const uint8_t* cm, const uint8_t* p, const uint64_t* boff, size_t k,
+                            uint8_t* verdicts, bool device_inputs) {
+    constexpr uint64_t kMaxBlobs = 0x7fffffff / 2 / kCellsPerExtBlob;       // 128 x blobs within the cell path's limit
+    if (!ctx || (k && (!boff || !verdicts)) || k > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
+    size_t nb = 0;
+    if (k) {
+        if (boff[0] != 0) return KZGB200_BAD_ARGS;
+        for (size_t g = 0; g < k; g++) if (boff[g + 1] < boff[g] || boff[g + 1] > kMaxBlobs) return KZGB200_BAD_ARGS;
+        nb = boff[k];
+    }
+    if (nb && (!blobs || !cm || !p)) return KZGB200_BAD_ARGS;
+    if (!ctx->cells) return KZGB200_INVALID_SETUP;
+    std::vector<uint64_t> off(k + 1, 0);
+    for (size_t g = 1; g <= k; g++) off[g] = boff[g] * kCellsPerExtBlob;
+    if (nb == 0) return cell_verify(ctx, nullptr, nullptr, nullptr, nullptr, off.data(), k, verdicts, false);   // every group empty
+    const size_t n = nb * kCellsPerExtBlob;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    CellCtx* c = ctx->cells;
+    int rc = cell_capacity(ctx, n, true, true);                       // d_cells for the computed cells, the pinned h_* for the transcripts
+    if (!rc && !device_inputs) rc = ensure_capacity(ctx, nb, true);   // the blob staging buffer
+    if (rc) return rc;
+    const uint8_t *d_blobs = blobs, *d_p = p, *hc = cm, *hp = p;
+    CK(cudaStreamWaitEvent(ctx->stream, ctx->ev_parse, 0));
+    if (device_inputs) {                              // as the cell _device form: commitments and proofs back to pinned memory once
+        CK(cudaStreamWaitEvent(ctx->s_d2h, ctx->ev_parse, 0));
+        CK(cudaMemcpyAsync(ctx->h_c, cm, nb * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
+        CK(cudaMemcpyAsync(c->h_p, p, n * 48, cudaMemcpyDeviceToHost, ctx->s_d2h));
+        hc = ctx->h_c; hp = c->h_p;
+    } else {
+        CK(cudaMemcpyAsync(ctx->d_blobs, blobs, nb * kBytesPerBlob, cudaMemcpyHostToDevice, ctx->stream));
+        CK(cudaMemcpyAsync(c->d_p, p, n * 48, cudaMemcpyHostToDevice, ctx->stream));
+        d_blobs = ctx->d_blobs; d_p = c->d_p;
+    }
+    // No canonicity check here: compute_cells_kernel copies the raw blob bytes into cells 0..63, where cell_check_kernel flags any
+    // element >= q and makes the group BadArgs -- the spec's compute_cells failing.  (The flags this kernel sets in d_status are cleared
+    // by cell_verify_groups before its parse.)
+    compute_cells_kernel<<<(unsigned)nb, kCellNttThreads, kCellNttSmemBytes, ctx->stream>>>(d_blobs, (int)nb, c->tables, c->d_cells, ctx->d_status);
+    CK(cudaGetLastError());
+    CK(cudaMemcpyAsync(c->h_cells, c->d_cells, n * kBytesPerCell, cudaMemcpyDeviceToHost, ctx->stream));
+    if (device_inputs) CK(cudaStreamSynchronize(ctx->s_d2h));
+    for (size_t b = 0; b < nb; b++)
+        for (int j = 0; j < kCellsPerExtBlob; j++) {
+            const size_t e = b * kCellsPerExtBlob + j;
+            memcpy(c->h_c + 48 * e, hc + 48 * b, 48);
+            c->h_idx[e] = (uint64_t)j;
+        }
+    CK(cudaStreamSynchronize(ctx->stream));
+    return cell_verify_groups(ctx, c->h_c, c->h_idx, c->h_cells, hp, c->d_cells, d_p, off.data(), k, verdicts, false);
+}
+// one group: its verdict 2 is the call's BAD_ARGS
+static int blob_cell_verify_one(kzgb200_ctx* ctx, const uint8_t* blobs, const uint8_t* cm, const uint8_t* p, size_t n_blobs, int* ok,
+                                bool device_inputs) {
+    if (!ok) return KZGB200_BAD_ARGS;
+    const uint64_t boff[2] = {0, n_blobs};
+    uint8_t v = kFalse;
+    int rc = blob_cell_verify(ctx, blobs, cm, p, boff, 1, &v, device_inputs);
+    if (rc) return rc;
+    if (v == kBadArgs) return KZGB200_BAD_ARGS;
+    *ok = v == kTrue;
+    return KZGB200_OK;
+}
+
+extern "C" int kzgb200_verify_blob_cell_kzg_proof_batch(kzgb200_ctx* ctx, const uint8_t* blobs, size_t n_blobs, const uint8_t* commitments,
+                                                        size_t n_commitments, const uint8_t* cell_proofs, size_t n_cell_proofs, int* ok) {
+    if (!ctx || !ok) return KZGB200_BAD_ARGS;
+    if (n_commitments != n_blobs || n_cell_proofs % kCellsPerExtBlob || n_cell_proofs / kCellsPerExtBlob != n_blobs) return KZGB200_INVALID_LENGTH;
+    return blob_cell_verify_one(ctx, blobs, commitments, cell_proofs, n_blobs, ok, false);
+}
+extern "C" int kzgb200_verify_blob_cell_kzg_proof_batch_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t* d_commitments,
+                                                               const uint8_t* d_cell_proofs, size_t n_blobs, int* ok) {
+    return blob_cell_verify_one(ctx, d_blobs, d_commitments, d_cell_proofs, n_blobs, ok, true);
+}
+extern "C" int kzgb200_verify_blob_cell_kzg_proof_batch_many(kzgb200_ctx* ctx, const uint8_t* blobs, const uint8_t* commitments,
+                                                             const uint8_t* cell_proofs, const uint64_t* blob_offsets, size_t n_groups,
+                                                             uint8_t* verdicts) {
+    return blob_cell_verify(ctx, blobs, commitments, cell_proofs, blob_offsets, n_groups, verdicts, false);
+}
+extern "C" int kzgb200_verify_blob_cell_kzg_proof_batch_many_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, const uint8_t* d_commitments,
+                                                                    const uint8_t* d_cell_proofs, const uint64_t* blob_offsets, size_t n_groups,
+                                                                    uint8_t* verdicts) {
+    return blob_cell_verify(ctx, d_blobs, d_commitments, d_cell_proofs, blob_offsets, n_groups, verdicts, true);
+}
+
 // test hook: r_g of every group of the last cell verification call (zeros for empty groups) and rho, canonical big-endian
 extern "C" int kzgb200_last_cell_many_r(kzgb200_ctx* ctx, uint8_t* r_out, size_t n_groups, uint8_t* rho_out32) {
     if (!ctx || !rho_out32 || (n_groups && !r_out)) return KZGB200_BAD_ARGS;
