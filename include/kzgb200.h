@@ -297,6 +297,16 @@ int kzgb200_verify_blob_cell_kzg_proof_batch_many_device(kzgb200_ctx* ctx, const
  *   twice and every element canonical.  Inconsistent cells are not detected (as in the spec): the result is the spec's bytes.
  * kzgb200_recover_cells_and_kzg_proofs_batch_device: n_blobs blobs that share one index set (host cell_indices, n_cells); d_cells =
  *   n_blobs x n_cells x 2048 (device, blob-major, each blob's cells in index-set order); outputs as the batch compute call.
+ * kzgb200_recover_cells_and_kzg_proofs_many[_device]: n_blobs blobs in one call, each recovered from its own cells and index set.
+ *   cell_offsets (host, n_blobs + 1 entries, [0] = 0, never decreasing): blob b owns cells [off[b], off[b + 1]), one u64 index per cell
+ *   in cell_indices (host in both forms) and 2048 bytes per cell in cells (host; _device: device), any order of indices within a blob.
+ *   Outputs are blob-major, n_blobs x 128 x 2048 cells and n_blobs x 128 x 48 proofs (host; _device: device).  status (host, one
+ *   byte per blob) = the return code kzgb200_recover_cells_and_kzg_proofs gives for that blob alone: 0 = its outputs are that call's
+ *   bytes; 1 (BAD_ARGS) = fewer than 64 or more than 128 cells, an index >= 128, a repeated index or a non-canonical element, its
+ *   output slot unspecified.  A bad blob changes no other blob's output, and no blob's cells are read outside its own range.  The call
+ *   returns BAD_ARGS only when malformed (a null pointer with blobs to recover, bad offsets, n_blobs or off[n_blobs] above
+ *   0x7fffffff / 2), INVALID_SETUP before the proof setup, and OK for n_blobs == 0 (cell_offsets then unread).  Blobs that share one
+ *   index set cost about what the _batch_device call costs for them.
  * With kzgb200_set_profiling on, kzgb200_get_phase_ms reports for these calls {coefficients (with compute_cells), fixed-base products
  * (with the scalar DFTs), G1 transforms (with compression), recovery transforms, 0, 0, 0, 0}, first start to last end. */
 int kzgb200_load_cell_proof_setup(kzgb200_ctx* ctx, const uint8_t* g1_lagrange48, size_t n_points);
@@ -307,6 +317,11 @@ int kzgb200_recover_cells_and_kzg_proofs(kzgb200_ctx* ctx, const uint64_t* cell_
                                          uint8_t* cells_out, uint8_t* proofs_out);
 int kzgb200_recover_cells_and_kzg_proofs_batch_device(kzgb200_ctx* ctx, const uint64_t* cell_indices, size_t n_cells, const uint8_t* d_cells,
                                                       size_t n_blobs, uint8_t* d_cells_out, uint8_t* d_proofs_out);
+int kzgb200_recover_cells_and_kzg_proofs_many(kzgb200_ctx* ctx, const uint64_t* cell_indices, const uint8_t* cells, const uint64_t* cell_offsets,
+                                              size_t n_blobs, uint8_t* cells_out, uint8_t* proofs_out, uint8_t* status);
+int kzgb200_recover_cells_and_kzg_proofs_many_device(kzgb200_ctx* ctx, const uint64_t* cell_indices, const uint8_t* d_cells,
+                                                     const uint64_t* cell_offsets, size_t n_blobs, uint8_t* d_cells_out, uint8_t* d_proofs_out,
+                                                     uint8_t* status);
 
 /* per-phase device timing of batch calls (CUDA event pairs on the stream each phase runs on).  out8 = milliseconds of
  * {G1 decompression, challenge, evaluate, transcript r (exposed part: last chunk copy + host hash + upload), lincomb terms, reduce,

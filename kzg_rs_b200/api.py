@@ -138,6 +138,8 @@ class Library:
         d.kzgb200_compute_cells_and_kzg_proofs_batch_device.argtypes = [p, p, sz, p, p]
         d.kzgb200_recover_cells_and_kzg_proofs.argtypes = [p, p, p, sz, p, p]
         d.kzgb200_recover_cells_and_kzg_proofs_batch_device.argtypes = [p, p, sz, p, sz, p, p]
+        d.kzgb200_recover_cells_and_kzg_proofs_many.argtypes = [p, p, p, p, sz, p, p, p]
+        d.kzgb200_recover_cells_and_kzg_proofs_many_device.argtypes = [p, p, p, p, sz, p, p, p]
 
 
 def _raise(rc, ctx=None, msg=None):
@@ -561,6 +563,40 @@ def recover_cells_and_kzg_proofs(cell_indices, cells, kzg_settings, device=0):
     if rc:
         _raise(rc, ctx, "Invalid cell indices / cells" if rc == 1 else None)
     return _cells_and_proofs(out_cells.raw, out_proofs.raw)
+
+
+def recover_cells_and_kzg_proofs_many(blobs, kzg_settings, device=0):
+    """Many recover_cells_and_kzg_proofs in one GPU call, each blob from its own cells and index set (e.g. a block whose blobs
+    hold different columns): blobs is a sequence of (cell_indices, cells).  Returns one (cells, proofs) pair per blob, 128 of each,
+    or None where recover_cells_and_kzg_proofs would raise BadArgs; a bad blob does not change another's result.  Mismatched
+    lengths or wrong byte lengths in any blob -> KzgError(InvalidBytesLength) for the whole call, before any GPU work."""
+    idx, ce, offs, out_of_range = [], [], [0], set()
+    for b, (cell_indices, cells) in enumerate(blobs):
+        if len(cells) != len(cell_indices):
+            raise KzgError("InvalidBytesLength", "Invalid cells / cell indices length")
+        raw = b"".join(_b(x, BYTES_PER_CELL, "cell") for x in cells)
+        ids = [int(i) for i in cell_indices]
+        if any(not 0 <= i < 1 << 64 for i in ids):
+            out_of_range.add(b)            # no cells: the library reports the blob as bad
+            ids, raw = [], b""
+        idx.extend(ids)
+        ce.append(raw)
+        offs.append(offs[-1] + len(ids))
+    k = len(offs) - 1
+    ctx = kzg_settings.cell_proof_context(device)
+    ia = (C.c_uint64 * max(len(idx), 1))(*idx)
+    off = (C.c_uint64 * (k + 1))(*offs)
+    out_cells = C.create_string_buffer(BYTES_PER_CELL * CELLS_PER_EXT_BLOB * max(k, 1))
+    out_proofs = C.create_string_buffer(BYTES_PER_PROOF * CELLS_PER_EXT_BLOB * max(k, 1))
+    status = C.create_string_buffer(max(k, 1))
+    rc = Library.get().dll.kzgb200_recover_cells_and_kzg_proofs_many(ctx, C.cast(ia, C.c_void_p), _ptr(b"".join(ce)), C.cast(off, C.c_void_p), k,
+                                                                     out_cells, out_proofs, status)
+    if rc:
+        _raise(rc, ctx)
+    rc_cells, rc_proofs, st = out_cells.raw, out_proofs.raw, status.raw
+    cb, pb = BYTES_PER_CELL * CELLS_PER_EXT_BLOB, BYTES_PER_PROOF * CELLS_PER_EXT_BLOB
+    return [None if st[b] or b in out_of_range else _cells_and_proofs(rc_cells[cb * b:cb * (b + 1)], rc_proofs[pb * b:pb * (b + 1)])
+            for b in range(k)]
 
 
 def blob_to_kzg_commitment(blob, kzg_settings, device=0):

@@ -148,6 +148,15 @@ struct ProofTables {
     Fr pow7_inv[kFieldElementsPerBlob];     // 7^-i / 8192
     Fr s7_64;                               // 7^64
 };
+// One index set of the recovery (kzgb200.cu recover_plan): pos[k] = the input position of cell index k within the blob's cells
+// (-1: missing), the missing indices, and `first`, the blob's first cell relative to the cell pointer of its pass.  A plan with no
+// present and no missing cell reads nothing (the slot of a blob that failed the argument checks).
+struct RecoverPlan {
+    int8_t pos[kCellsPerExtBlob];
+    uint8_t missing[kCellsPerExtBlob];
+    int32_t n_missing;
+    uint32_t first;
+};
 // ---- kernels (k_*.cu) ----------------------------------------------------------------------------------------
 __global__ void setup_tables_kernel(DeviceTables* T, const uint8_t* g2_points);
 __global__ void setup_lines29_kernel(DeviceTables* T);
@@ -251,12 +260,13 @@ __global__ void fk20_table_kernel(const G1Affine* __restrict__ W, G1Affine* __re
 __global__ void fk20_scalars_kernel(const Fr* __restrict__ coeffs, const CellTables* __restrict__ T, Fr* __restrict__ U);
 __global__ void fk20_products_kernel(const Fr* __restrict__ U, const G1Affine* __restrict__ tab, G1* __restrict__ V);
 __global__ void fk20_proofs_kernel(const G1* __restrict__ V, const CellTables* __restrict__ T, uint8_t* __restrict__ proofs);
-__global__ void recover_z_kernel(const uint32_t* __restrict__ missing, int n_missing, const CellTables* __restrict__ T, const ProofTables* __restrict__ P,
+// recovery: blob i of a pass uses plan i * plan_stride (0: one index set shared by the pass) and its Z row
+__global__ void recover_z_kernel(const RecoverPlan* __restrict__ plans, const CellTables* __restrict__ T, const ProofTables* __restrict__ P,
                                  Fr* __restrict__ zvals);
-__global__ void recover_load_kernel(const uint8_t* __restrict__ cells, int n_cells, const int* __restrict__ pos, const Fr* __restrict__ zvals, int nb,
-                                    Fr* __restrict__ A, uint32_t* __restrict__ status);
+__global__ void recover_load_kernel(const uint8_t* __restrict__ cells, int cell_stride, const RecoverPlan* __restrict__ plans, int plan_stride,
+                                    const Fr* __restrict__ zvals, int nb, Fr* __restrict__ A, uint32_t* __restrict__ status);
 __global__ void recover_ntt_inv_kernel(Fr* __restrict__ A, const CellTables* __restrict__ T);
-__global__ void recover_ntt_div_kernel(Fr* __restrict__ A, const CellTables* __restrict__ T, const Fr* __restrict__ zvals);
+__global__ void recover_ntt_div_kernel(Fr* __restrict__ A, const CellTables* __restrict__ T, const Fr* __restrict__ zvals, int plan_stride);
 __global__ void recover_mid_kernel(Fr* __restrict__ A, const ProofTables* __restrict__ P, int nb);
 __global__ void recover_final_kernel(const Fr* __restrict__ A, const ProofTables* __restrict__ P, int nb, Fr* __restrict__ coeffs);
 __global__ void recover_blob_kernel(const Fr* __restrict__ coeffs, const CellTables* __restrict__ T, uint8_t* __restrict__ blobs);

@@ -211,29 +211,36 @@ __global__ void __launch_bounds__(64) fk20_proofs_kernel(const G1* __restrict__ 
 }
 
 // ---- recover_cells_and_kzg_proofs ------------------------------------------------------------------------------------
-// zvals[k] = z(s_k) (Z on cell k of the domain), zvals[128 + k] = 1 / z(7^64 s_k) (1 / Z on cell k of the coset transform's
-// bit-reversed output); missing = the absent cell indices
-__global__ void __launch_bounds__(256) recover_z_kernel(const uint32_t* __restrict__ missing, int n_missing, const CellTables* __restrict__ T,
+// one CTA per plan: zvals[256 j + k] = z_j(s_k) (Z of plan j on cell k of the domain), zvals[256 j + 128 + k] = 1 / z_j(7^64 s_k)
+// (1 / Z on cell k of the coset transform's bit-reversed output), z_j = prod over plan j's missing cell indices
+__global__ void __launch_bounds__(256) recover_z_kernel(const RecoverPlan* __restrict__ plans, const CellTables* __restrict__ T,
                                                         const ProofTables* __restrict__ P, Fr* __restrict__ zvals) {
+    const RecoverPlan* pl = plans + blockIdx.x;
     const int t = threadIdx.x;
     const int k = t & (kCellsPerExtBlob - 1);
     const Fr x = t < kCellsPerExtBlob ? T->shift64[k] : T->shift64[k].mul_inl(P->s7_64);
     Fr z = Fr::one();
-    for (int i = 0; i < n_missing; i++) z = z.mul_inl(x.sub_inl(T->shift64[missing[i]]));
-    zvals[t] = t < kCellsPerExtBlob ? z : fr_inv(z);
+    const int n_missing = pl->n_missing;
+    for (int i = 0; i < n_missing; i++) z = z.mul_inl(x.sub_inl(T->shift64[pl->missing[i]]));
+    zvals[(size_t)blockIdx.x * 2 * kCellsPerExtBlob + t] = t < kCellsPerExtBlob ? z : fr_inv(z);
 }
 // E times Z in bit-reversed order (the spec's extended_evaluation_rbo, which is what the inverse DIT transform reads): element p of
-// blob `blob` comes from input cell pos[p / 64] (-1: missing, zero); non-canonical elements flag the blob
-__global__ void __launch_bounds__(256) recover_load_kernel(const uint8_t* __restrict__ cells, int n_cells, const int* __restrict__ pos,
-                                                           const Fr* __restrict__ zvals, int nb, Fr* __restrict__ A, uint32_t* __restrict__ status) {
+// blob `blob` comes from input cell first + blob * cell_stride + pos[p / 64] of its plan (pos -1: missing, zero); non-canonical
+// elements flag the blob.  One shared index set: plan_stride 0, cell_stride = cells per blob; a plan per blob: 1 and 0.
+__global__ void __launch_bounds__(256) recover_load_kernel(const uint8_t* __restrict__ cells, int cell_stride, const RecoverPlan* __restrict__ plans,
+                                                           int plan_stride, const Fr* __restrict__ zvals, int nb, Fr* __restrict__ A,
+                                                           uint32_t* __restrict__ status) {
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= (size_t)nb * kExtElements) return;
-    const int blob = (int)(i / kExtElements), p = (int)(i % kExtElements), k = p / kFieldElementsPerCell, src = pos[k];
+    const int blob = (int)(i / kExtElements), p = (int)(i % kExtElements), k = p / kFieldElementsPerCell;
+    const size_t plan = (size_t)blob * plan_stride;
+    const int src = plans[plan].pos[k];
     Fr v = Fr::zero();
     if (src >= 0) {
-        const Fr raw = load_fe_be(reinterpret_cast<const uint4*>(cells + ((size_t)blob * n_cells + src) * kBytesPerCell) + 2 * (p % kFieldElementsPerCell));
+        const size_t cell = plans[plan].first + (size_t)blob * cell_stride + src;
+        const Fr raw = load_fe_be(reinterpret_cast<const uint4*>(cells + cell * kBytesPerCell) + 2 * (p % kFieldElementsPerCell));
         if (raw.geq_modulus()) atomicOr(&status[blob], kErrBlob);
-        v = Fr::from_raw(raw).mul_inl(zvals[k]);
+        v = Fr::from_raw(raw).mul_inl(zvals[plan * 2 * kCellsPerExtBlob + k]);
     }
     A[i] = v;
 }
@@ -277,14 +284,17 @@ __global__ void __launch_bounds__(kCellNttThreads) recover_ntt_inv_kernel(Fr* __
     for (int i = threadIdx.x; i < kFieldElementsPerBlob; i += kCellNttThreads) g[i] = a[i];
 }
 // coset transform, second part (the 4096-point levels), division by Z on the coset, and the inverse transform's 4096-point levels
-__global__ void __launch_bounds__(kCellNttThreads) recover_ntt_div_kernel(Fr* __restrict__ A, const CellTables* __restrict__ T, const Fr* __restrict__ zvals) {
+// (the blob's Z row: blockIdx.y * plan_stride, as in recover_load_kernel)
+__global__ void __launch_bounds__(kCellNttThreads) recover_ntt_div_kernel(Fr* __restrict__ A, const CellTables* __restrict__ T, const Fr* __restrict__ zvals,
+                                                                          int plan_stride) {
     extern __shared__ __align__(16) unsigned char dyn_smem[];
     Fr* a = reinterpret_cast<Fr*>(dyn_smem);
     Fr* g = ntt_half_load(A, a);
     ntt4096_dif_fwd(a, T);
     const int base = blockIdx.x * kFieldElementsPerBlob;
+    const Fr* zinv = zvals + ((size_t)blockIdx.y * plan_stride * 2 + 1) * kCellsPerExtBlob;
     for (int i = threadIdx.x; i < kFieldElementsPerBlob; i += kCellNttThreads)
-        a[i] = a[i].mul_inl(zvals[kCellsPerExtBlob + (base + i) / kFieldElementsPerCell]);
+        a[i] = a[i].mul_inl(zinv[(base + i) / kFieldElementsPerCell]);
     __syncthreads();
     ntt4096_dit_inv(a, T);
     for (int i = threadIdx.x; i < kFieldElementsPerBlob; i += kCellNttThreads) g[i] = a[i];

@@ -1111,10 +1111,12 @@ extern "C" void kzgb200_free_pinned(void* p) { if (p) cudaFreeHost(p); }
 
 // ---- EIP-7594 cells (k_cells.cu; consensus-specs Fulu polynomial-commitments-sampling.md) ---------------------------------
 static void proof_destroy(CellCtx* c) {
-    void* d[] = {c->ptables, c->d_mono, c->d_fk_tab, c->d_pcoef, c->d_fkU, c->d_A, c->d_V, c->d_rblobs, c->d_rin, c->d_pout, c->d_pos, c->d_missing, c->d_z};
+    void* d[] = {c->ptables, c->d_mono, c->d_fk_tab, c->d_pcoef, c->d_fkU, c->d_A, c->d_V, c->d_rblobs, c->d_rin, c->d_pout, c->d_plans, c->d_z,
+                 c->d_mstage, c->d_mcells, c->d_mproofs};
     for (void* p : d) if (p) cudaFree(p);
     c->ptables = nullptr; c->d_mono = c->d_fk_tab = nullptr; c->d_pcoef = c->d_fkU = c->d_A = c->d_z = nullptr; c->d_V = nullptr;
-    c->d_rblobs = c->d_rin = c->d_pout = nullptr; c->d_pos = nullptr; c->d_missing = nullptr; c->proof_cap = 0;
+    c->d_rblobs = c->d_rin = c->d_pout = nullptr; c->d_plans = nullptr; c->proof_cap = 0;
+    c->d_mstage = c->d_mcells = c->d_mproofs = nullptr; c->mstage_cells = c->mout_cap = 0;
 }
 static void cell_destroy(kzgb200_ctx* ctx) {
     CellCtx* c = ctx->cells;
@@ -1750,8 +1752,6 @@ extern "C" int kzgb200_load_cell_proof_setup(kzgb200_ctx* ctx, const uint8_t* g1
         CK(cudaFuncSetAttribute(recover_ntt_div_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCellNttSmemBytes));
         CK(cudaFuncSetAttribute(recover_blob_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kCellNttSmemBytes));
         CK(cudaMalloc(&c->d_rin, (size_t)kCellsPerExtBlob * kBytesPerCell)); CK(cudaMalloc(&c->d_pout, (size_t)kCellsPerExtBlob * 48));
-        CK(cudaMalloc(&c->d_pos, kCellsPerExtBlob * sizeof(int))); CK(cudaMalloc(&c->d_missing, kCellsPerExtBlob * sizeof(uint32_t)));
-        CK(cudaMalloc(&c->d_z, 2 * kCellsPerExtBlob * sizeof(Fr)));
         CK(cudaStreamSynchronize(ctx->stream));
         return KZGB200_OK;
     }();
@@ -1786,6 +1786,7 @@ static int proof_workspace(kzgb200_ctx* ctx, size_t n) {
     c->proof_cap = 0;
     CK(regrow(c->d_pcoef, nb * kFieldElementsPerBlob)); CK(regrow(c->d_fkU, nb * kFk20Bases)); CK(regrow(c->d_A, nb * kExtElements));
     CK(regrow(c->d_V, nb * kCellsPerExtBlob)); CK(regrow(c->d_rblobs, nb * kBytesPerBlob));
+    CK(regrow(c->d_plans, nb)); CK(regrow(c->d_z, nb * 2 * kCellsPerExtBlob));
     c->proof_cap = nb;
     return KZGB200_OK;
 }
@@ -1829,6 +1830,15 @@ static int proof_result(kzgb200_ctx* ctx, size_t n) {
     collect_phase_times(ctx);
     return ctx->h_result[0] ? KZGB200_BAD_ARGS : KZGB200_OK;
 }
+// per-blob form of proof_result: status[b] = BAD_ARGS if blob b had a non-canonical element or host_bad[b], else OK
+static int proof_result_each(kzgb200_ctx* ctx, size_t n, const uint8_t* host_bad, uint8_t* status) {
+    std::vector<uint32_t> flags(n);
+    CK(cudaMemcpyAsync(flags.data(), ctx->d_status, n * sizeof(uint32_t), cudaMemcpyDeviceToHost, ctx->stream));
+    CK(cudaStreamSynchronize(ctx->stream));
+    collect_phase_times(ctx);
+    for (size_t b = 0; b < n; b++) status[b] = (host_bad[b] || flags[b]) ? KZGB200_BAD_ARGS : KZGB200_OK;
+    return KZGB200_OK;
+}
 static bool proof_ready(kzgb200_ctx* ctx) { return ctx->cells && ctx->cells->d_fk_tab; }
 
 extern "C" int kzgb200_compute_cells_and_kzg_proofs(kzgb200_ctx* ctx, const uint8_t* blob, uint8_t* cells_out, uint8_t* proofs_out) {
@@ -1860,53 +1870,66 @@ extern "C" int kzgb200_compute_cells_and_kzg_proofs_batch_device(kzgb200_ctx* ct
     return rc ? rc : proof_result(ctx, n);
 }
 
-// The spec's argument checks on one index set: 64 <= n_cells <= 128, every index < 128, no index twice.  pos[k] = the input
-// position of cell index k or -1; missing = the absent indices.
-static int recover_plan(const uint64_t* idx, size_t n_cells, int* pos, uint32_t* missing, int* n_missing) {
+// The spec's argument checks on one index set: 64 <= n_cells <= 128, every index < 128, no index twice.  plan: pos[k] = the input
+// position of cell index k or -1, missing = the absent indices, first = 0.  On failure the plan is the empty plan (reads nothing).
+static int recover_plan(const uint64_t* idx, size_t n_cells, RecoverPlan* plan) {
+    memset(plan->pos, 0xff, sizeof(plan->pos));
+    plan->n_missing = 0;
+    plan->first = 0;
     if (!idx || n_cells < (size_t)kCellsPerExtBlob / 2 || n_cells > (size_t)kCellsPerExtBlob) return KZGB200_BAD_ARGS;
-    for (int k = 0; k < kCellsPerExtBlob; k++) pos[k] = -1;
     for (size_t j = 0; j < n_cells; j++) {
-        if (idx[j] >= (uint64_t)kCellsPerExtBlob || pos[idx[j]] >= 0) return KZGB200_BAD_ARGS;
-        pos[idx[j]] = (int)j;
+        if (idx[j] >= (uint64_t)kCellsPerExtBlob || plan->pos[idx[j]] >= 0) {
+            memset(plan->pos, 0xff, sizeof(plan->pos));
+            return KZGB200_BAD_ARGS;
+        }
+        plan->pos[idx[j]] = (int8_t)j;
     }
-    *n_missing = 0;
-    for (int k = 0; k < kCellsPerExtBlob; k++) if (pos[k] < 0) missing[(*n_missing)++] = (uint32_t)k;
+    for (int k = 0; k < kCellsPerExtBlob; k++) if (plan->pos[k] < 0) plan->missing[plan->n_missing++] = (uint8_t)k;
     return KZGB200_OK;
 }
-// recovery of nb blobs that share one index set: d_in = nb x n_cells cells (blob-major), outputs as compute_cells_and_kzg_proofs.
+// n plans (n <= proof_cap) to the workspace, and their Z rows
+static int recover_upload(kzgb200_ctx* ctx, const RecoverPlan* plans, size_t n) {
+    CellCtx* c = ctx->cells;
+    CK(cudaMemcpyAsync(c->d_plans, plans, n * sizeof(RecoverPlan), cudaMemcpyHostToDevice, ctx->stream));
+    recover_z_kernel<<<(unsigned)n, 2 * kCellsPerExtBlob, 0, ctx->stream>>>(c->d_plans, c->tables, c->ptables, c->d_z);
+    return KZGB200_OK;
+}
+// one pass of cnt <= kProofChunk blobs through the workspace: blob i uses uploaded plan i * plan_stride and reads its cells from
+// d_in + (first + i * cell_stride + pos) x 2048; outputs as compute_cells_and_kzg_proofs; status: cnt flags.
 // Profiling slot 3 = the recovery transforms (E Z, the three 8192-point transforms, the 4096-point transform back to the blob).
-static int recover_launch(kzgb200_ctx* ctx, const int* pos, const uint32_t* missing, int n_missing, const uint8_t* d_in, size_t n_cells, size_t nb,
-                          uint8_t* d_cells_out, uint8_t* d_proofs_out) {
+static int recover_pass(kzgb200_ctx* ctx, int plan_stride, const uint8_t* d_in, size_t cell_stride, int cnt, uint8_t* d_cells_out,
+                        uint8_t* d_proofs_out, uint32_t* status) {
     CellCtx* c = ctx->cells;
     cudaStream_t st = ctx->stream;
-    CK(cudaMemcpyAsync(c->d_pos, pos, kCellsPerExtBlob * sizeof(int), cudaMemcpyHostToDevice, st));
-    if (n_missing) CK(cudaMemcpyAsync(c->d_missing, missing, n_missing * sizeof(uint32_t), cudaMemcpyHostToDevice, st));
-    recover_z_kernel<<<1, 2 * kCellsPerExtBlob, 0, st>>>(c->d_missing, n_missing, c->tables, c->ptables, c->d_z);
-    for (size_t lo = 0; lo < nb; lo += kProofChunk) {
+    phase_begin(ctx, 3, st);
+    recover_load_kernel<<<(unsigned)((size_t)cnt * kExtElements / 256), 256, 0, st>>>(d_in, (int)cell_stride, c->d_plans, plan_stride, c->d_z, cnt,
+                                                                                     c->d_A, status);
+    recover_ntt_inv_kernel<<<dim3(2, cnt), kCellNttThreads, kCellNttSmemBytes, st>>>(c->d_A, c->tables);
+    recover_mid_kernel<<<(unsigned)((size_t)cnt * kFieldElementsPerBlob / 256), 256, 0, st>>>(c->d_A, c->ptables, cnt);
+    recover_ntt_div_kernel<<<dim3(2, cnt), kCellNttThreads, kCellNttSmemBytes, st>>>(c->d_A, c->tables, c->d_z, plan_stride);
+    recover_final_kernel<<<(unsigned)((size_t)cnt * kFieldElementsPerBlob / 256), 256, 0, st>>>(c->d_A, c->ptables, cnt, c->d_pcoef);
+    recover_blob_kernel<<<cnt, kCellNttThreads, kCellNttSmemBytes, st>>>(c->d_pcoef, c->tables, c->d_rblobs);
+    phase_end(ctx, 3, st);
+    CK(cudaGetLastError());
+    return fk20_launch(ctx, c->d_rblobs, cnt, d_cells_out, d_proofs_out, status);
+}
+// recovery of nb blobs that share one index set: d_in = nb x n_cells cells (blob-major).  One plan, one Z, for every pass.
+static int recover_launch(kzgb200_ctx* ctx, const RecoverPlan& plan, const uint8_t* d_in, size_t n_cells, size_t nb, uint8_t* d_cells_out,
+                          uint8_t* d_proofs_out) {
+    int rc = recover_upload(ctx, &plan, 1);
+    for (size_t lo = 0; !rc && lo < nb; lo += kProofChunk) {
         const int cnt = (int)(nb - lo < kProofChunk ? nb - lo : kProofChunk);
-        phase_begin(ctx, 3, st);
-        recover_load_kernel<<<(unsigned)((size_t)cnt * kExtElements / 256), 256, 0, st>>>(d_in + lo * n_cells * kBytesPerCell, (int)n_cells, c->d_pos,
-                                                                                         c->d_z, cnt, c->d_A, ctx->d_status + lo);
-        recover_ntt_inv_kernel<<<dim3(2, cnt), kCellNttThreads, kCellNttSmemBytes, st>>>(c->d_A, c->tables);
-        recover_mid_kernel<<<(unsigned)((size_t)cnt * kFieldElementsPerBlob / 256), 256, 0, st>>>(c->d_A, c->ptables, cnt);
-        recover_ntt_div_kernel<<<dim3(2, cnt), kCellNttThreads, kCellNttSmemBytes, st>>>(c->d_A, c->tables, c->d_z);
-        recover_final_kernel<<<(unsigned)((size_t)cnt * kFieldElementsPerBlob / 256), 256, 0, st>>>(c->d_A, c->ptables, cnt, c->d_pcoef);
-        recover_blob_kernel<<<cnt, kCellNttThreads, kCellNttSmemBytes, st>>>(c->d_pcoef, c->tables, c->d_rblobs);
-        phase_end(ctx, 3, st);
-        CK(cudaGetLastError());
-        int rc = fk20_launch(ctx, c->d_rblobs, cnt, d_cells_out + lo * kCellsPerExtBlob * kBytesPerCell, d_proofs_out + lo * kCellsPerExtBlob * 48,
-                             ctx->d_status + lo);
-        if (rc) return rc;
+        rc = recover_pass(ctx, 0, d_in + lo * n_cells * kBytesPerCell, n_cells, cnt, d_cells_out + lo * kCellsPerExtBlob * kBytesPerCell,
+                          d_proofs_out + lo * kCellsPerExtBlob * 48, ctx->d_status + lo);
     }
-    return KZGB200_OK;
+    return rc;
 }
 extern "C" int kzgb200_recover_cells_and_kzg_proofs(kzgb200_ctx* ctx, const uint64_t* cell_indices, const uint8_t* cells, size_t n_cells,
                                                     uint8_t* cells_out, uint8_t* proofs_out) {
     if (!ctx || !cells || !cells_out || !proofs_out) return KZGB200_BAD_ARGS;
     if (!proof_ready(ctx)) return KZGB200_INVALID_SETUP;
-    int pos[kCellsPerExtBlob], n_missing = 0;
-    uint32_t missing[kCellsPerExtBlob];
-    int rc = recover_plan(cell_indices, n_cells, pos, missing, &n_missing);
+    RecoverPlan plan;
+    int rc = recover_plan(cell_indices, n_cells, &plan);
     if (rc) return rc;
     std::lock_guard<std::mutex> g(ctx->lock);
     DeviceGuard dev(ctx->device);
@@ -1914,7 +1937,7 @@ extern "C" int kzgb200_recover_cells_and_kzg_proofs(kzgb200_ctx* ctx, const uint
     CellCtx* c = ctx->cells;
     if (!c->d_ext) CK(cudaMalloc(&c->d_ext, (size_t)kCellsPerExtBlob * kBytesPerCell));
     CK(cudaMemcpyAsync(c->d_rin, cells, n_cells * kBytesPerCell, cudaMemcpyHostToDevice, ctx->stream));
-    if ((rc = recover_launch(ctx, pos, missing, n_missing, c->d_rin, n_cells, 1, c->d_ext, c->d_pout))) return rc;
+    if ((rc = recover_launch(ctx, plan, c->d_rin, n_cells, 1, c->d_ext, c->d_pout))) return rc;
     if ((rc = proof_result(ctx, 1))) return rc;
     CK(cudaMemcpyAsync(cells_out, c->d_ext, (size_t)kCellsPerExtBlob * kBytesPerCell, cudaMemcpyDeviceToHost, ctx->stream));
     CK(cudaMemcpyAsync(proofs_out, c->d_pout, (size_t)kCellsPerExtBlob * 48, cudaMemcpyDeviceToHost, ctx->stream));
@@ -1925,13 +1948,94 @@ extern "C" int kzgb200_recover_cells_and_kzg_proofs_batch_device(kzgb200_ctx* ct
                                                                  size_t n_blobs, uint8_t* d_cells_out, uint8_t* d_proofs_out) {
     if (!ctx || (n_blobs && (!d_cells || !d_cells_out || !d_proofs_out)) || n_blobs > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
     if (!proof_ready(ctx)) return KZGB200_INVALID_SETUP;
-    int pos[kCellsPerExtBlob], n_missing = 0;
-    uint32_t missing[kCellsPerExtBlob];
-    int rc = recover_plan(cell_indices, n_cells, pos, missing, &n_missing);
+    RecoverPlan plan;
+    int rc = recover_plan(cell_indices, n_cells, &plan);
     if (rc || n_blobs == 0) return rc;
     std::lock_guard<std::mutex> g(ctx->lock);
     DeviceGuard dev(ctx->device);
     if ((rc = proof_begin(ctx, n_blobs))) return rc;
-    if ((rc = recover_launch(ctx, pos, missing, n_missing, d_cells, n_cells, n_blobs, d_cells_out, d_proofs_out))) return rc;
+    if ((rc = recover_launch(ctx, plan, d_cells, n_cells, n_blobs, d_cells_out, d_proofs_out))) return rc;
     return proof_result(ctx, n_blobs);
+}
+// recover_cells_and_kzg_proofs of n_blobs blobs, each from its own cells and index set: blob b owns cells and indices [off[b], off[b + 1]).
+// The plans are built on the host; a blob that fails the argument checks keeps the empty plan (its kernels read nothing) and gets
+// status BAD_ARGS.  Passes of kProofChunk blobs: the pass's plans and Z rows, then the recovery and FK20 kernels with one plan per
+// blob.  Host form (host = true): the cells of a pass's good blobs are staged packed (one copy per run of consecutive good blobs),
+// and the pass's outputs are copied back.
+static int recover_many(kzgb200_ctx* ctx, const uint64_t* idx, const uint8_t* cells, const uint64_t* off, size_t n_blobs, uint8_t* cells_out,
+                        uint8_t* proofs_out, uint8_t* status, bool host) {
+    const size_t limit = 0x7fffffff / 2;
+    if (!ctx || n_blobs > limit || (n_blobs && (!off || !cells_out || !proofs_out || !status))) return KZGB200_BAD_ARGS;
+    if (n_blobs) {
+        if (off[0] != 0) return KZGB200_BAD_ARGS;
+        for (size_t b = 0; b < n_blobs; b++) if (off[b + 1] < off[b]) return KZGB200_BAD_ARGS;
+        if (off[n_blobs] > limit || (off[n_blobs] && (!idx || !cells))) return KZGB200_BAD_ARGS;
+    }
+    if (!proof_ready(ctx)) return KZGB200_INVALID_SETUP;
+    if (n_blobs == 0) return KZGB200_OK;
+    std::vector<RecoverPlan> plans(n_blobs);
+    std::vector<uint8_t> bad(n_blobs);
+    size_t stage_cells = 0, pass_cells = 0;      // host form: the largest pass's cells of good blobs
+    for (size_t b = 0; b < n_blobs; b++) {
+        if (b % kProofChunk == 0) pass_cells = 0;
+        bad[b] = recover_plan(idx + off[b], off[b + 1] - off[b], &plans[b]) != KZGB200_OK;
+        if (!bad[b]) pass_cells += off[b + 1] - off[b];
+        stage_cells = std::max(stage_cells, pass_cells);
+    }
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    int rc = proof_begin(ctx, n_blobs);
+    if (rc) return rc;
+    CellCtx* c = ctx->cells;
+    cudaStream_t st = ctx->stream;
+    const size_t chunk = std::min(n_blobs, kProofChunk);
+    if (host && stage_cells > c->mstage_cells) {
+        c->mstage_cells = 0;
+        CK(regrow(c->d_mstage, stage_cells * kBytesPerCell));
+        c->mstage_cells = stage_cells;
+    }
+    if (host && chunk > c->mout_cap) {
+        c->mout_cap = 0;
+        CK(regrow(c->d_mcells, chunk * kCellsPerExtBlob * kBytesPerCell)); CK(regrow(c->d_mproofs, chunk * kCellsPerExtBlob * 48));
+        c->mout_cap = chunk;
+    }
+    for (size_t lo = 0; lo < n_blobs; lo += kProofChunk) {
+        const size_t cnt = std::min(n_blobs - lo, kProofChunk), hi = lo + cnt;
+        const uint8_t* d_in = nullptr;
+        if (host) {
+            size_t packed = 0;
+            for (size_t b = lo; b < hi;) {
+                if (bad[b]) { b++; continue; }
+                size_t e = b;
+                for (; e < hi && !bad[e]; e++) plans[e].first = (uint32_t)(packed + off[e] - off[b]);
+                const size_t n = off[e] - off[b];
+                CK(cudaMemcpyAsync(c->d_mstage + packed * kBytesPerCell, cells + off[b] * kBytesPerCell, n * kBytesPerCell, cudaMemcpyHostToDevice, st));
+                packed += n;
+                b = e;
+            }
+            d_in = c->d_mstage;
+        } else {
+            for (size_t b = lo; b < hi; b++) plans[b].first = (uint32_t)(off[b] - off[lo]);
+            d_in = cells + off[lo] * kBytesPerCell;
+        }
+        if ((rc = recover_upload(ctx, plans.data() + lo, cnt))) return rc;
+        uint8_t* d_c = host ? c->d_mcells : cells_out + lo * kCellsPerExtBlob * kBytesPerCell;
+        uint8_t* d_p = host ? c->d_mproofs : proofs_out + lo * kCellsPerExtBlob * 48;
+        if ((rc = recover_pass(ctx, 1, d_in, 0, (int)cnt, d_c, d_p, ctx->d_status + lo))) return rc;
+        if (host) {
+            CK(cudaMemcpyAsync(cells_out + lo * kCellsPerExtBlob * kBytesPerCell, d_c, cnt * kCellsPerExtBlob * kBytesPerCell, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(proofs_out + lo * kCellsPerExtBlob * 48, d_p, cnt * kCellsPerExtBlob * 48, cudaMemcpyDeviceToHost, st));
+        }
+    }
+    return proof_result_each(ctx, n_blobs, bad.data(), status);
+}
+extern "C" int kzgb200_recover_cells_and_kzg_proofs_many(kzgb200_ctx* ctx, const uint64_t* cell_indices, const uint8_t* cells,
+                                                         const uint64_t* cell_offsets, size_t n_blobs, uint8_t* cells_out, uint8_t* proofs_out,
+                                                         uint8_t* status) {
+    return recover_many(ctx, cell_indices, cells, cell_offsets, n_blobs, cells_out, proofs_out, status, true);
+}
+extern "C" int kzgb200_recover_cells_and_kzg_proofs_many_device(kzgb200_ctx* ctx, const uint64_t* cell_indices, const uint8_t* d_cells,
+                                                                const uint64_t* cell_offsets, size_t n_blobs, uint8_t* d_cells_out,
+                                                                uint8_t* d_proofs_out, uint8_t* status) {
+    return recover_many(ctx, cell_indices, d_cells, cell_offsets, n_blobs, d_cells_out, d_proofs_out, status, false);
 }

@@ -70,9 +70,10 @@ struct CellCtx {
     G1* d_V = nullptr;                                             // V[f] = sum_b U_b[f] W_b[f]
     uint8_t* d_rblobs = nullptr;                                   // recovered blobs
     uint8_t *d_rin = nullptr, *d_pout = nullptr;                   // staging of one host call: input cells, 128 proofs
-    int* d_pos = nullptr;                                          // recovery: input position of each cell index (-1: missing)
-    uint32_t* d_missing = nullptr;
-    Fr* d_z = nullptr;                                             // see recover_z_kernel
+    RecoverPlan* d_plans = nullptr;                                // recovery: the index sets of a pass (proof_cap), see recover_plan
+    Fr* d_z = nullptr;                                             // their Z rows (2 x 128 per plan), see recover_z_kernel
+    size_t mstage_cells = 0, mout_cap = 0;                         // recover_cells_and_kzg_proofs_many, host form: staging of one pass's
+    uint8_t *d_mstage = nullptr, *d_mcells = nullptr, *d_mproofs = nullptr;   // input cells, output cells and proofs (grow on demand)
     // verify_cell_kzg_proof_batch_many: per-group buffers for gcap groups, the fallback's workspace (per cell, per (group, index)
     // run), and the last call's r_g (32 bytes each, canonical big-endian) followed by rho
     size_t gcap = 0, fmeta_cap = 0, terms_cap = 0, rcoef_cap = 0;
