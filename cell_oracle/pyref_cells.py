@@ -104,24 +104,30 @@ def recover_cells(cell_indices, cells):
     return [flat[BYTES_PER_CELL * k:BYTES_PER_CELL * (k + 1)] for k in range(CELLS_PER_EXT_BLOB)]
 
 
-def fk20_in_exponent(coeffs, tau):
-    """FK20 as the GPU computes it, with every [tau^j]G1 replaced by tau^j: the 128 "proofs" q_k(tau) of the polynomial with these
-    4096 coefficients, in cell order.  u_b[a] = c_{64a+b} (zero-padded to 128), w_b[0] = tau^b, w_b[128-d] = tau^(64d+b)
-    (d = 1..62); V[f] = sum_b DFT(u_b)[f] DFT(w_b)[f]; H_t = IDFT(V)[t+1] (t < 63); pi_k = DFT(H)[rev7(k)]."""
+def fk20_commitment_and_proofs_in_exponent(coeffs, tau, d_max=63):
+    """FK20 as the GPU computes it, with every [tau^j]G1 replaced by tau^j: (p(tau), the 128 "proofs" q_k(tau) in cell order) of the
+    polynomial with these 4096 coefficients.  u_b[a] = c_{64a+b} (zero-padded to 128), w_b[0] = tau^b, w_b[128-d] = tau^(64d+b)
+    (d = 1..d_max); V[f] = sum_b DFT(u_b)[f] DFT(w_b)[f]; the commitment is IDFT(V)[0], H_t = IDFT(V)[t+1] (t < 63),
+    pi_k = DFT(H)[rev7(k)].  The proofs need d <= 62 only; d = 63 completes IDFT(V)[0] (d_max=62 leaves out the terms m >= 4032)."""
     w128 = pow(PRIMITIVE_ROOT_OF_UNITY, (Q - 1) // 128, Q)
     V = [0] * 128
     for b in range(FIELD_ELEMENTS_PER_CELL):
         u = [coeffs[64 * a + b] for a in range(64)] + [0] * 64
         w = [0] * 128
         w[0] = pow(tau, b, Q)
-        for d in range(1, 63):
+        for d in range(1, d_max + 1):
             w[128 - d] = pow(tau, 64 * d + b, Q)
         U, W = _fft(u, w128), _fft(w, w128)
         V = [(V[f] + U[f] * W[f]) % Q for f in range(128)]
     conv = _ifft(V, w128)
     H = conv[1:64] + [0] * 65
     out = _fft(H, w128)
-    return [out[bit_reverse(k, 7)] for k in range(CELLS_PER_EXT_BLOB)]
+    return conv[0], [out[bit_reverse(k, 7)] for k in range(CELLS_PER_EXT_BLOB)]
+
+
+def fk20_in_exponent(coeffs, tau):
+    """The 128 proofs of fk20_commitment_and_proofs_in_exponent."""
+    return fk20_commitment_and_proofs_in_exponent(coeffs, tau)[1]
 
 
 def cell_quotient_at(coeffs, tau, k):

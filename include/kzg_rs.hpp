@@ -6,7 +6,8 @@
 //   kzg_rs::Blob / Bytes32 / Bytes48 (from_slice length check, as_slice)                        src/dtypes.rs:7-46
 //   kzg_rs::KzgError                                                                            src/enums.rs:6-18
 // plus the EIP-4844 publisher calls kzg_rs::blob_to_kzg_commitment / compute_kzg_proof / compute_blob_kzg_proof, and EIP-7594 cells: kzg_rs::Cell, KzgProof::verify_cell_kzg_proof_batch[_many], kzg_rs::compute_cells, kzg_rs::compute_cells_and_kzg_proofs,
-// kzg_rs::recover_cells_and_kzg_proofs (c-kzg-4844 / rust-kzg names).
+// kzg_rs::recover_cells_and_kzg_proofs (c-kzg-4844 / rust-kzg names), and kzg_rs::compute_commitments_and_cell_proofs (a blob publisher's
+// commitments and cell proofs in one call).
 // Result<bool, KzgError> is kzg_rs::Result<bool>: either a value or an error.
 #pragma once
 #include <array>
@@ -256,6 +257,23 @@ inline Result<CellsAndProofs> recover_cells_and_kzg_proofs(const std::vector<uin
     int rc = kzgb200_recover_cells_and_kzg_proofs(kzg_settings.ctx(), cell_indices.data(), reinterpret_cast<const uint8_t*>(cells.data()),
                                                   cells.size(), reinterpret_cast<uint8_t*>(out.cells.data()),
                                                   reinterpret_cast<uint8_t*>(out.proofs.data()));
+    if (rc) return detail::to_result(rc, 0).unwrap_err();
+    return out;
+}
+// A publisher's outputs for many blobs in one FK20 pass per 512 blobs, with only the proof setup: blob b's commitment (commitments[b],
+// the bytes of blob_to_kzg_commitment), its 128 cell proofs (proofs[128 b ..], cell order) and, with want_cells, its cells
+// (cells[128 b ..]).  status[b] = 0, or 1 where the blob alone would give BadArgs (its slots then unspecified).  An error only for
+// the call itself (setup, device).
+struct CommitmentsAndCellProofs { std::vector<Bytes48> commitments; std::vector<Cell> cells; std::vector<Bytes48> proofs; std::vector<uint8_t> status; };
+inline Result<CommitmentsAndCellProofs> compute_commitments_and_cell_proofs(const std::vector<Blob>& blobs, const KzgSettings& kzg_settings,
+                                                                            bool want_cells = false) {
+    const size_t n = blobs.size();
+    CommitmentsAndCellProofs out{std::vector<Bytes48>(n), std::vector<Cell>(want_cells ? CELLS_PER_EXT_BLOB * n : 0),
+                                 std::vector<Bytes48>(CELLS_PER_EXT_BLOB * n), std::vector<uint8_t>(n)};
+    int rc = kzgb200_compute_commitments_and_cell_proofs(kzg_settings.ctx(), reinterpret_cast<const uint8_t*>(blobs.data()), n,
+                                                         reinterpret_cast<uint8_t*>(out.commitments.data()),
+                                                         reinterpret_cast<uint8_t*>(out.proofs.data()),
+                                                         want_cells ? reinterpret_cast<uint8_t*>(out.cells.data()) : nullptr, out.status.data());
     if (rc) return detail::to_result(rc, 0).unwrap_err();
     return out;
 }

@@ -307,6 +307,14 @@ int kzgb200_verify_blob_cell_kzg_proof_batch_many_device(kzgb200_ctx* ctx, const
  *   returns BAD_ARGS only when malformed (a null pointer with blobs to recover, bad offsets, n_blobs or off[n_blobs] above
  *   0x7fffffff / 2), INVALID_SETUP before the proof setup, and OK for n_blobs == 0 (cell_offsets then unread).  Blobs that share one
  *   index set cost about what the _batch_device call costs for them.
+ * kzgb200_compute_commitments_and_cell_proofs[_device]: what a blob publisher needs, in one FK20 pass per 512 blobs: for blob b its
+ *   commitment (commitments_out + 48 b, the bytes of kzgb200_blob_to_kzg_commitment), its 128 cell proofs (proofs_out + 128 x 48 b, in
+ *   cell order) and, when cells_out is not null, its cells (cells_out + 128 x 2048 b).  The commitment is output 0 of FK20's inverse
+ *   G1 DFT, so only the proof setup is needed (not kzgb200_load_g1_lagrange).  blobs n_blobs x 131072 bytes; host pointers, _device:
+ *   device pointers except status.  status (host, one byte per blob) = what kzgb200_blob_to_kzg_commitment /
+ *   kzgb200_compute_cells_and_kzg_proofs return for that blob alone: 0, or 1 (BAD_ARGS: a non-canonical element), its output slots
+ *   unspecified; a bad blob changes no other blob's output.  The call returns OK for n_blobs == 0 (nothing read, ctx may be null),
+ *   BAD_ARGS for a null pointer other than cells_out or n_blobs above 0x7fffffff / 2, INVALID_SETUP before the proof setup.
  * With kzgb200_set_profiling on, kzgb200_get_phase_ms reports for these calls {coefficients (with compute_cells), fixed-base products
  * (with the scalar DFTs), G1 transforms (with compression), recovery transforms, 0, 0, 0, 0}, first start to last end. */
 int kzgb200_load_cell_proof_setup(kzgb200_ctx* ctx, const uint8_t* g1_lagrange48, size_t n_points);
@@ -322,6 +330,10 @@ int kzgb200_recover_cells_and_kzg_proofs_many(kzgb200_ctx* ctx, const uint64_t* 
 int kzgb200_recover_cells_and_kzg_proofs_many_device(kzgb200_ctx* ctx, const uint64_t* cell_indices, const uint8_t* d_cells,
                                                      const uint64_t* cell_offsets, size_t n_blobs, uint8_t* d_cells_out, uint8_t* d_proofs_out,
                                                      uint8_t* status);
+int kzgb200_compute_commitments_and_cell_proofs(kzgb200_ctx* ctx, const uint8_t* blobs, size_t n_blobs, uint8_t* commitments_out,
+                                                uint8_t* proofs_out, uint8_t* cells_out, uint8_t* status);
+int kzgb200_compute_commitments_and_cell_proofs_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n_blobs, uint8_t* d_commitments_out,
+                                                       uint8_t* d_proofs_out, uint8_t* d_cells_out, uint8_t* status);
 
 /* per-phase device timing of batch calls (CUDA event pairs on the stream each phase runs on).  out8 = milliseconds of
  * {G1 decompression, challenge, evaluate, transcript r (exposed part: last chunk copy + host hash + upload), lincomb terms, reduce,

@@ -140,6 +140,8 @@ class Library:
         d.kzgb200_recover_cells_and_kzg_proofs_batch_device.argtypes = [p, p, sz, p, sz, p, p]
         d.kzgb200_recover_cells_and_kzg_proofs_many.argtypes = [p, p, p, p, sz, p, p, p]
         d.kzgb200_recover_cells_and_kzg_proofs_many_device.argtypes = [p, p, p, p, sz, p, p, p]
+        d.kzgb200_compute_commitments_and_cell_proofs.argtypes = [p, p, sz, p, p, p, p]
+        d.kzgb200_compute_commitments_and_cell_proofs_device.argtypes = [p, p, sz, p, p, p, p]
 
 
 def _raise(rc, ctx=None, msg=None):
@@ -597,6 +599,34 @@ def recover_cells_and_kzg_proofs_many(blobs, kzg_settings, device=0):
     cb, pb = BYTES_PER_CELL * CELLS_PER_EXT_BLOB, BYTES_PER_PROOF * CELLS_PER_EXT_BLOB
     return [None if st[b] or b in out_of_range else _cells_and_proofs(rc_cells[cb * b:cb * (b + 1)], rc_proofs[pb * b:pb * (b + 1)])
             for b in range(k)]
+
+
+def compute_commitments_and_cell_proofs(blobs, kzg_settings, device=0, want_cells=False):
+    """What a publisher of EIP-7594 blob transactions needs, in one GPU call: per blob its commitment (blob_to_kzg_commitment's
+    48 bytes) and its 128 cell proofs, both from one FK20 pass, so only the proof setup is loaded (cell_proof_context).  Returns one
+    (commitment, proofs) per blob, or (commitment, cells, proofs) with want_cells, or None where blob_to_kzg_commitment /
+    compute_cells_and_kzg_proofs would raise BadArgs (a non-canonical element); a bad blob does not change another's result.  A
+    wrong blob length anywhere -> KzgError(InvalidBytesLength) for the whole call, before any GPU work."""
+    raw = b"".join(_b(x, BYTES_PER_BLOB, "blob") for x in blobs)
+    k = len(raw) // BYTES_PER_BLOB
+    ctx = kzg_settings.cell_proof_context(device)
+    pb, cb = BYTES_PER_PROOF * CELLS_PER_EXT_BLOB, BYTES_PER_CELL * CELLS_PER_EXT_BLOB
+    commitments, proofs = C.create_string_buffer(48 * max(k, 1)), C.create_string_buffer(pb * max(k, 1))
+    cells = C.create_string_buffer(cb * max(k, 1)) if want_cells else None
+    status = C.create_string_buffer(max(k, 1))
+    rc = Library.get().dll.kzgb200_compute_commitments_and_cell_proofs(ctx, _ptr(raw), k, commitments, proofs, cells, status)
+    if rc:
+        _raise(rc, ctx)
+    cm, pr, st = commitments.raw, proofs.raw, status.raw
+    cr = cells.raw if want_cells else None
+    out = []
+    for b in range(k):
+        if st[b]:
+            out.append(None)
+            continue
+        c, p = _cells_and_proofs(cr[cb * b:cb * (b + 1)] if want_cells else b"", pr[pb * b:pb * (b + 1)])
+        out.append((cm[48 * b:48 * (b + 1)], c, p) if want_cells else (cm[48 * b:48 * (b + 1)], p))
+    return out
 
 
 def blob_to_kzg_commitment(blob, kzg_settings, device=0):

@@ -260,6 +260,8 @@ __global__ void fk20_table_kernel(const G1Affine* __restrict__ W, G1Affine* __re
 __global__ void fk20_scalars_kernel(const Fr* __restrict__ coeffs, const CellTables* __restrict__ T, Fr* __restrict__ U);
 __global__ void fk20_products_kernel(const Fr* __restrict__ U, const G1Affine* __restrict__ tab, G1* __restrict__ V);
 __global__ void fk20_proofs_kernel(const G1* __restrict__ V, const CellTables* __restrict__ T, uint8_t* __restrict__ proofs);
+__global__ void fk20_proofs_commit_kernel(const G1* __restrict__ V, const CellTables* __restrict__ T, uint8_t* __restrict__ proofs, G1* __restrict__ commit);
+__global__ void fk20_commit_kernel(const G1* __restrict__ commit, int n, uint8_t* __restrict__ out48);
 // recovery: blob i of a pass uses plan i * plan_stride (0: one index set shared by the pass) and its Z row
 __global__ void recover_z_kernel(const RecoverPlan* __restrict__ plans, const CellTables* __restrict__ T, const ProofTables* __restrict__ P,
                                  Fr* __restrict__ zvals);

@@ -4,8 +4,10 @@
 // FK20.  p = sum_{m<4096} c_m X^m, m = 64a + b, s_k = h_k^64 = omega128^rev7(k).  The proof of cell k is [q_k(tau)]G1 with
 // q_k = p div (X^64 - s_k) = sum_{t<63} s_k^t Q_t, so pi_k = sum_t s_k^t H_t, H_t = [Q_t(tau)]G1 -- a 128-point G1 DFT of
 // (H_0..H_62, 0, ..): pi_k is output rev7(k).  H_t = sum_b (u_b (*) w_b)[t + 1] (cyclic length-128 convolutions) with
-// u_b[a] = c_{64a+b} (a < 64, zero above) and w_b[0] = [tau^b], w_b[128 - d] = [tau^(64d+b)] (d = 1..62), zero elsewhere; by the
-// convolution theorem H = IDFT(V)[1..63], V[f] = sum_b U_b[f] W_b[f], U_b = DFT(u_b), W_b = DFT_G1(w_b) fixed at setup.
+// u_b[a] = c_{64a+b} (a < 64, zero above) and w_b[0] = [tau^b], w_b[128 - d] = [tau^(64d+b)] (d = 1..63), zero elsewhere; by the
+// convolution theorem H = IDFT(V)[1..63], V[f] = sum_b U_b[f] W_b[f], U_b = DFT(u_b), W_b = DFT_G1(w_b) fixed at setup.  Output 0 of
+// the same IDFT is sum_b sum_{a<64} c_{64a+b} [tau^(64a+b)] = [p(tau)], the blob's commitment: w_b[65] (d = 63) meets u_b only there
+// (at a = 63; for outputs 1..63 at a >= 64, where u_b is zero), so it completes the commitment and changes no H_t.
 //
 // Recovery follows recover_polynomialcoeff literally: E (zeros at the missing cells) times Z on the 8192-point domain, inverse
 // transform, coset (shift 7) transform, division by Z on the coset, inverse coset transform, first 4096 coefficients.  Z(X) = z(X^64)
@@ -122,7 +124,7 @@ __global__ void __launch_bounds__(64) fk20_w_kernel(const G1Affine* __restrict__
     for (int n = t; n < kCellsPerExtBlob; n += 64) {
         G1 v = G1::identity();
         if (n == 0) v = G1::from_affine(mono[b]);
-        else if (n >= 66) v = G1::from_affine(mono[64 * (128 - n) + b]);      // d = 128 - n = 1..62
+        else if (n >= 65) v = G1::from_affine(mono[64 * (128 - n) + b]);      // d = 128 - n = 1..63
         s[rev_bits_p((uint32_t)n, 7)] = v;
     }
     __syncthreads();
@@ -189,13 +191,18 @@ __global__ void __launch_bounds__(64) fk20_products_kernel(const Fr* __restrict_
     }
     if (b == 0) V[row] = sm[0];
 }
-// per blob (64 threads): H = IDFT(V)[1..63], then the proofs pi_k = DFT(H)[rev7(k)], compressed (blob-major, cell order)
-__global__ void __launch_bounds__(64) fk20_proofs_kernel(const G1* __restrict__ V, const CellTables* __restrict__ T, uint8_t* __restrict__ proofs) {
+// per blob (64 threads): H = IDFT(V)[1..63], then the proofs pi_k = DFT(H)[rev7(k)], compressed (blob-major, cell order).
+// kCommit: also IDFT(V)[0], the blob's commitment (Jacobian; fk20_commit_kernel compresses it), stored by thread 63, whose H is the
+// identity, so that no point is held across the forward DFT.  A template flag, so that fk20_proofs_kernel's code stays as it was.
+template <bool kCommit>
+__device__ __forceinline__ void fk20_proofs_body(const G1* __restrict__ V, const CellTables* __restrict__ T, uint8_t* __restrict__ proofs,
+                                                 G1* __restrict__ commit) {
     __shared__ G1 s[kCellsPerExtBlob];
     const int blob = blockIdx.x, t = threadIdx.x;
     for (int f = t; f < kCellsPerExtBlob; f += 64) s[rev_bits_p((uint32_t)f, 7)] = V[(size_t)blob * kCellsPerExtBlob + f];
     __syncthreads();
     g1_dft128(s, T, true);
+    if (kCommit && t == 63) commit[blob] = s[0];
     const G1 h = t < 63 ? s[t + 1] : G1::identity();     // H_t
     __syncthreads();
     s[rev_bits_p((uint32_t)t, 7)] = h;
@@ -208,6 +215,21 @@ __global__ void __launch_bounds__(64) fk20_proofs_kernel(const G1* __restrict__ 
         uint8_t* dst = proofs + ((size_t)blob * kCellsPerExtBlob + k) * 48;
         for (int i = 0; i < 48; i++) dst[i] = enc[i];
     }
+}
+__global__ void __launch_bounds__(64) fk20_proofs_kernel(const G1* __restrict__ V, const CellTables* __restrict__ T, uint8_t* __restrict__ proofs) {
+    fk20_proofs_body<false>(V, T, proofs, nullptr);
+}
+__global__ void __launch_bounds__(64) fk20_proofs_commit_kernel(const G1* __restrict__ V, const CellTables* __restrict__ T, uint8_t* __restrict__ proofs,
+                                                                G1* __restrict__ commit) {
+    fk20_proofs_body<true>(V, T, proofs, commit);
+}
+// the n commitments of fk20_proofs_kernel, compressed (one thread per blob)
+__global__ void __launch_bounds__(128) fk20_commit_kernel(const G1* __restrict__ commit, int n, uint8_t* __restrict__ out48) {
+    const int i = blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= n) return;
+    uint8_t enc[48];
+    g1_to_compressed(enc, g1_to_affine(commit[i]));
+    for (int k = 0; k < 48; k++) out48[(size_t)i * 48 + k] = enc[k];
 }
 
 // ---- recover_cells_and_kzg_proofs ------------------------------------------------------------------------------------

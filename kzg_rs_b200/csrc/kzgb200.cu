@@ -1111,10 +1111,10 @@ extern "C" void kzgb200_free_pinned(void* p) { if (p) cudaFreeHost(p); }
 
 // ---- EIP-7594 cells (k_cells.cu; consensus-specs Fulu polynomial-commitments-sampling.md) ---------------------------------
 static void proof_destroy(CellCtx* c) {
-    void* d[] = {c->ptables, c->d_mono, c->d_fk_tab, c->d_pcoef, c->d_fkU, c->d_A, c->d_V, c->d_rblobs, c->d_rin, c->d_pout, c->d_plans, c->d_z,
+    void* d[] = {c->ptables, c->d_mono, c->d_fk_tab, c->d_pcoef, c->d_fkU, c->d_A, c->d_V, c->d_pcommit, c->d_rblobs, c->d_rin, c->d_pout, c->d_plans, c->d_z,
                  c->d_mstage, c->d_mcells, c->d_mproofs};
     for (void* p : d) if (p) cudaFree(p);
-    c->ptables = nullptr; c->d_mono = c->d_fk_tab = nullptr; c->d_pcoef = c->d_fkU = c->d_A = c->d_z = nullptr; c->d_V = nullptr;
+    c->ptables = nullptr; c->d_mono = c->d_fk_tab = nullptr; c->d_pcoef = c->d_fkU = c->d_A = c->d_z = nullptr; c->d_V = c->d_pcommit = nullptr;
     c->d_rblobs = c->d_rin = c->d_pout = nullptr; c->d_plans = nullptr; c->proof_cap = 0;
     c->d_mstage = c->d_mcells = c->d_mproofs = nullptr; c->mstage_cells = c->mout_cap = 0;
 }
@@ -1785,14 +1785,17 @@ static int proof_workspace(kzgb200_ctx* ctx, size_t n) {
     if (nb <= c->proof_cap) return KZGB200_OK;
     c->proof_cap = 0;
     CK(regrow(c->d_pcoef, nb * kFieldElementsPerBlob)); CK(regrow(c->d_fkU, nb * kFk20Bases)); CK(regrow(c->d_A, nb * kExtElements));
-    CK(regrow(c->d_V, nb * kCellsPerExtBlob)); CK(regrow(c->d_rblobs, nb * kBytesPerBlob));
+    CK(regrow(c->d_V, nb * kCellsPerExtBlob)); CK(regrow(c->d_pcommit, nb)); CK(regrow(c->d_rblobs, nb * kBytesPerBlob));
     CK(regrow(c->d_plans, nb)); CK(regrow(c->d_z, nb * 2 * kCellsPerExtBlob));
     c->proof_cap = nb;
     return KZGB200_OK;
 }
-// cells and proofs of n device blobs (the caller has checked n <= proof_cap or chunks; status: n flags, zeroed by the caller).
-// Profiling slots: 0 = coefficients (with the cells), 1 = fixed-base products (with the scalar DFTs), 2 = G1 transforms.
-static int fk20_launch(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8_t* d_cells, uint8_t* d_proofs, uint32_t* status) {
+// cells and proofs of n device blobs (the caller has checked n <= proof_cap or chunks; status: n flags, zeroed by the caller), and
+// with d_commitments (nullable) their commitments, output 0 of FK20's inverse G1 DFT.
+// Profiling slots: 0 = coefficients (with the cells), 1 = fixed-base products (with the scalar DFTs), 2 = G1 transforms (with the
+// commitments' compression).
+static int fk20_launch(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8_t* d_cells, uint8_t* d_proofs, uint32_t* status,
+                       uint8_t* d_commitments = nullptr) {
     CellCtx* c = ctx->cells;
     cudaStream_t st = ctx->stream;
     for (size_t lo = 0; lo < n; lo += kProofChunk) {
@@ -1806,7 +1809,12 @@ static int fk20_launch(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n, uint8
         fk20_products_kernel<<<dim3(kCellsPerExtBlob, cnt), 64, 0, st>>>(c->d_fkU, c->d_fk_tab, c->d_V);
         phase_end(ctx, 1, st);
         phase_begin(ctx, 2, st);
-        fk20_proofs_kernel<<<cnt, 64, 0, st>>>(c->d_V, c->tables, d_proofs + lo * kCellsPerExtBlob * 48);
+        if (d_commitments) {
+            fk20_proofs_commit_kernel<<<cnt, 64, 0, st>>>(c->d_V, c->tables, d_proofs + lo * kCellsPerExtBlob * 48, c->d_pcommit);
+            fk20_commit_kernel<<<(cnt + 127) / 128, 128, 0, st>>>(c->d_pcommit, cnt, d_commitments + lo * 48);
+        } else {
+            fk20_proofs_kernel<<<cnt, 64, 0, st>>>(c->d_V, c->tables, d_proofs + lo * kCellsPerExtBlob * 48);
+        }
         phase_end(ctx, 2, st);
     }
     CK(cudaGetLastError());
@@ -1868,6 +1876,58 @@ extern "C" int kzgb200_compute_cells_and_kzg_proofs_batch_device(kzgb200_ctx* ct
     int rc = proof_begin(ctx, n);
     if (!rc) rc = fk20_launch(ctx, d_blobs, n, d_cells, d_proofs, ctx->d_status);
     return rc ? rc : proof_result(ctx, n);
+}
+// the commitment and the cell proofs (and, with cells_out, the cells) of n blobs, one FK20 pass per kProofChunk blobs, the commitment from the same
+// inverse G1 DFT (fk20_launch with commitments): blob-major outputs, status[b] = what blob_to_kzg_commitment /
+// compute_cells_and_kzg_proofs would return for blob b alone.  Host form (host = true): each pass of kProofChunk blobs is staged in
+// the context's blob buffer and its outputs are copied back.  Without cells_out the cells go to the _many workspace (d_mcells).
+static int commit_cells_proofs(kzgb200_ctx* ctx, const uint8_t* blobs, size_t n, uint8_t* commitments_out, uint8_t* proofs_out,
+                               uint8_t* cells_out, uint8_t* status, bool host) {
+    if (n == 0) return KZGB200_OK;
+    if (!ctx || !blobs || !commitments_out || !proofs_out || !status || n > 0x7fffffff / 2) return KZGB200_BAD_ARGS;
+    if (!proof_ready(ctx)) return KZGB200_INVALID_SETUP;
+    std::lock_guard<std::mutex> g(ctx->lock);
+    DeviceGuard dev(ctx->device);
+    int rc = proof_begin(ctx, n);
+    const size_t chunk = std::min(n, kProofChunk);
+    if (!rc && host) rc = ensure_capacity(ctx, chunk, true);
+    if (rc) return rc;
+    CellCtx* c = ctx->cells;
+    cudaStream_t st = ctx->stream;
+    if ((host || !cells_out) && chunk > c->mout_cap) {
+        c->mout_cap = 0;
+        CK(regrow(c->d_mcells, chunk * kCellsPerExtBlob * kBytesPerCell)); CK(regrow(c->d_mproofs, chunk * kCellsPerExtBlob * 48));
+        c->mout_cap = chunk;
+    }
+    for (size_t lo = 0; lo < n; lo += kProofChunk) {
+        const size_t cnt = std::min(n - lo, kProofChunk);
+        const uint8_t* d_in = blobs + lo * kBytesPerBlob;
+        uint8_t* d_cm = commitments_out + lo * 48;
+        uint8_t* d_c = cells_out && !host ? cells_out + lo * kCellsPerExtBlob * kBytesPerCell : c->d_mcells;
+        uint8_t* d_p = host ? c->d_mproofs : proofs_out + lo * kCellsPerExtBlob * 48;
+        if (host) {
+            CK(cudaMemcpyAsync(ctx->d_blobs, d_in, cnt * kBytesPerBlob, cudaMemcpyHostToDevice, st));
+            d_in = ctx->d_blobs;
+            d_cm = ctx->d_c;
+        }
+        if ((rc = fk20_launch(ctx, d_in, cnt, d_c, d_p, ctx->d_status + lo, d_cm))) return rc;
+        if (host) {
+            CK(cudaMemcpyAsync(commitments_out + lo * 48, d_cm, cnt * 48, cudaMemcpyDeviceToHost, st));
+            CK(cudaMemcpyAsync(proofs_out + lo * kCellsPerExtBlob * 48, d_p, cnt * kCellsPerExtBlob * 48, cudaMemcpyDeviceToHost, st));
+            if (cells_out)
+                CK(cudaMemcpyAsync(cells_out + lo * kCellsPerExtBlob * kBytesPerCell, d_c, cnt * kCellsPerExtBlob * kBytesPerCell, cudaMemcpyDeviceToHost, st));
+        }
+    }
+    const std::vector<uint8_t> no_host_checks(n);
+    return proof_result_each(ctx, n, no_host_checks.data(), status);
+}
+extern "C" int kzgb200_compute_commitments_and_cell_proofs(kzgb200_ctx* ctx, const uint8_t* blobs, size_t n_blobs, uint8_t* commitments_out,
+                                                           uint8_t* proofs_out, uint8_t* cells_out, uint8_t* status) {
+    return commit_cells_proofs(ctx, blobs, n_blobs, commitments_out, proofs_out, cells_out, status, true);
+}
+extern "C" int kzgb200_compute_commitments_and_cell_proofs_device(kzgb200_ctx* ctx, const uint8_t* d_blobs, size_t n_blobs, uint8_t* d_commitments_out,
+                                                                  uint8_t* d_proofs_out, uint8_t* d_cells_out, uint8_t* status) {
+    return commit_cells_proofs(ctx, d_blobs, n_blobs, d_commitments_out, d_proofs_out, d_cells_out, status, false);
 }
 
 // The spec's argument checks on one index set: 64 <= n_cells <= 128, every index < 128, no index twice.  plan: pos[k] = the input

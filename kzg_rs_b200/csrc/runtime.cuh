@@ -68,6 +68,7 @@ struct CellCtx {
     size_t proof_cap = 0;
     Fr *d_pcoef = nullptr, *d_fkU = nullptr, *d_A = nullptr;        // coefficients x 4096 / recovered coefficients, U_b[f], 8192-point work
     G1* d_V = nullptr;                                             // V[f] = sum_b U_b[f] W_b[f]
+    G1* d_pcommit = nullptr;                                       // IDFT(V)[0] per blob: the commitments of a pass (Jacobian)
     uint8_t* d_rblobs = nullptr;                                   // recovered blobs
     uint8_t *d_rin = nullptr, *d_pout = nullptr;                   // staging of one host call: input cells, 128 proofs
     RecoverPlan* d_plans = nullptr;                                // recovery: the index sets of a pass (proof_cap), see recover_plan
